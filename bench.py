@@ -263,6 +263,22 @@ def reference_inflate_check(stream_ptr, stream_len, total, kind=1, seed=1, piece
     return bool(ok)
 
 
+def oracle_inflate_check(stream_ptr, stream_len, total, kind=1, seed=1):
+    """reference_inflate_check where the reference is not built: the oracle (oracle/libzoracle.so, the reference's inflate
+    restated in C) decodes the whole stream in one call; True when it ends exactly at stream_len with a good trailer and
+    the output is the regenerated corpus."""
+    import numpy as np
+    import zhelpers
+    from zlib_b200 import synth
+    orc = zhelpers.Oracle()
+    out = np.empty(max(total, 1), dtype=np.uint8)
+    ol, used = C.c_size_t(0), C.c_size_t(0)
+    rc = orc.dll.zo_inflate(C.c_void_p(stream_ptr), stream_len, C.c_void_p(out.ctypes.data), total, C.byref(ol), C.byref(used), 1)
+    if rc != 0 or ol.value != total or used.value != stream_len:
+        return False
+    return bool(np.array_equal(out[:total], synth.synth(total, kind, seed)))
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -390,6 +406,32 @@ class SharedHost:
         self.ptr = self.private = None
 
 
+DUMP_SAMPLE = 1 << 22                  # stream bytes --dump-outputs keeps: 16 MiB of float32 values and 32 MiB of float64
+                                       # positions, within 64 MB
+DUMP_EDGE = 1 << 16                    # the stream's first and last bytes are always kept (header, last block, trailer)
+
+
+def dump_stream(out_dir, lib, ptr, clen):
+    """What the caller of the timed deflate receives, for comparing two builds output for output:
+    deflate_level1_length.npy    the stream's length in bytes (float64, one element);
+    deflate_level1_stream.npy    its bytes as float32: all of them when they fit DUMP_SAMPLE, else the first and last
+                                 DUMP_EDGE bytes and positions drawn with a fixed seed, in stream order;
+    deflate_level1_positions.npy where in the stream each of those bytes sits (float64)."""
+    import numpy as np
+    host = np.empty(clen, dtype=np.uint8)
+    lib.dll.zb200_copy(C.c_void_p(host.ctypes.data), C.c_void_p(ptr), clen, None)
+    if clen <= DUMP_SAMPLE:
+        pos = np.arange(clen)
+    else:
+        drawn = np.random.default_rng(0).integers(DUMP_EDGE, clen - DUMP_EDGE, DUMP_SAMPLE - 2 * DUMP_EDGE)
+        pos = np.unique(np.concatenate([np.arange(DUMP_EDGE), drawn, np.arange(clen - DUMP_EDGE, clen)]))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "deflate_level1_length.npy"), np.array([clen], dtype=np.float64))
+    np.save(os.path.join(out_dir, "deflate_level1_stream.npy"), host[pos].astype(np.float32))
+    np.save(os.path.join(out_dir, "deflate_level1_positions.npy"), pos.astype(np.float64))
+    log(f"[rank 0] {len(pos)} of the {clen} stream bytes written to {out_dir}")
+
+
 def traffic_of(kernel):
     """dram__bytes_read + dram__bytes_write per launch of `kernel` from the ncu capture summarised in profiles/traffic.json
     -- only when that capture was taken from the kernel sources as they are now (their hash is stored beside it)."""
@@ -412,7 +454,8 @@ def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the headline and the end-to-end measurement (at "
+                    "least 1); the side measurements of the extras keep their own counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="zb200", choices=["zb200", "reference"])
     ap.add_argument("--size-mib", type=int, default=1024)
@@ -420,7 +463,13 @@ def main():
                     "such as 0.5,0.375,0.125 (default: 0.5,0.375,0.125)")
     ap.add_argument("--no-extra", action="store_true", help="skip level 6 / inflate / checksum / zip side measurements")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the stream the last timed deflate step produced to DIR/*.npy (see dump_stream)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the GPU path computed; --impl reference has no such output")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -522,6 +571,9 @@ def main():
     ms1, launches = timed(lambda: step_deflate(1), args.steps, warm)
     clocks = sampler.summary()
     clen1 = state["clen"]
+    if args.dump_outputs and rank == 0:                      # before anything else reuses the output buffer
+        dump_ptr = d_dst.data_ptr() if world == 1 else final_ptr if final_ptr is not None else d_final.data_ptr()
+        dump_stream(args.dump_outputs, lib, dump_ptr, int(clen1))
     value = total / ms1 / 1e6
     log(f"[rank {rank}] deflate L1: {ms1:.2f} ms/step  {value:.2f} GB/s aggregate  ratio {total / clen1:.3f}")
 
@@ -606,27 +658,29 @@ def main():
     import zhelpers
     have_ref = os.path.exists(zhelpers.REF_PATH)
     if rank == 0:
-        # ---- correctness gate (a) on the measured outputs: the reference decodes them bit-exact ----
-        if not args.no_verify and have_ref:
+        # ---- correctness gate (a) on the measured outputs: the reference (else the oracle) decodes them bit-exact ----
+        check = reference_inflate_check if have_ref else oracle_inflate_check
+        verified_with = "reference inflate (oracle/_ref)" if have_ref else "oracle inflate (oracle/libzoracle.so)"
+        if not args.no_verify:
             t0 = time.perf_counter()
             if world == 1:
-                verified = reference_inflate_check(pin_dst, int(state["e2e_len"]), total)
+                verified = check(pin_dst, int(state["e2e_len"]), total)
             else:
                 h_final = np.empty(int(clen1), dtype=np.uint8)
                 lib.dll.zb200_copy(C.c_void_p(h_final.ctypes.data), C.c_void_p(final_ptr if final_ptr is not None else d_final.data_ptr()), int(clen1), None)
                 if shm.ptr is not None:                         # the stream in the shared host buffer is decoded by the reference;
-                    ok_host = reference_inflate_check(shm_ptr, int(state["e2e_len"]), total)
+                    ok_host = check(shm_ptr, int(state["e2e_len"]), total)
                     same = int(clen1) == int(state["e2e_len"]) and bool(np.array_equal(                    # the one on the root GPU must be the same bytes
                         h_final, np.ctypeslib.as_array(C.cast(shm_ptr, C.POINTER(C.c_uint8)), shape=(int(clen1),))))
-                    ok_dev = same or reference_inflate_check(h_final.ctypes.data, int(clen1), total)
+                    ok_dev = same or check(h_final.ctypes.data, int(clen1), total)
                 else:
-                    ok_host, ok_dev = True, reference_inflate_check(h_final.ctypes.data, int(clen1), total)
+                    ok_host, ok_dev = True, check(h_final.ctypes.data, int(clen1), total)
                 verified = bool(ok_dev and ok_host)
                 assembled = True
                 del h_final
-            log(f"[rank 0] assembled stream(s) decoded and compared by the reference inflate (oracle/_ref): {verified} "
+            log(f"[rank 0] assembled stream(s) decoded and compared by the {verified_with}: {verified} "
                 f"({time.perf_counter() - t0:.1f} s)")
-            assert verified, "reference could not decode the GPU deflate output"
+            assert verified, f"the {verified_with} could not decode the GPU deflate output"
         # ---- CPU baseline beside it: same number of bytes as one GPU's share ----
         if have_ref:
             rb = RefBench(n)
@@ -652,7 +706,8 @@ def main():
                 "config": workload_config(args.size_mib, world),
                 "ratio": round(total / clen1, 4), "compressed_bytes": int(clen1),
                 "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": int(launches),
-                "clocks": clocks, "verified_by_reference": verified, "assembled": assembled if world > 1 else True,
+                "clocks": clocks, "verified_by_reference": verified,
+                "verified_with": None if verified is None else verified_with, "assembled": assembled if world > 1 else True,
                 "gather": (None if world == 1 else "copy engines over NVLink into rank 0's buffer (CUDA IPC)" if final_ptr is not None
                            else "NCCL send / recv into rank 0's buffer"),
                 "extra": extra}

@@ -29,6 +29,18 @@ def ref():
 
 
 @pytest.fixture(scope="session")
+def reference_codec(oracle):
+    """compress2 / uncompress / deflate with a strategy as the reference computes them: the unmodified reference build
+    when oracle/_ref has it, else the oracle, whose compress2 and uncompress tests/test_oracle_pin.py holds byte for byte
+    to outputs recorded from the reference (tests/golden).  The oracle has no strategies: those streams then come from
+    the system zlib."""
+    import zhelpers
+    if os.path.exists(zhelpers.REF_PATH):
+        return zhelpers.Ref()
+    return zhelpers.OracleAsReference(oracle)
+
+
+@pytest.fixture(scope="session")
 def lib():
     from zlib_b200 import load
     return load()

@@ -51,7 +51,7 @@ def test_all_levels(gpu_lib, oracle):
     assert rc == 0 and len(z) == sizes[6]
 
 
-def test_level_ladder_against_the_reference(gpu_lib, ref):
+def test_level_ladder_against_the_reference(gpu_lib, reference_codec):
     """Every level: no larger than the reference's output at the SAME level (+2 %, gate (d)), sizes do not grow with the
     level (0.1 % slack: the budgets are knees of a sweep, not a proof), and the reference decodes each stream."""
     for kind, seed in ((0, 21), (1, 22)):
@@ -61,23 +61,23 @@ def test_level_ladder_against_the_reference(gpu_lib, ref):
         for level in range(1, 10):
             rc, z = gpu_lib.compress2(data, level)
             assert rc == 0
-            want = len(ref.compress2(raw, level))
+            want = len(reference_codec.compress2(raw, level))
             assert len(z) <= 1.02 * want, (kind, level, len(z), want)
             if prev is not None:
                 assert len(z) <= 1.001 * prev, (kind, level, len(z), prev)
             prev = len(z)
-            rc, out = ref.uncompress(z, len(raw))
+            rc, out = reference_codec.uncompress(z, len(raw))
             assert rc == 0 and out == raw
 
 
-def test_reference_decodes_gpu_output(gpu_lib, oracle, ref):
+def test_reference_decodes_gpu_output(gpu_lib, oracle, reference_codec):
     rng = random.Random(3)
     for t in range(20):
         data = zhelpers.corpus(rng.randrange(5), rng.randint(0, 500000), 50 + t)
         for level in (1, 6):
             rc, z = gpu_lib.compress2(data, level)
             assert rc == 0
-            _decode_everywhere(z, data, oracle, ref)
+            _decode_everywhere(z, data, oracle, reference_codec)
 
 
 @pytest.mark.parametrize("kind", [0, 1])
@@ -93,7 +93,7 @@ def test_ratio_gate_vs_reference(gpu_lib, oracle, kind):
         assert rc == 0 and out == data.tobytes()
 
 
-def test_ratio_gate_at_config_one_shape(gpu_lib, ref):
+def test_ratio_gate_at_config_one_shape(gpu_lib, reference_codec):
     """Gate (d) at BASELINE config 1's shape: 64 MiB of synthetic text, levels 1 and 6, against the unmodified reference
     build compressing the WHOLE buffer as one stream; and the reference decodes what we wrote (gate (a))."""
     n = 64 << 20
@@ -101,9 +101,9 @@ def test_ratio_gate_at_config_one_shape(gpu_lib, ref):
     for level in (1, 6):
         rc, z = gpu_lib.compress2(text, level)
         assert rc == 0
-        want = len(ref.compress2(text, level))
+        want = len(reference_codec.compress2(text, level))
         assert len(z) <= 1.02 * want, (level, len(z), want, len(z) / want)
-        rc, out = ref.uncompress(z, n)
+        rc, out = reference_codec.uncompress(z, n)
         assert rc == 0 and out == text.tobytes()
 
 

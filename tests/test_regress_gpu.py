@@ -27,10 +27,10 @@ def _runs(n, seed):
     return bytes(out[:n])
 
 
-def test_runs_through_small_feeds(gpu_lib, oracle, ref):
+def test_runs_through_small_feeds(gpu_lib, oracle, reference_codec):
     for seed, n in ((1, 1 << 20), (2, 3 << 20), (3, 300000)):
         data = _runs(n, seed) if seed != 2 else bytes(n)
-        for z in (ref.compress2(data, 9), oracle.deflate(data, 6), zlib.compress(data, 1)):
+        for z in (reference_codec.compress2(data, 9), oracle.deflate(data, 6), zlib.compress(data, 1)):
             for in_chunk in (64, 77, 100):
                 rc, out, msg, tin = gpu_lib.inflate_stream(z, 15, in_chunk, 1 << 20)
                 assert rc == zb.Z_STREAM_END and msg is None, (seed, in_chunk, rc, msg)

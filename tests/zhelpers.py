@@ -140,6 +140,50 @@ class Ref:
         return z
 
 
+class OracleAsReference:
+    """The calls of Ref that the GPU gates use, answered by the oracle (system zlib for deflate strategies)."""
+
+    def __init__(self, oracle):
+        self.oracle = oracle
+
+    def compress2(self, data, level=6):
+        return self.oracle.deflate(data, level)
+
+    def uncompress(self, comp, cap):
+        rc, out, _ = self.oracle.inflate(comp, cap)
+        return rc, (out if rc == 0 else b"")
+
+    def deflate_stream(self, data, level=6, wbits=15, strategy=0):
+        import zlib
+        co = zlib.compressobj(level, zlib.DEFLATED, wbits, 8, strategy)
+        return co.compress(bytes(data)) + co.flush()
+
+
+def unzip_with_oracle(path, oracle):
+    """{name: bytes} of every member of the ZIP archive at `path`: the central directory as Python's zipfile reads it,
+    each member's data found through its own local header and decoded by the oracle's raw inflate; the decoded length
+    and CRC-32 must be the ones the directory records."""
+    import struct
+    import zipfile
+    blob = open(path, "rb").read()
+    out = {}
+    for info in zipfile.ZipFile(path).infolist():
+        sig = struct.unpack_from("<I", blob, info.header_offset)[0]
+        name_len, extra_len = struct.unpack_from("<HH", blob, info.header_offset + 26)
+        assert sig == 0x04034B50, (info.filename, hex(sig))
+        start = info.header_offset + 30 + name_len + extra_len
+        raw = blob[start:start + info.compress_size]
+        if info.compress_type == zipfile.ZIP_DEFLATED:
+            rc, data, used = oracle.inflate(raw, info.file_size, 0)
+            assert rc == 0 and used == len(raw), (info.filename, rc, oracle.last_msg())
+        else:
+            assert info.compress_type == zipfile.ZIP_STORED, (info.filename, info.compress_type)
+            data = raw
+        assert len(data) == info.file_size and oracle.crc32(data) == info.CRC, info.filename
+        out[info.filename] = data
+    return out
+
+
 def corpus(kind, n, seed=0):
     """Small deterministic test inputs (pure Python, independent of the product's generator)."""
     rng = random.Random(seed * 1000003 + kind * 7919 + n)
