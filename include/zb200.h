@@ -135,6 +135,35 @@ int zb200_zip_segment(const char *const *names, const void *src, const uint64_t 
 int zb200_zip_directory(const char *const *names, const zb200_zip_member *members, size_t n,
                         uint32_t dos_datetime, uint64_t cd_offset, void *dst, size_t *dst_len);
 
+/* ---- ZIP32 archives: reading (qcsrc/unzip.c, member by member in the reference) ----
+ * zb200_zip_list parses the central directory on the host, as unzOpen does: the end record is searched back through
+ * the archive comment, leading bytes in front of the archive are allowed (every offset below is into the buffer as
+ * given), multi-disk and ZIP64 archives are refused with Z_STREAM_ERROR.  The archive may be host or device memory (a
+ * device archive has its end record and directory copied to the host).  *n: in = capacity, out = member count;
+ * Z_BUF_ERROR (with *n = the count needed) when the capacity is too small.
+ * zb200_zip_extract decodes entries[0 .. n) -- any subset of an archive, in any order -- into dst[dst_off[i] ..
+ * dst_off[i+1]), all on the GPU; archive and dst may each be host or device memory.  dst_len[i] = bytes produced;
+ * status[i] = Z_OK (length and CRC-32 as the directory states), ZB200_UNZ_BADZIPFILE (local header missing or not
+ * coherent with the directory as unzip.c checks it, a method other than stored / deflated, a stored member whose sizes
+ * differ, data outside the archive), Z_STREAM_ERROR (encrypted), Z_BUF_ERROR (slot smaller than raw_len), Z_DATA_ERROR
+ * (invalid deflate data or a length other than raw_len), ZB200_UNZ_CRCERROR.  Returns Z_OK when the batch ran. */
+typedef struct zb200_zip_entry {
+    uint64_t local_off;          /* local header, as an offset into the archive buffer */
+    uint64_t comp_len, raw_len;
+    uint64_t name_off;           /* the member name inside the archive buffer (its central directory record) */
+    uint32_t crc32;
+    uint16_t method, flags;      /* compression method, general purpose bit flag */
+    uint16_t name_len, reserved16;
+    uint32_t reserved32;
+} zb200_zip_entry;               /* 48 bytes */
+
+#define ZB200_UNZ_BADZIPFILE (-103)   /* values of minizip's unzip.h */
+#define ZB200_UNZ_CRCERROR   (-105)
+
+int zb200_zip_list(const void *archive, size_t arc_len, zb200_zip_entry *entries, size_t *n);
+int zb200_zip_extract(const void *archive, size_t arc_len, const zb200_zip_entry *entries, size_t n,
+                      void *dst, const uint64_t *dst_off, uint64_t *dst_len, int32_t *status, void *stream);
+
 /* ---- inflate: n independent streams (qcsrc/uncompr.c:26 uncompress, batched) ----
  * Stream i occupies src[src_off[i] .. src_off[i+1]) and is decoded into
  * dst[dst_off[i] .. dst_off[i+1]).  Per stream: dst_len[i] = bytes produced,

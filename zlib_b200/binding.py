@@ -21,6 +21,7 @@ WRAP_RAW, WRAP_ZLIB, WRAP_GZIP = 0, 1, 2
 DOS_DATETIME = 46 << 25 | 10 << 21 | 18 << 16            # 2026-10-18 00:00:00 in zip.c's dosDate layout
 ZB200_DEFLATE_NOT_LAST, ZB200_DEFLATE_NO_HEADER, ZB200_DEFLATE_NO_TRAILER = 1, 2, 4
 ZLIB_VERSION = b"1.2.3"
+ZB200_UNZ_BADZIPFILE, ZB200_UNZ_CRCERROR = -103, -105          # minizip's unzip.h values
 
 
 class z_stream(C.Structure):
@@ -70,6 +71,35 @@ class gz_header(C.Structure):
                 ("extra", C.c_void_p), ("extra_len", C.c_uint), ("extra_max", C.c_uint),
                 ("name", C.c_void_p), ("name_max", C.c_uint), ("comment", C.c_void_p), ("comm_max", C.c_uint),
                 ("hcrc", C.c_int), ("done", C.c_int)]
+
+
+class ZipEntry:
+    """One member as zb200_zip_list reports it; `raw` is the 48-byte zb200_zip_entry record."""
+    __slots__ = ("name", "local_off", "comp_len", "raw_len", "crc32", "method", "flags", "raw")
+
+    def __init__(self, name, rec):
+        self.name = name
+        self.local_off, self.comp_len, self.raw_len = int(rec["local_off"]), int(rec["comp_len"]), int(rec["raw_len"])
+        self.crc32, self.method, self.flags = int(rec["crc32"]), int(rec["method"]), int(rec["flags"])
+        self.raw = rec.copy()
+
+    def __repr__(self):
+        return (f"ZipEntry({self.name!r}, local_off={self.local_off}, comp_len={self.comp_len}, raw_len={self.raw_len}, "
+                f"crc32={self.crc32:#010x}, method={self.method}, flags={self.flags:#x})")
+
+
+def _zip_entry_dtype():
+    import numpy as np
+    return np.dtype([("local_off", "<u8"), ("comp_len", "<u8"), ("raw_len", "<u8"), ("name_off", "<u8"), ("crc32", "<u4"),
+                     ("method", "<u2"), ("flags", "<u2"), ("name_len", "<u2"), ("reserved16", "<u2"), ("reserved32", "<u4")])
+
+
+def _nbytes(buf) -> int:
+    if hasattr(buf, "data_ptr"):                                  # torch tensor
+        return buf.numel() * buf.element_size()
+    if hasattr(buf, "nbytes"):
+        return int(buf.nbytes)
+    return len(buf)
 
 
 class Lib:
@@ -130,6 +160,8 @@ class Lib:
             "zb200_zip_build": (C.c_int, [vp, vp, vp, sz, C.c_int, C.c_uint32, vp, C.POINTER(sz)]),
             "zb200_zip_segment": (C.c_int, [vp, vp, vp, sz, C.c_int, C.c_uint32, vp, C.POINTER(sz), vp]),
             "zb200_zip_directory": (C.c_int, [vp, vp, sz, C.c_uint32, C.c_uint64, vp, C.POINTER(sz)]),
+            "zb200_zip_list": (C.c_int, [vp, sz, vp, C.POINTER(sz)]),
+            "zb200_zip_extract": (C.c_int, [vp, sz, vp, sz, vp, vp, vp, vp, vp]),
             "zb200_inflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
             "zb200_inflate_batch_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
             "zb200_multi_devices": (C.c_int, []),
@@ -324,6 +356,65 @@ class Lib:
         self._check(self.dll.zb200_zip_directory(arr, members.ctypes.data, n, dos_datetime, cd_offset, out, C.byref(ol)),
                     "zb200_zip_directory")
         return out.raw[:ol.value]
+
+    def zip_list(self, archive):
+        """zb200_zip_list -> [ZipEntry]; names decoded as zipfile does (UTF-8 with flag bit 11, else cp437).
+        `archive`: bytes, a numpy array or a CUDA torch tensor of uint8."""
+        import numpy as np
+        p, keep = _ptr(archive)
+        size = _nbytes(archive)
+        cnt = C.c_size_t(0)
+        rc = self.dll.zb200_zip_list(p, size, None, C.byref(cnt))
+        if rc not in (Z_OK, Z_BUF_ERROR):
+            self._check(rc, "zb200_zip_list")
+        recs = np.zeros(max(cnt.value, 1), dtype=_zip_entry_dtype())
+        if cnt.value:
+            self._check(self.dll.zb200_zip_list(p, size, recs.ctypes.data, C.byref(cnt)), "zb200_zip_list")
+        recs = recs[:cnt.value]
+        names = []
+        if cnt.value:
+            lo = int(recs["name_off"].min())
+            hi = int((recs["name_off"] + recs["name_len"]).max())
+            if hasattr(archive, "data_ptr"):
+                blob = archive[lo:hi].cpu().numpy().tobytes()
+            else:
+                blob = bytes(memoryview(archive).cast("B")[lo:hi]) if not hasattr(archive, "ctypes") else archive[lo:hi].tobytes()
+            for r in recs:
+                raw = blob[int(r["name_off"]) - lo:int(r["name_off"]) - lo + int(r["name_len"])]
+                names.append(raw.decode("utf-8") if int(r["flags"]) & 0x800 else raw.decode("cp437"))
+        return [ZipEntry(nm, r) for nm, r in zip(names, recs)]
+
+    def zip_extract(self, archive, entries=None, caps=None, stream=None):
+        """zb200_zip_extract -> (outputs, statuses).  entries: ZipEntry list (default: every member, from zip_list); caps:
+        slot sizes (default raw_len).  With the archive in a CUDA torch tensor the outputs are views of one CUDA tensor,
+        otherwise bytes."""
+        import numpy as np
+        if entries is None:
+            entries = self.zip_list(archive)
+        n = len(entries)
+        recs = np.zeros(max(n, 1), dtype=_zip_entry_dtype())
+        for i, e in enumerate(entries):
+            recs[i] = e.raw
+        caps = [e.raw_len for e in entries] if caps is None else list(caps)
+        dst_off = np.zeros(n + 1, dtype=np.uint64)
+        dst_off[1:] = np.cumsum(caps, dtype=np.uint64)
+        on_dev = hasattr(archive, "data_ptr") and getattr(archive, "is_cuda", False)
+        if on_dev:
+            import torch
+            dst = torch.empty(int(dst_off[-1]) + 8, dtype=torch.uint8, device=archive.device)
+        else:
+            dst = np.zeros(int(dst_off[-1]) + 8, dtype=np.uint8)
+        dst_len = np.zeros(max(n, 1), dtype=np.uint64)
+        status = np.full(max(n, 1), -99, dtype=np.int32)
+        pa, keep = _ptr(archive)
+        pd, keep2 = _ptr(dst)
+        self._check(self.dll.zb200_zip_extract(pa, _nbytes(archive), recs.ctypes.data, n, pd, dst_off.ctypes.data,
+                                               dst_len.ctypes.data, status.ctypes.data, _stream(stream)), "zb200_zip_extract")
+        if on_dev:
+            outs = [dst[int(dst_off[i]):int(dst_off[i]) + int(dst_len[i])] for i in range(n)]
+        else:
+            outs = [dst[int(dst_off[i]):int(dst_off[i]) + int(dst_len[i])].tobytes() for i in range(n)]
+        return outs, [int(x) for x in status[:n]]
 
     def inflate_batch(self, streams, caps, wrap: int = WRAP_ZLIB, stream=None):
         """zb200_inflate_batch over a list of bytes objects; returns (outputs, statuses)."""

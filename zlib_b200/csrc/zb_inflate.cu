@@ -709,19 +709,23 @@ __device__ void inflate_warp(const uint8_t* in, uint64_t in_len, uint8_t* out, u
 __global__ void __launch_bounds__(kInfWarps * 32)
 k_inflate_batch(const uint8_t* __restrict__ src, const uint64_t* __restrict__ src_off, uint64_t n,
                 uint8_t* __restrict__ dst, const uint64_t* __restrict__ dst_off,
-                uint64_t* __restrict__ dst_len, int32_t* __restrict__ status, int wrap, uint32_t* __restrict__ expect)
+                uint64_t* __restrict__ dst_len, int32_t* __restrict__ status, int wrap, uint32_t* __restrict__ expect,
+                const uint32_t* __restrict__ ids, const uint64_t* __restrict__ src_end, const uint64_t* __restrict__ dst_end)
 {
     __shared__ WarpTables s_tab[kInfWarps];
     __shared__ InfState s_state[kInfWarps];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint64_t i = (uint64_t)blockIdx.x * kInfWarps + warp;
-    if (i >= n) return;
+    const uint64_t k = (uint64_t)blockIdx.x * kInfWarps + warp;
+    if (k >= n) return;
+    // ids == nullptr: stream k is [src_off[k], src_off[k + 1]); otherwise stream ids[k], whose ranges end at src_end / dst_end
+    // (members of an archive: any subset, each with its own slot)
+    const uint64_t i = ids ? ids[k] : k;
     InfState* st = &s_state[warp];
     for (int k = lane; k < (int)(sizeof(InfState) / 4); k += 32) reinterpret_cast<uint32_t*>(st)[k] = 0;
     __syncwarp();
     if (lane == 0) st->wrap = wrap;
     __syncwarp();
-    const uint64_t a = src_off[i], e = src_off[i + 1], oa = dst_off[i], oe = dst_off[i + 1];
+    const uint64_t a = src_off[i], e = ids ? src_end[i] : src_off[i + 1], oa = dst_off[i], oe = ids ? dst_end[i] : dst_off[i + 1];
     inflate_warp(src + a, e - a, dst + oa, oe - oa, false, st, &s_tab[warp], &dst_len[i], nullptr, &status[i], nullptr);
     __syncwarp();
     if (expect && lane == 0) {                                  // gzip members: {crc32, isize, 1} for the check that follows
@@ -750,10 +754,21 @@ int inflate_batch_launch(const uint8_t* d_src, const uint64_t* d_src_off, size_t
     if (gz && !d_expect) { set_error("inflate batch: gzip needs check scratch"); return ZB_STREAM_ERROR; }
     const unsigned blocks = (unsigned)((n + kInfWarps - 1) / kInfWarps);
     ZB_LAUNCH(k_inflate_batch, blocks, kInfWarps * 32, 0, s, d_src, d_src_off, (uint64_t)n, d_dst, d_dst_off, d_dst_len, d_status, wrap,
-              gz ? d_expect : nullptr);
+              gz ? d_expect : nullptr, (const uint32_t*)nullptr, (const uint64_t*)nullptr, (const uint64_t*)nullptr);
     ZB_CHECK_LAUNCH();
     // gzip trailer (inflate.c:1099-1112): CRC-32 and length of what was produced, for every member that decoded
     if (gz) return checksum_batch_launch(d_dst, d_dst_off, d_dst_len, n, nullptr, nullptr, d_expect, d_status, s);
+    return 0;
+}
+
+int inflate_members_launch(const uint8_t* d_src, const uint64_t* d_beg, const uint64_t* d_end, uint8_t* d_dst, const uint64_t* d_dst_beg,
+                           const uint64_t* d_dst_end, const uint32_t* d_ids, size_t nids, uint64_t* d_dst_len, int32_t* d_status,
+                           cudaStream_t s)
+{
+    if (nids == 0) return 0;
+    ZB_LAUNCH(k_inflate_batch, (unsigned)((nids + kInfWarps - 1) / kInfWarps), kInfWarps * 32, 0, s, d_src, d_beg, (uint64_t)nids, d_dst,
+              d_dst_beg, d_dst_len, d_status, (int)ZB200_WRAP_RAW, (uint32_t*)nullptr, d_ids, d_end, d_dst_end);
+    ZB_CHECK_LAUNCH();
     return 0;
 }
 
@@ -800,7 +815,16 @@ __global__ void __launch_bounds__(1024) k_slide_history(uint8_t* arena, uint64_t
 //   tails    one CTA walks the segments in order and resolves the last 32 KiB of each against the 32 KiB in front of it
 //            (already final by then): the only sequential part, ~64 KiB of traffic per segment;
 //   rest     every other symbol of every segment resolves in parallel against the final bytes in front of its segment.
-struct SegDesc { uint64_t start, stop, out_off, out_len; };     // BIT range of the segment's blocks; its place in the output
+//
+// The same kernels decode the segments of MANY streams in one set of launches (the members of a ZIP archive, whose lengths
+// the central directory states): a segment carries a "first segment of its stream" mark, and its symbols live at sym_off
+// of the scratch, which need not follow the output layout (one stream: sym_off == out_off).  sym_off == out_off mod 8.
+struct SegDesc {
+    uint64_t start, stop, out_off, out_len;                     // BIT range of the segment's blocks; its place in the output
+    uint64_t sym_off;                                           // its 16-bit symbols in the scratch
+    uint32_t flags, pad;                                        // kSegFirst / kSegLast: first / last segment of its stream
+};
+constexpr uint32_t kSegFirst = 1, kSegLast = 2;
 struct SegResult { uint64_t out_len, end_bit; int32_t status, final; uint32_t arrive, pad; };   // status 0 = ok, 1 = missed, 2 = invalid data
 constexpr uint64_t kSegMinOut = 128u << 10;                     // accepted segments are merged up to this much output (less for short streams)
 constexpr size_t kParFewStreams = 8;                            // with more streams than this in a call, only the really long ones are tried
@@ -972,7 +996,7 @@ __device__ void seg_decode(const uint8_t* in, uint64_t in_len, const SegDesc sd,
     b.nwords = (uint32_t)(((((uintptr_t)in + in_len + 3) & ~(uintptr_t)3) - (uintptr_t)b.words) >> 2);
     b.total = in_len * 8;
     seek_bits(b, in, sd.start);
-    uint16_t* out = kEmit ? sym + sd.out_off : nullptr;
+    uint16_t* out = kEmit ? sym + sd.sym_off : nullptr;
     uint64_t produced = 0;
     int status = 2, last = 0;
     uint32_t nx = self + 1, arrive = 0xffffffffu;
@@ -1080,6 +1104,12 @@ __device__ void seg_decode(const uint8_t* in, uint64_t in_len, const SegDesc sd,
         }
         if (bad) break;
     }
+    if (kEmit && produced < sd.out_len) {
+        // a segment that stopped short: the symbols it did not write are plain zero bytes, not whatever an earlier call left
+        // in the scratch -- the tail and rest kernels then read no window for them (the call falls back on it anyway)
+        __syncwarp();
+        for (uint64_t i = produced + lane; i < sd.out_len; i += 32) out[i] = 0;
+    }
     if (lane == 0) { res->out_len = produced; res->end_bit = b.used; res->status = status; res->final = last; res->arrive = arrive; res->pad = 0; }
 }
 
@@ -1094,8 +1124,11 @@ k_inflate_segments(const uint8_t* __restrict__ in, uint64_t in_len, const SegDes
     __shared__ WarpTables s_tab[kInfWarps];
     const uint32_t j = j_lo + blockIdx.x * kInfWarps + (threadIdx.x >> 5);
     if (j >= j_hi) return;
-    if (kEmit) seg_decode<true>(in, in_len, segs[j], j == 0, j == nseg - 1, sym, &s_tab[threadIdx.x >> 5], &res[j], nullptr, 0, 0);
-    else seg_decode<false>(in, in_len, SegDesc{cand[j], 0, 0, 0}, j == 0, false, nullptr, &s_tab[threadIdx.x >> 5], &res[j], cand, nseg, j);
+    if (kEmit) {
+        const SegDesc sd = segs[j];
+        seg_decode<true>(in, in_len, sd, (sd.flags & kSegFirst) != 0, (sd.flags & kSegLast) != 0, sym, &s_tab[threadIdx.x >> 5], &res[j], nullptr, 0, 0);
+    }
+    else seg_decode<false>(in, in_len, SegDesc{cand[j], 0, 0, 0, 0, 0, 0}, j == 0, false, nullptr, &s_tab[threadIdx.x >> 5], &res[j], cand, nseg, j);
 }
 
 // Tails in parallel.  The last 32 KiB of a segment only depend on the segment in front of it where they still hold
@@ -1113,25 +1146,27 @@ k_tails_round(const uint16_t* __restrict__ sym, uint8_t* __restrict__ out, const
     __shared__ uint32_t s_any;
     const uint32_t j = j_lo + blockIdx.x;
     const SegDesc sd = segs[j];
-    const uint64_t t = min(sd.out_len, (uint64_t)kWindow32), lo = sd.out_off + sd.out_len - t;
+    const uint64_t t = min(sd.out_len, (uint64_t)kWindow32), lo = sd.out_off + sd.out_len - t, slo = sd.sym_off + sd.out_len - t;
     if (round == 0) {
         if (threadIdx.x == 0) s_any = 0;
         __syncthreads();
         uint32_t any = 0;
-        for (uint64_t i = threadIdx.x; i < t; i += 256) any |= sym[lo + i] & 0x8000u;
+        for (uint64_t i = threadIdx.x; i < t; i += 256) any |= sym[slo + i] & 0x8000u;
         if (any) s_any = 1;                                     // benign race: every writer stores 1
         __syncthreads();
         if (s_any) { if (threadIdx.x == 0) done[j] = 0; return; }
-        for (uint64_t i = threadIdx.x; i < t; i += 256) out[lo + i] = (uint8_t)sym[lo + i];
+        for (uint64_t i = threadIdx.x; i < t; i += 256) out[lo + i] = (uint8_t)sym[slo + i];
         if (threadIdx.x == 0) done[j] = 1;
         return;
     }
     if (done[j] != 0) return;
-    if (j != 0) { const uint32_t d = done[j - 1]; if (d == 0 || d > round) return; }   // the window must be final since an EARLIER launch
+    // the window must be final since an EARLIER launch; a first segment has no window (it holds no window symbols, so round 0
+    // has finished it) and never waits on the segment in front of it, which belongs to another stream
+    if (!(sd.flags & kSegFirst)) { const uint32_t d = done[j - 1]; if (d == 0 || d > round) return; }
     const int64_t wbase = (int64_t)sd.out_off - (int64_t)kWindow32;
     uint32_t bad = 0;
     for (uint64_t i = threadIdx.x; i < t; i += 256) {
-        uint32_t v = sym[lo + i];
+        uint32_t v = sym[slo + i];
         if (v & 0x8000u) {
             const int64_t q = wbase + (int64_t)(v & 0x7fffu);
             if (q < 0) { bad++; v = 0; }
@@ -1164,6 +1199,10 @@ __global__ void k_tails_first_open(const uint32_t* __restrict__ done, uint32_t j
 // other CTAs through distributed shared memory.  A trip (one segment's tail) is then 4 K symbols per SM instead of 32 K
 // on one (the single-CTA form was bound by that one SM's instruction issue: 7 us per trip), two cluster barriers, and no
 // scattered L2 gathers; the symbols of the NEXT trip are requested before this trip's work.
+// Many streams in one walk need nothing else here: the ring runs on across a stream boundary, which is safe only because a
+// first segment holds no window symbols (seg_decode refuses them), so the bytes of another stream that the ring holds in
+// front of it are never read; every other segment's window is the end of its own stream's previous segment, the trip
+// before.  The symbols are read at sym_off, which keeps the output position's residue mod 8 (the 16-byte loads).
 constexpr int kTailCtas = 8, kTailThreads = 512;
 constexpr uint32_t kTailSlice = kWindow32 / kTailCtas;          // 4096 positions per CTA and trip
 
@@ -1199,28 +1238,35 @@ k_resolve_tails(const uint16_t* __restrict__ sym, uint8_t* __restrict__ out, con
             const uint64_t g = m * (kTailSlice / 8) + threadIdx.x;
             if (g * 8 + 8 > lo && g * 8 < hi && n < 2) {
                 w.grp[n] = g;
-                w.v[n] = *reinterpret_cast<const uint4*>(sym + g * 8);
+                w.v[n] = *reinterpret_cast<const uint4*>(sym + (g * 8 - d.out_off + d.sym_off));
                 n++;
             }
         }
     };
-    TailWork cur, nxt;
-    SegDesc sd = segs[j0], sn = sd;
-    fetch(sd, nxt);
-    if (j0 > 0) {
-        // a later launch of the same walk: the ring is the 32 KiB of final output in front of the first segment
-        const uint64_t hi = sd.out_off, lo = hi > kWindow32 ? hi - kWindow32 : 0;
+    // the ring from the 32 KiB of final output in front of a segment
+    auto load_ring = [&](const SegDesc& d) {
+        const uint64_t hi = d.out_off, lo = hi > kWindow32 ? hi - kWindow32 : 0;
         for (uint64_t m = lo >> 12; hi && m <= (hi - 1) >> 12; m++) {
             if ((m & (kTailCtas - 1)) != r) continue;
             for (uint64_t p = max(lo, m << 12) + threadIdx.x; p < min(hi, (m + 1) << 12); p += kTailThreads)
                 ring[(uint32_t)p & (kTailSlice - 1)] = __ldcg(out + p);
         }
         cluster.sync();
-    }
+    };
+    TailWork cur, nxt;
+    SegDesc sd = segs[j0], sn = sd;
+    fetch(sd, nxt);
+    bool stale = j0 > 0;                                        // a later launch of the same walk: the ring comes from the output
     uint32_t bad = 0;
     for (uint32_t j = j0; j < nseg; j++) {
         sd = sn; cur = nxt;
         if (j + 1 < nseg) { sn = segs[j + 1]; fetch(sn, nxt); }
+        // A tail the parallel rounds finished is final in the output already: no trip (every CTA reads the same word, written
+        // by an earlier launch), and the ring is reloaded in front of the next open one.  With many segments -- the members
+        // of an archive -- one long chain of dependent tails otherwise costs a trip for every segment behind it.
+        if (first_open && j > j0 && done[j] != 0) { stale = true; continue; }
+        if (stale && !(sd.flags & kSegFirst)) load_ring(sd);   // a first segment has no window to load
+        stale = false;
         const uint64_t t = min(sd.out_len, (uint64_t)kWindow32), lo = sd.out_off + sd.out_len - t, hi = lo + t;
         const int64_t wbase = (int64_t)sd.out_off - (int64_t)kWindow32;
         uint32_t bytes[2][8];
@@ -1273,7 +1319,7 @@ __global__ void __launch_bounds__(256) k_resolve_rest(const uint16_t* __restrict
     const SegDesc sd = segs[blockIdx.x];
     const uint64_t t = min(sd.out_len, (uint64_t)kWindow32), n = sd.out_len - t;
     for (uint64_t i = threadIdx.x; i < n; i += 256) {
-        const uint32_t v = sym[sd.out_off + i];
+        const uint32_t v = sym[sd.sym_off + i];
         uint32_t byte = v;
         if (v & 0x8000u) {
             const int64_t q = (int64_t)sd.out_off - (int64_t)kWindow32 + (int64_t)(v & 0x7fffu);
@@ -1348,15 +1394,36 @@ k_find_blocks_check(const uint8_t* __restrict__ in, uint64_t in_len, const uint6
     }
 }
 
+// Segments [j0, j1) of a list: emit (16-bit symbols), tails (parallel rounds, then the sequential walk for what they left
+// open), rest.  One stream or many: the launch shape does not depend on it, but for the number of tail rounds.
+static int launch_segment_phase(const uint8_t* d_src, uint64_t len, uint8_t* d_dst, const SegDesc* d_segs, uint32_t nseg,
+                                uint16_t* d_sym, SegResult* d_res, uint32_t* d_done, uint32_t* d_err, uint32_t* d_first_open,
+                                uint32_t j0, uint32_t j1, cudaStream_t s, int rounds = kTailRounds)
+{
+    ZB_LAUNCH((k_inflate_segments<true>), (j1 - j0 + kInfWarps - 1) / kInfWarps, kInfWarps * 32, 0, s, d_src, len, d_segs, nseg, d_sym, d_res,
+              (const uint64_t*)nullptr, j0, j1);
+    for (int r = 0; r < rounds; r++)
+        ZB_LAUNCH(k_tails_round, j1 - j0, 256, 0, s, d_sym, d_dst, d_segs, j0, d_done, (uint32_t)r, d_err);
+    ZB_LAUNCH(k_tails_first_open, 1, 1024, 0, s, d_done, j0, j1, d_first_open);
+    ZB_LAUNCH(k_resolve_tails, kTailCtas, kTailThreads, 0, s, d_sym, d_dst, d_segs, j0, j1, d_err, d_first_open, d_done);
+    ZB_LAUNCH(k_resolve_rest, j1 - j0, 256, 0, s, d_sym, d_dst, d_segs + j0, d_err);
+    ZB_CHECK_LAUNCH();
+    return 0;
+}
+
 // Second half of the one-stream decoder: emit (16-bit symbols), tails, rest, trailer check -- for a list of segments whose
 // sizes are known (counted) or assumed (speculative: every segment but the last is exactly out_len bytes, the last one at
 // most out_len; used for streams that look like this library's own, see inflate_single_parallel).  In speculative mode
 // `final_end` and the total are learnt from the last segment.  Returns 0 = decoded, 1 = not taken, negative = CUDA error.
-static int emit_segments(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_dst, const std::vector<SegDesc>& segs, uint64_t total,
+static int emit_segments(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_dst, std::vector<SegDesc> segs, uint64_t total,
                          uint64_t final_end, bool speculative, int wrap, cudaStream_t s, void* h_dst, uint64_t* total_out,
                          uint64_t* used_out, uint32_t* check_out)
 {
     const uint32_t nseg = (uint32_t)segs.size();
+    for (uint32_t j = 0; j < nseg; j++) {                       // one stream: symbols laid out like the output
+        segs[j].sym_off = segs[j].out_off;
+        segs[j].flags = (j == 0 ? kSegFirst : 0u) | (j == nseg - 1 ? kSegLast : 0u);
+    }
     const uint64_t sym_len = segs.back().out_off + segs.back().out_len;
     const uint64_t trailer_len = wrap == ZB200_WRAP_ZLIB ? 4 : wrap == ZB200_WRAP_GZIP ? 8 : 0;
     int rc;
@@ -1380,13 +1447,7 @@ static int emit_segments(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_
     for (uint32_t k = 0; k < nphase; k++) {
         const uint32_t j0 = (uint32_t)((uint64_t)nseg * k / nphase), j1 = (uint32_t)((uint64_t)nseg * (k + 1) / nphase);
         if (j1 == j0) continue;
-        ZB_LAUNCH((k_inflate_segments<true>), (j1 - j0 + kInfWarps - 1) / kInfWarps, kInfWarps * 32, 0, s, d_src, len, d_segs, nseg, d_sym, d_res,
-                  (const uint64_t*)nullptr, j0, j1);
-        for (int r = 0; r < kTailRounds; r++)
-            ZB_LAUNCH(k_tails_round, j1 - j0, 256, 0, s, d_sym, d_dst, d_segs, j0, d_done, (uint32_t)r, d_err);
-        ZB_LAUNCH(k_tails_first_open, 1, 1024, 0, s, d_done, j0, j1, d_first_open);
-        ZB_LAUNCH(k_resolve_tails, kTailCtas, kTailThreads, 0, s, d_sym, d_dst, d_segs, j0, j1, d_err, d_first_open, d_done);
-        ZB_LAUNCH(k_resolve_rest, j1 - j0, 256, 0, s, d_sym, d_dst, d_segs + j0, d_err);
+        if ((rc = launch_segment_phase(d_src, len, d_dst, d_segs, nseg, d_sym, d_res, d_done, d_err, d_first_open, j0, j1, s)) != 0) return rc;
         if (h_dst && !(speculative && k == nphase - 1)) {       // (the last speculative phase is copied once its true length is known)
             const uint64_t a = segs[j0].out_off, b = segs[j1 - 1].out_off + segs[j1 - 1].out_len;
             ZB_CUDA(cudaEventRecord(c->evs[k], s));
@@ -1444,8 +1505,8 @@ static int emit_segments(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_
 // Returns 0 when the stream was decoded here (*status, *out_len set), 1 when the caller should use the serial decoder
 // (no usable boundaries, output that does not fit, damaged data), negative on CUDA errors.
 int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_dst, uint64_t cap, int wrap,
-                            uint64_t* out_len, int32_t* status, cudaStream_t s, uint64_t* in_used = nullptr, uint32_t* adler = nullptr,
-                            int* wrap_found = nullptr, void* h_dst = nullptr)
+                            uint64_t* out_len, int32_t* status, cudaStream_t s, uint64_t* in_used, uint32_t* adler,
+                            int* wrap_found, void* h_dst)
 {
     if (len < kParMinInput || wrap < 0 || wrap > kWrapAuto) return 1;
     uint64_t hdr = 0;
@@ -1578,6 +1639,99 @@ int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t*
     if (in_used) *in_used = used;
     if (adler) *adler = check;
     if (wrap_found) *wrap_found = wrap;
+    return 0;
+}
+
+// ---- many raw streams of known output length in one segment decode (the large members of a ZIP archive) ----
+// A ZIP central directory states every member's uncompressed length, and a member this library wrote ends each ZB200_CHUNK
+// bytes of its input with a marker.  So a stream with exactly ceil(out_len / ZB200_CHUNK) - 1 markers has its segments
+// planned before anything is decoded -- segment j is output [j, j + 1) * ZB200_CHUNK, starting behind marker j - 1 -- and
+// no counting pass is needed: the non-speculative form of emit_segments, for all such streams at once.  The emit pass checks
+// every segment's length and arrival; a stream that misses either (a marker pattern that was data stands in for a real one)
+// leaves the plan with ok[i] = 0 and its output undefined, for the caller to decode another way.  Streams are taken in groups
+// of about kPlanGroupBytes of output, which bounds the symbol scratch (2 bytes per output byte).
+// Tails: a chain of dependent tails runs through a stream, and each round of k_tails_round finishes one more link of it in
+// EVERY stream at once, where the sequential walk would take the chains of all streams one after the other (text: most
+// tails hold window symbols, so the chain is most of a member; 2280 long members of the config-5 archive took 92 ms in the
+// walk with four rounds).  So the plan runs as many rounds as its longest stream has segments, up to kPlanTailRounds.
+constexpr uint64_t kPlanGroupBytes = 1ull << 30;
+constexpr uint32_t kPlanTailRounds = 64;
+
+int find_markers_launch(const uint8_t* d_src, uint64_t first, uint64_t last, uint32_t* d_count, uint64_t* d_pos, uint32_t cap, cudaStream_t s)
+{
+    ZB_LAUNCH(k_find_markers, device_sms() * 8, 256, 0, s, d_src, first, last, d_count, d_pos, cap);
+    ZB_CHECK_LAUNCH();
+    return 0;
+}
+
+int inflate_planned(Ctx* c, const uint8_t* d_src, uint64_t src_len, uint8_t* d_dst, const PlannedStream* ps, size_t np,
+                    const uint64_t* marks, uint8_t* ok, cudaStream_t s)
+{
+    int rc;
+    if ((rc = c->small.ensure(256)) != 0) return rc;
+    uint32_t* d_err = c->small.as<uint32_t>() + 17;
+    uint32_t* d_first_open = c->small.as<uint32_t>() + 18;
+    std::vector<SegDesc> segs;
+    std::vector<SegResult> res;
+    std::vector<uint32_t> seg0;                                 // first segment of each stream of the group
+    for (size_t g0 = 0; g0 < np;) {
+        size_t g1 = g0;
+        uint64_t out = 0;
+        while (g1 < np && (g1 == g0 || out + ps[g1].out_len <= kPlanGroupBytes)) out += ps[g1++].out_len;
+        segs.clear(); seg0.clear();
+        uint64_t sym = 16;                                      // k_resolve_tails reads whole groups of 8 around a segment's ends
+        for (size_t i = g0; i < g1; i++) {
+            const PlannedStream& p = ps[i];
+            sym += (p.out_off - sym) & 7;                       // the scratch keeps the output's residue mod 8
+            seg0.push_back((uint32_t)segs.size());
+            const uint32_t nseg = p.nmarks + 1;
+            for (uint32_t j = 0; j < nseg; j++) {
+                SegDesc d;
+                d.start = 8 * (j == 0 ? p.in_beg : marks[p.first_mark + j - 1]);
+                d.stop = j + 1 < nseg ? 8 * marks[p.first_mark + j] : 0;
+                d.out_off = p.out_off + (uint64_t)j * ZB200_CHUNK;
+                d.out_len = std::min<uint64_t>(ZB200_CHUNK, p.out_len - (uint64_t)j * ZB200_CHUNK);
+                d.sym_off = sym + (uint64_t)j * ZB200_CHUNK;
+                d.flags = (j == 0 ? kSegFirst : 0u) | (j + 1 == nseg ? kSegLast : 0u);
+                d.pad = 0;
+                segs.push_back(d);
+            }
+            sym += p.out_len + 8;
+        }
+        seg0.push_back((uint32_t)segs.size());
+        const uint32_t nseg = (uint32_t)segs.size();
+        uint32_t longest = 0;
+        for (size_t i = g0; i < g1; i++) longest = std::max(longest, ps[i].nmarks + 1);
+        const int rounds = (int)std::min(kPlanTailRounds, std::max<uint32_t>(longest, kTailRounds));
+        if ((rc = c->ws[2].ensure((size_t)nseg * sizeof(SegDesc))) != 0) return rc;
+        if ((rc = c->ws[3].ensure((size_t)nseg * sizeof(SegResult))) != 0) return rc;
+        if ((rc = c->ws[4].ensure((size_t)sym * 2 + 64)) != 0) return rc;
+        if ((rc = c->ws[6].ensure((size_t)nseg * 4 + 64)) != 0) return rc;
+        SegDesc* d_segs = c->ws[2].as<SegDesc>();
+        SegResult* d_res = c->ws[3].as<SegResult>();
+        ZB_CUDA(cudaMemsetAsync(d_err, 0, 4, s));
+        ZB_CUDA(cudaMemcpyAsync(d_segs, segs.data(), (size_t)nseg * sizeof(SegDesc), cudaMemcpyHostToDevice, s));
+        if ((rc = launch_segment_phase(d_src, src_len, d_dst, d_segs, nseg, c->ws[4].as<uint16_t>(), d_res, c->ws[6].as<uint32_t>(), d_err,
+                                       d_first_open, 0, nseg, s, rounds)) != 0) return rc;
+        res.resize(nseg);
+        ZB_CUDA(cudaMemcpyAsync(res.data(), d_res, (size_t)nseg * sizeof(SegResult), cudaMemcpyDeviceToHost, s));
+        ZB_CUDA(cudaStreamSynchronize(s));
+        // The window-error count of the tail and rest kernels is not consulted, and each stream is judged by its own
+        // segments: a stream whose segments all pass holds no window symbol in its first segment (seg_decode refuses them
+        // there) and starts every other segment ZB200_CHUNK or more into its own output, so none of its window references
+        // reaches in front of that output; a segment that failed wrote zeros where it stopped (seg_decode), so one damaged
+        // or foreign member neither reads outside its slot nor takes the other members of its group off the plan.
+        for (size_t i = g0; i < g1; i++) {
+            bool good = true;
+            for (uint32_t j = seg0[i - g0]; j < seg0[i - g0 + 1] && good; j++) {
+                const SegResult& r = res[j];
+                good = r.status == 0 && r.out_len == segs[j].out_len;
+                if (good && (segs[j].flags & kSegLast)) good = r.final != 0 && r.end_bit <= 8 * ps[i].in_end;
+            }
+            ok[i] = good ? 1 : 0;
+        }
+        g0 = g1;
+    }
     return 0;
 }
 

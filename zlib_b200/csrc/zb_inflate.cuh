@@ -37,4 +37,23 @@ struct InfCallResult {                 // written by the streaming kernel
     int32_t  status, msg;
 };
 
+// ---- entry points for the ZIP reader (zb_zip.cu) ----
+// k_inflate_batch over a subset of members: stream k of the launch is member ids[k], which occupies d_src[d_beg[i] ..
+// d_end[i]) and decodes (raw deflate) into d_dst[d_dst_beg[i] .. d_dst_end[i]); d_dst_len / d_status are indexed by member.
+int inflate_members_launch(const uint8_t* d_src, const uint64_t* d_beg, const uint64_t* d_end, uint8_t* d_dst, const uint64_t* d_dst_beg,
+                           const uint64_t* d_dst_end, const uint32_t* d_ids, size_t nids, uint64_t* d_dst_len, int32_t* d_status,
+                           cudaStream_t s);
+// The one-stream segment decoder (counting pass, then the block finder): 0 = decoded, 1 = declined, negative = CUDA error.
+int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_dst, uint64_t cap, int wrap,
+                            uint64_t* out_len, int32_t* status, cudaStream_t s, uint64_t* in_used = nullptr, uint32_t* adler = nullptr,
+                            int* wrap_found = nullptr, void* h_dst = nullptr);
+// A raw stream at d_src[in_beg .. in_end) whose output is exactly out_len bytes at d_dst + out_off, with nmarks sync markers:
+// marks[first_mark ..] are the byte positions right behind them, ascending.
+struct PlannedStream { uint64_t in_beg, in_end, out_off, out_len; uint32_t first_mark, nmarks; };
+// Segment decode of all of them together; ok[i] = 1 where stream i came out exactly as planned.
+int inflate_planned(Ctx* c, const uint8_t* d_src, uint64_t src_len, uint8_t* d_dst, const PlannedStream* ps, size_t np,
+                    const uint64_t* marks, uint8_t* ok, cudaStream_t s);
+// k_find_markers: every 00 00 FF FF in d_src[first .. last) -> pos[] (the byte behind it), count in *d_count.
+int find_markers_launch(const uint8_t* d_src, uint64_t first, uint64_t last, uint32_t* d_count, uint64_t* d_pos, uint32_t cap, cudaStream_t s);
+
 }  // namespace zb

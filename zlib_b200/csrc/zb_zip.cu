@@ -12,9 +12,20 @@
 // A *segment* is the run of [local header | name | data] records of some members; segments built on different GPUs
 // concatenate (BASELINE config 5: files are dealt to the ranks, the root appends the central directory).
 // ZIP32 only: at most 65535 members and 4 GiB - 1 for every size and offset; larger inputs are refused.
+//
+// Reading (zb200_zip_list / zb200_zip_extract) is the reverse: the central directory is parsed on the host (unzOpen,
+// unzip.c), then every member is decoded in one pass over the archive on the device instead of unzOpenCurrentFile /
+// unzReadCurrentFile member by member.  k_zip_locate checks every local header against the directory at once; stored
+// members are copied by k_zip_gather, short deflated members share one k_inflate_batch launch (a warp each), and the long
+// ones -- which a warp would decode at ~15 MB/s -- are cut at their sync markers into 128 KiB segments planned from the
+// lengths the directory states and decoded all together by the segment kernels of zb_inflate.cu.  CRC-32 and length of
+// every member are checked on the device.
 #include "zb_common.cuh"
+#include "zb_deflate.cuh"
+#include "zb_inflate.cuh"
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
 #include <vector>
 
 namespace zb {
@@ -53,6 +64,57 @@ __global__ void __launch_bounds__(kGatherThreads) k_zip_gather(const Piece* __re
 
 static void put16(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); }
 static void put32(uint8_t* p, uint64_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24); }
+__host__ __device__ static inline uint32_t get16(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
+__host__ __device__ static inline uint32_t get32(const uint8_t* p) { return get16(p) | (get16(p + 2) << 16); }
+
+// ---- reading ----
+enum { kZipSkip = 0, kZipStored = 1, kZipDeflated = 2 };        // where a member goes once its local header is checked
+struct ZipLoc { uint64_t data_off; int32_t route, status; };    // 16 bytes per member, read back once
+
+// One thread per member: the local header, byte by byte (headers sit at any alignment), against the directory the way
+// unzlocal_CheckCurrentFileCoherencyHeader does it (unzip.c:963-1047): signature, method, name length, and CRC-32 and
+// sizes unless the local header's bit 3 says they follow the data.  The data start from the LOCAL name and extra lengths.
+__global__ void k_zip_locate(const uint8_t* __restrict__ arc, uint64_t arc_len, const zb200_zip_entry* __restrict__ ent,
+                             const uint64_t* __restrict__ dst_off, uint32_t n, ZipLoc* __restrict__ loc)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const zb200_zip_entry e = ent[i];
+    ZipLoc r{0, kZipSkip, ZB_OK};
+    const uint64_t lo = e.local_off;
+    if (lo > arc_len || arc_len - lo < 30) r.status = ZB200_UNZ_BADZIPFILE;
+    else {
+        const uint8_t* h = arc + lo;
+        const uint32_t lflags = get16(h + 6);
+        if (get32(h) != 0x04034b50u || get16(h + 8) != e.method || get16(h + 26) != e.name_len) r.status = ZB200_UNZ_BADZIPFILE;
+        else if (e.method != 0 && e.method != 8) r.status = ZB200_UNZ_BADZIPFILE;
+        else if (!(lflags & 8) && (get32(h + 14) != e.crc32 || get32(h + 18) != e.comp_len || get32(h + 22) != e.raw_len))
+            r.status = ZB200_UNZ_BADZIPFILE;
+        else {
+            r.data_off = lo + 30 + get16(h + 26) + get16(h + 28);
+            if (e.flags & 1) r.status = ZB_STREAM_ERROR;                              // encrypted
+            else if (e.method == 0 && e.comp_len != e.raw_len) r.status = ZB200_UNZ_BADZIPFILE;
+            else if (r.data_off > arc_len || arc_len - r.data_off < e.comp_len) r.status = ZB200_UNZ_BADZIPFILE;
+            else if (dst_off[i + 1] - dst_off[i] < e.raw_len) r.status = ZB_BUF_ERROR;
+            else r.route = e.method == 0 ? kZipStored : kZipDeflated;
+        }
+    }
+    loc[i] = r;
+}
+
+// The last word on every member that reached a decoder: any decoder failure is invalid data, then the length, then the
+// CRC-32 (crc[slot[i]], computed from the output) against the directory.
+__global__ void k_zip_verdict(const zb200_zip_entry* __restrict__ ent, const ZipLoc* __restrict__ loc, const uint32_t* __restrict__ crc,
+                              const uint32_t* __restrict__ slot, const uint64_t* __restrict__ len, int32_t* __restrict__ status, uint32_t n)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || loc[i].route == kZipSkip) return;
+    int32_t st = status[i];
+    if (st != ZB_OK) st = ZB_DATA_ERROR;                        // (the batch's Z_BUF_ERROR: more output than raw_len)
+    else if (len[i] != ent[i].raw_len) st = ZB_DATA_ERROR;
+    else if (crc[slot[i]] != ent[i].crc32) st = ZB200_UNZ_CRCERROR;
+    status[i] = st;
+}
 
 }  // namespace zb
 
@@ -207,4 +269,281 @@ ZB_API int zb200_zip_build(const char* const* names, const void* src, const uint
     if ((rc = zb200_zip_directory(names, members.data(), n, dos_datetime, seg, (uint8_t*)dst + seg, &dl)) != 0) return rc;
     *dst_len = seg + dl;
     return 0;
+}
+
+// ---- reading: the central directory (unzOpen2, unzip.c:380-491) ----
+// The end record is searched back from the end through at most 65535 bytes of comment; byte_before_the_zipfile (bytes in
+// front of the archive: a self-extractor stub, concatenated data) is where the directory really starts minus where the
+// end record says it starts, and is added to every offset.  ZIP64 and multi-disk archives are refused as the writer
+// refuses them.  A device archive has its tail and then its directory copied to the host.
+ZB_API int zb200_zip_list(const void* archive, size_t arc_len, zb200_zip_entry* entries, size_t* n)
+{
+    if (archive == nullptr || n == nullptr || (entries == nullptr && *n != 0)) return ZB_STREAM_ERROR;
+    const bool on_dev = classify(archive) == kDevice;
+    auto fetch = [&](std::vector<uint8_t>& v, uint64_t off, uint64_t len) -> int {
+        v.resize(len);
+        if (!on_dev) { memcpy(v.data(), (const uint8_t*)archive + off, len); return 0; }
+        ZB_CUDA(cudaMemcpy(v.data(), (const uint8_t*)archive + off, len, cudaMemcpyDeviceToHost));
+        return 0;
+    };
+    if (arc_len < 22) { set_error("zb200_zip_list: %zu bytes hold no end record", arc_len); return ZB_STREAM_ERROR; }
+    const uint64_t tail_len = std::min<uint64_t>(arc_len, 22 + 0xffff + 20);
+    const uint64_t tail_at = arc_len - tail_len;
+    std::vector<uint8_t> tail, cd;
+    int rc = fetch(tail, tail_at, tail_len);
+    if (rc) return rc;
+    int64_t e = -1;
+    for (int64_t p = (int64_t)tail_len - 22; p >= 0 && e < 0; p--)
+        if (get32(&tail[p]) == 0x06054b50u && (uint64_t)p + 22 + get16(&tail[p + 20]) <= tail_len) e = p;
+    if (e < 0) { set_error("zb200_zip_list: no end of central directory record"); return ZB_STREAM_ERROR; }
+    const uint8_t* er = &tail[e];
+    const uint64_t end_pos = tail_at + (uint64_t)e;
+    const uint32_t disk = get16(er + 4), cd_disk = get16(er + 6), n_here = get16(er + 8), n_all = get16(er + 10);
+    const uint64_t cd_size = get32(er + 12), cd_off = get32(er + 16);
+    if (e >= 20 && get32(er - 20) == 0x07064b50u) { set_error("zb200_zip_list: ZIP64 archive"); return ZB_STREAM_ERROR; }
+    if (disk != 0 || cd_disk != 0 || n_here != n_all) { set_error("zb200_zip_list: multi-disk archive"); return ZB_STREAM_ERROR; }
+    if (n_all == 0xffffu || cd_size == 0xffffffffull || cd_off == 0xffffffffull) { set_error("zb200_zip_list: ZIP64 archive"); return ZB_STREAM_ERROR; }
+    if (end_pos < cd_off + cd_size) { set_error("zb200_zip_list: central directory outside the archive"); return ZB_STREAM_ERROR; }
+    const uint64_t before = end_pos - (cd_off + cd_size);      // byte_before_the_zipfile
+    if (n_all > *n) { *n = n_all; set_error("zb200_zip_list: %u members, room for fewer", n_all); return ZB_BUF_ERROR; }
+    if ((rc = fetch(cd, before + cd_off, cd_size)) != 0) return rc;
+    uint64_t p = 0;
+    for (uint32_t i = 0; i < n_all; i++) {
+        if (p + 46 > cd_size || get32(&cd[p]) != 0x02014b50u) { set_error("zb200_zip_list: directory record %u is damaged", i); return ZB_STREAM_ERROR; }
+        const uint8_t* h = &cd[p];
+        const uint32_t nl = get16(h + 28), xl = get16(h + 30), cl = get16(h + 32);
+        if (p + 46 + nl + xl + cl > cd_size) { set_error("zb200_zip_list: directory record %u is truncated", i); return ZB_STREAM_ERROR; }
+        zb200_zip_entry& z = entries[i];
+        z.crc32 = get32(h + 16);
+        z.comp_len = get32(h + 20); z.raw_len = get32(h + 24); z.local_off = get32(h + 42);
+        if (z.comp_len == 0xffffffffull || z.raw_len == 0xffffffffull || z.local_off == 0xffffffffull || get16(h + 34) == 0xffffu) {
+            set_error("zb200_zip_list: member %u needs ZIP64", i);
+            return ZB_STREAM_ERROR;
+        }
+        z.local_off += before;
+        z.name_off = before + cd_off + p + 46;
+        z.method = (uint16_t)get16(h + 10); z.flags = (uint16_t)get16(h + 8);
+        z.name_len = (uint16_t)nl; z.reserved16 = 0; z.reserved32 = 0;
+        p += 46 + nl + xl + cl;
+    }
+    *n = n_all;
+    return 0;
+}
+
+// ---- reading: the members ----
+constexpr uint64_t kZipShortMax = ZB200_CHUNK;                  // members with at most one chunk of output: a warp each in the batch
+
+ZB_API int zb200_zip_extract(const void* archive, size_t arc_len, const zb200_zip_entry* entries, size_t n, void* dst,
+                             const uint64_t* dst_off, uint64_t* dst_len, int32_t* status, void* stream)
+{
+    int rc = ensure_init();
+    if (rc) return rc;
+    if (n == 0) return 0;
+    if (archive == nullptr || entries == nullptr || dst == nullptr || dst_off == nullptr || dst_len == nullptr || status == nullptr ||
+        n > 0xffffffffu) {
+        set_error("zb200_zip_extract: bad argument");
+        return ZB_STREAM_ERROR;
+    }
+    for (size_t i = 0; i < n; i++)
+        if (dst_off[i + 1] < dst_off[i]) { set_error("zb200_zip_extract: dst_off must not decrease"); return ZB_STREAM_ERROR; }
+    const uint32_t nn = (uint32_t)n;
+    const uint64_t dst_base = dst_off[0], dst_span = dst_off[n] - dst_off[0];   // the slots: nothing outside them is touched
+    Ctx* c = ctx_acquire((cudaStream_t)stream);
+    if (!c) return ZB_MEM_ERROR;
+    cudaStream_t s = pick_stream(c, stream);
+    do {
+        const uint8_t* d_arc = to_device(c, archive, arc_len, s, &rc);
+        if (rc) break;
+        const bool dst_on_host = classify(dst) != kDevice;
+        uint8_t* d_dst = (uint8_t*)dst;
+        if (dst_on_host) {                                      // staged: only the span of the slots, d_dst[dst_off[0]] is its first byte
+            if ((rc = c->out.ensure(dst_span + 16)) != 0) break;
+            d_dst = c->out.as<uint8_t>() - dst_base;
+        }
+        // per-member tables: [entries][dst_off n+1][loc] | [len][status, 8 bytes each][beg][end][dst beg][dst end][crc off][crc len]
+        // [slot][ids] | [crc][adler]
+        const size_t tab = n * sizeof(zb200_zip_entry) + (n + 1) * 8 + n * sizeof(ZipLoc), per = 8 * 8 + 4 * 4;
+        if ((rc = c->ws[7].ensure(tab + n * per + 64)) != 0) break;
+        uint8_t* w = c->ws[7].as<uint8_t>();
+        zb200_zip_entry* d_ent = (zb200_zip_entry*)w;
+        uint64_t* d_doff = (uint64_t*)(w + n * sizeof(zb200_zip_entry));
+        ZipLoc* d_loc = (ZipLoc*)(d_doff + n + 1);
+        uint8_t* up = (uint8_t*)(d_loc + n);                    // everything from here on is uploaded in one piece after the routing
+        uint64_t* d_len = (uint64_t*)up;
+        int32_t* d_st = (int32_t*)(d_len + n);                  // right behind the lengths: the results come back in one copy
+        uint64_t* d_beg = d_len + 2 * n;
+        uint64_t* d_end = d_beg + n;
+        uint64_t* d_dbeg = d_end + n;
+        uint64_t* d_dend = d_dbeg + n;
+        uint64_t* d_coff = d_dend + n;
+        uint64_t* d_clen = d_coff + n;
+        uint32_t* d_slot = (uint32_t*)(d_clen + n);
+        uint32_t* d_ids = d_slot + n;
+        uint32_t* d_crc = d_ids + n;
+        uint32_t* d_adl = d_crc + n;
+        const size_t up_bytes = (size_t)((uint8_t*)d_crc - up);
+        cudaError_t e = cudaMemcpyAsync(d_ent, entries, n * sizeof(zb200_zip_entry), cudaMemcpyHostToDevice, s);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d_doff, dst_off, (n + 1) * 8, cudaMemcpyHostToDevice, s);
+        if (e != cudaSuccess) { set_error("zb200_zip_extract: table upload failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+        ZB_LAUNCH(k_zip_locate, (nn + 255) / 256, 256, 0, s, d_arc, (uint64_t)arc_len, d_ent, d_doff, nn, d_loc);
+        std::vector<ZipLoc> loc(n);
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaMemcpyAsync(loc.data(), d_loc, n * sizeof(ZipLoc), cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) { set_error("zb200_zip_extract: locate failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+
+        // ---- routes ----
+        std::vector<uint8_t> hup(up_bytes, 0);
+        uint64_t* h_len = (uint64_t*)hup.data();
+        int32_t* h_st = (int32_t*)(h_len + n);
+        uint64_t* h_beg = h_len + 2 * n;
+        uint64_t* h_end = h_beg + n;
+        uint64_t* h_dbeg = h_end + n;
+        uint64_t* h_dend = h_dbeg + n;
+        uint64_t* h_coff = h_dend + n;
+        uint64_t* h_clen = h_coff + n;
+        uint32_t* h_slot = (uint32_t*)(h_clen + n);
+        uint32_t* h_ids = h_slot + n;
+        std::vector<Piece> pieces;
+        std::vector<uint32_t> large, batch, one_crc, chunk_crc;  // members by route; CRC by one CTA / by chunks
+        for (uint32_t i = 0; i < nn; i++) {
+            const zb200_zip_entry& z = entries[i];
+            h_st[i] = loc[i].status;
+            h_beg[i] = loc[i].data_off; h_end[i] = loc[i].data_off + z.comp_len;
+            h_dbeg[i] = dst_off[i]; h_dend[i] = dst_off[i] + z.raw_len;
+            if (loc[i].route == kZipStored) {
+                for (uint64_t o = 0; o < z.raw_len; o += kPieceBytes)
+                    pieces.push_back(Piece{d_arc + loc[i].data_off + o, d_dst + dst_off[i] + o, std::min<uint64_t>(kPieceBytes, z.raw_len - o)});
+                h_len[i] = z.raw_len;
+                one_crc.push_back(i);
+            } else if (loc[i].route == kZipDeflated) {
+                if (z.raw_len > kZipShortMax) large.push_back(i); else batch.push_back(i);
+            }
+        }
+        // ---- long members: markers in their data, then the planned segment decode of all that fit the plan ----
+        std::vector<uint32_t> fallback;
+        if (!large.empty()) {
+            std::sort(large.begin(), large.end(), [&](uint32_t a, uint32_t b) { return loc[a].data_off < loc[b].data_off; });
+            uint64_t lo = ~0ull, hi = 0;
+            for (uint32_t i : large) { lo = std::min(lo, h_beg[i]); hi = std::max(hi, h_end[i]); }
+            const uint32_t cap = (uint32_t)std::min<uint64_t>((hi - lo) / 32 + 4096, 1u << 26);
+            if ((rc = c->small.ensure(256)) != 0) break;
+            if ((rc = c->ws[9].ensure((size_t)cap * 8 + 64)) != 0) break;
+            uint32_t* d_count = c->small.as<uint32_t>() + 24;
+            uint32_t nmark = 0;
+            std::vector<uint64_t> mk;
+            e = cudaMemsetAsync(d_count, 0, 4, s);
+            if (e == cudaSuccess && (rc = find_markers_launch(d_arc, lo, hi, d_count, c->ws[9].as<uint64_t>(), cap, s)) != 0) break;
+            if (e == cudaSuccess) e = cudaMemcpyAsync(&nmark, d_count, 4, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+            if (e == cudaSuccess && nmark <= cap && nmark) {
+                mk.resize(nmark);
+                e = cudaMemcpyAsync(mk.data(), c->ws[9].p, (size_t)nmark * 8, cudaMemcpyDeviceToHost, s);
+                if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+                std::sort(mk.begin(), mk.end());
+            }
+            if (e != cudaSuccess) { set_error("zb200_zip_extract: marker search failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+            std::vector<PlannedStream> plan;
+            std::vector<uint64_t> marks;
+            std::vector<uint32_t> planned;
+            for (uint32_t i : large) {
+                // a marker ends a chunk and the next one starts behind it: strictly inside the member's data
+                const auto a = std::upper_bound(mk.begin(), mk.end(), h_beg[i]), b = std::lower_bound(mk.begin(), mk.end(), h_end[i]);
+                const uint64_t have = (uint64_t)(b - a), want = (entries[i].raw_len + ZB200_CHUNK - 1) / ZB200_CHUNK - 1;
+                if (nmark > cap || have != want) { fallback.push_back(i); continue; }
+                plan.push_back(PlannedStream{h_beg[i], h_end[i], dst_off[i], entries[i].raw_len, (uint32_t)marks.size(), (uint32_t)have});
+                marks.insert(marks.end(), a, b);
+                planned.push_back(i);
+            }
+            std::vector<uint8_t> ok(plan.size(), 0);
+            if (!plan.empty() && (rc = inflate_planned(c, d_arc, arc_len, d_dst, plan.data(), plan.size(), marks.data(), ok.data(), s)) != 0) break;
+            for (size_t k = 0; k < planned.size(); k++) {
+                if (ok[k]) { h_len[planned[k]] = entries[planned[k]].raw_len; chunk_crc.push_back(planned[k]); }
+                else fallback.push_back(planned[k]);
+            }
+            // ---- what does not fit the plan: the one-stream decoder (counting pass, block finder), else the batch ----
+            for (uint32_t i : fallback) {
+                uint64_t got = 0;
+                int32_t st = ZB_OK;
+                const int pr = inflate_single_parallel(c, d_arc + h_beg[i], entries[i].comp_len, d_dst + dst_off[i], entries[i].raw_len,
+                                                       ZB200_WRAP_RAW, &got, &st, s);
+                if (pr < 0) { rc = pr; break; }
+                if (pr == 0) { h_len[i] = got; h_st[i] = st; chunk_crc.push_back(i); }
+                else batch.push_back(i);
+            }
+            if (rc) break;
+        }
+        // ---- short members (and declined long ones): one batch launch; stored members: one gather launch ----
+        for (size_t k = 0; k < batch.size(); k++) { h_ids[k] = batch[k]; one_crc.push_back(batch[k]); }
+        for (size_t k = 0; k < one_crc.size(); k++) { h_slot[one_crc[k]] = (uint32_t)k; h_coff[k] = dst_off[one_crc[k]]; h_clen[k] = entries[one_crc[k]].raw_len; }
+        // long members by output position (ChunkDesc positions are 32-bit: one checksum launch per window below 4 GiB)
+        std::sort(chunk_crc.begin(), chunk_crc.end(), [&](uint32_t a, uint32_t b) { return dst_off[a] < dst_off[b]; });
+        for (size_t k = 0; k < chunk_crc.size(); k++) h_slot[chunk_crc[k]] = (uint32_t)(one_crc.size() + k);
+        e = cudaMemcpyAsync(up, hup.data(), up_bytes, cudaMemcpyHostToDevice, s);
+        if (e == cudaSuccess && !pieces.empty()) {
+            if ((rc = c->ws[10].ensure(pieces.size() * sizeof(Piece))) != 0) break;
+            e = cudaMemcpyAsync(c->ws[10].p, pieces.data(), pieces.size() * sizeof(Piece), cudaMemcpyHostToDevice, s);
+            if (e == cudaSuccess) ZB_LAUNCH(k_zip_gather, (unsigned)pieces.size(), kGatherThreads, 0, s, c->ws[10].as<const Piece>());
+        }
+        if (e != cudaSuccess) { set_error("zb200_zip_extract: upload failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+        if ((rc = inflate_members_launch(d_arc, d_beg, d_end, d_dst, d_dbeg, d_dend, d_ids, batch.size(), d_len, d_st, s)) != 0) break;
+        // ---- CRC-32 of every decoded member: one CTA per short member, per 128 KiB chunk (joined) for long ones ----
+        if ((rc = checksum_batch_launch(d_dst, d_coff, d_clen, one_crc.size(), d_crc, d_adl, nullptr, nullptr, s)) != 0) break;
+        if (!chunk_crc.empty()) {
+            std::vector<ChunkDesc> cd;
+            std::vector<JobDesc> jobs;
+            for (size_t k0 = 0; k0 < chunk_crc.size() && !rc;) {
+                const uint64_t base = dst_off[chunk_crc[k0]];
+                size_t k1 = k0;
+                cd.clear(); jobs.clear();
+                // the first member always (one ZIP32 member is below 4 GiB), further ones while the window stays below 3 GiB
+                while (k1 < chunk_crc.size() && (k1 == k0 || dst_off[chunk_crc[k1]] + entries[chunk_crc[k1]].raw_len - base < (3ull << 30))) {
+                    const uint32_t i = chunk_crc[k1];
+                    JobDesc jd{};
+                    jd.first_chunk = (uint32_t)cd.size();
+                    for (uint64_t o = 0; o < entries[i].raw_len; o += ZB200_CHUNK) {
+                        ChunkDesc d{};
+                        d.beg = (uint32_t)(dst_off[i] - base + o);
+                        d.len = (uint32_t)std::min<uint64_t>(ZB200_CHUNK, entries[i].raw_len - o);
+                        cd.push_back(d);
+                    }
+                    jd.nchunks = (uint32_t)cd.size() - jd.first_chunk;
+                    jobs.push_back(jd);
+                    k1++;
+                }
+                const size_t cd_bytes = cd.size() * sizeof(ChunkDesc), jb_bytes = jobs.size() * sizeof(JobDesc);
+                if ((rc = c->ws[8].ensure(cd_bytes + jb_bytes + jobs.size() * 4 + 64)) != 0) break;
+                uint8_t* d8 = c->ws[8].as<uint8_t>();
+                uint32_t* d_jadl = (uint32_t*)(d8 + cd_bytes + jb_bytes);
+                e = cudaMemcpyAsync(d8, cd.data(), cd_bytes, cudaMemcpyHostToDevice, s);
+                if (e == cudaSuccess) e = cudaMemcpyAsync(d8 + cd_bytes, jobs.data(), jb_bytes, cudaMemcpyHostToDevice, s);
+                if (e != cudaSuccess) { set_error("zb200_zip_extract: upload failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+                uint32_t* d_wcrc = d_crc + one_crc.size() + k0;         // this window's slots are consecutive
+                if ((rc = checksum_jobs_launch(c, d_dst + base, (const ChunkDesc*)d8, (uint32_t)cd.size(), (const JobDesc*)(d8 + cd_bytes),
+                                               (uint32_t)jobs.size(), d_wcrc, d_jadl, s)) != 0) break;
+                k0 = k1;
+            }
+            if (rc) break;
+        }
+        ZB_LAUNCH(k_zip_verdict, (nn + 255) / 256, 256, 0, s, d_ent, d_loc, d_crc, d_slot, d_len, d_st, nn);
+        if ((rc = c->ensure_pinned(n * 12 + 16)) != 0) break;
+        uint64_t* p_len = (uint64_t*)c->pinned;
+        int32_t* p_st = (int32_t*)(p_len + n);
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaMemcpyAsync(p_len, d_len, n * 12, cudaMemcpyDeviceToHost, s);
+        uint8_t* h_span = (uint8_t*)dst + dst_base;
+        const bool drain_threads = dst_on_host && dst_span >= HostStager::kMinBytes && classify(dst) == kHostPageable;
+        if (e == cudaSuccess && dst_on_host && !drain_threads && dst_span)
+            e = cudaMemcpyAsync(h_span, d_dst + dst_base, dst_span, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) { set_error("zb200_zip_extract: failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+        if (drain_threads) {
+            HostDrainer drainer;
+            if ((rc = drainer.drain(h_span, d_dst + dst_base, dst_span)) != 0) break;
+        }
+        for (size_t i = 0; i < n; i++) { dst_len[i] = p_len[i]; status[i] = p_st[i]; }
+    } while (0);
+    if (rc) cudaStreamSynchronize(s);
+    ctx_release(c, s);
+    return rc;
 }
