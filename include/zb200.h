@@ -164,6 +164,23 @@ int zb200_zip_list(const void *archive, size_t arc_len, zb200_zip_entry *entries
 int zb200_zip_extract(const void *archive, size_t arc_len, const zb200_zip_entry *entries, size_t n,
                       void *dst, const uint64_t *dst_off, uint64_t *dst_len, int32_t *status, void *stream);
 
+/* ---- gzip files of several members (RFC 1952 2.2: cat a.gz b.gz, gzip append mode, BGZF) ----
+ * zb200_gunzip: gzip FILE -> its content, all members decoded on the GPU (what gzip -d / Python's gzip.decompress return).
+ * src, dst: host or device memory.  *dst_len: in = capacity, out = bytes written; on Z_BUF_ERROR, the sum of the
+ * members' ISIZE fields (exact when every member is below 4 GiB).  *members: out = member count on Z_OK, index of the
+ * first member that failed on Z_DATA_ERROR (zb200_last_error() names it and its byte offset).
+ * Accepted and refused exactly as Python 3.12's gzip.decompress does (zero bytes after a member are skipped, empty input
+ * is zero members; leading zeros, trailing non-zero bytes, truncation, a wrong CRC-32 or ISIZE, a method other than 8
+ * are Z_DATA_ERROR), except that reserved FLG bits and a wrong FHCRC are Z_DATA_ERROR as in zlib's inflate.
+ * inflate(), uncompress() and zb200_inflate_batch still stop at the end of the first member. */
+int zb200_gunzip(const void *src, size_t src_len, void *dst, size_t *dst_len, size_t *members, void *stream);
+
+/* BGZF (SAM/BAM specification 4.1): src cut into 65280-byte blocks (bgzip's BGZF_BLOCK_SIZE), each one independent gzip
+ * member with the 'BC' extra subfield holding BSIZE = member length - 1, followed by the 28-byte BGZF EOF block.
+ * level 0..9 or -1.  src, dst: host or device memory.  *dst_len: in = capacity, out = bytes written. */
+size_t zb200_bgzf_bound(size_t src_len);     /* ceil(src_len / 65280) * 65536 + 28 */
+int    zb200_bgzf_compress(const void *src, size_t src_len, void *dst, size_t *dst_len, int level, void *stream);
+
 /* ---- inflate: n independent streams (qcsrc/uncompr.c:26 uncompress, batched) ----
  * Stream i occupies src[src_off[i] .. src_off[i+1]) and is decoded into
  * dst[dst_off[i] .. dst_off[i+1]).  Per stream: dst_len[i] = bytes produced,

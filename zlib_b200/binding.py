@@ -162,6 +162,9 @@ class Lib:
             "zb200_zip_directory": (C.c_int, [vp, vp, sz, C.c_uint32, C.c_uint64, vp, C.POINTER(sz)]),
             "zb200_zip_list": (C.c_int, [vp, sz, vp, C.POINTER(sz)]),
             "zb200_zip_extract": (C.c_int, [vp, sz, vp, sz, vp, vp, vp, vp, vp]),
+            "zb200_gunzip": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.POINTER(sz), vp]),
+            "zb200_bgzf_bound": (sz, [sz]),
+            "zb200_bgzf_compress": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, vp]),
             "zb200_inflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
             "zb200_inflate_batch_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
             "zb200_multi_devices": (C.c_int, []),
@@ -415,6 +418,44 @@ class Lib:
         else:
             outs = [dst[int(dst_off[i]):int(dst_off[i]) + int(dst_len[i])].tobytes() for i in range(n)]
         return outs, [int(x) for x in status[:n]]
+
+    def _out_like(self, data, n):
+        """An output buffer of n bytes: a CUDA tensor when `data` is one, else numpy."""
+        import numpy as np
+        if hasattr(data, "data_ptr") and getattr(data, "is_cuda", False):
+            import torch
+            return torch.empty(max(n, 1), dtype=torch.uint8, device=data.device)
+        return np.empty(max(n, 1), dtype=np.uint8)
+
+    def gunzip(self, data, stream=None):
+        """zb200_gunzip: every member of a gzip file -> bytes, or a CUDA tensor when `data` is one.  Raises RuntimeError
+        (the library's message names the member) on damaged data.  A first guess of 4x the input is retried once at the
+        size the library reports."""
+        p, keep = _ptr(data)
+        n = _nbytes(data)
+        cap = max(4 * n, 1 << 20)
+        for _ in range(2):
+            out = self._out_like(data, cap)
+            po, keep2 = _ptr(out)
+            ol, cnt = C.c_size_t(cap), C.c_size_t(0)
+            rc = self.dll.zb200_gunzip(p, n, po, C.byref(ol), C.byref(cnt), _stream(stream))
+            if rc != Z_BUF_ERROR:
+                break
+            cap = ol.value
+        self._check(rc, "zb200_gunzip")
+        self.last_members = cnt.value
+        return out[:ol.value] if hasattr(out, "data_ptr") else out[:ol.value].tobytes()
+
+    def bgzf_compress(self, data, level: int = 6, stream=None):
+        """zb200_bgzf_compress -> BGZF bytes, or a CUDA tensor when `data` is one."""
+        p, keep = _ptr(data)
+        n = _nbytes(data)
+        cap = self.dll.zb200_bgzf_bound(n)
+        out = self._out_like(data, cap)
+        po, keep2 = _ptr(out)
+        ol = C.c_size_t(cap)
+        self._check(self.dll.zb200_bgzf_compress(p, n, po, C.byref(ol), level, _stream(stream)), "zb200_bgzf_compress")
+        return out[:ol.value] if hasattr(out, "data_ptr") else out[:ol.value].tobytes()
 
     def inflate_batch(self, streams, caps, wrap: int = WRAP_ZLIB, stream=None):
         """zb200_inflate_batch over a list of bytes objects; returns (outputs, statuses)."""

@@ -1149,12 +1149,17 @@ __global__ void k_frame_jobs(uint8_t* __restrict__ out, const JobDesc* __restric
         const uint8_t g[10] = {31, 139, 8, 0, 0, 0, 0, 0, (uint8_t)(level == 9 ? 2 : (level < 2 || strat >= 2) ? 4 : 0), 3};   // deflate.c:590-593
         for (int i = 0; i < 10; i++) o[i] = g[i];
         hl = 10;
+    } else if (wrap == kWrapBgzf) {                             // htslib's bgzf.c header bytes; BSIZE is known only here
+        const uint8_t g[16] = {31, 139, 8, 4, 0, 0, 0, 0, 0, 255, 6, 0, 'B', 'C', 2, 0};
+        for (int i = 0; i < 16; i++) o[i] = g[i];
+        o[16] = (uint8_t)(total - 1); o[17] = (uint8_t)((total - 1) >> 8);   // total > 65536 is refused by the caller
+        hl = kBgzfHeader;
     }
     if (jd.nchunks == 0) { o[hl] = 3; o[hl + 1] = 0; }
     if (wrap == ZB200_WRAP_ZLIB) {
         uint8_t* t = o + total - 4;
         t[0] = ad >> 24; t[1] = ad >> 16; t[2] = ad >> 8; t[3] = ad;
-    } else if (wrap == ZB200_WRAP_GZIP) {
+    } else if (wrap == ZB200_WRAP_GZIP || wrap == kWrapBgzf) {
         uint8_t* t = o + total - 8;
         for (int i = 0; i < 4; i++) t[i] = cr >> (8 * i);
         for (int i = 0; i < 4; i++) t[4 + i] = (uint8_t)(jd.src_len >> (8 * i));
@@ -1601,8 +1606,8 @@ static int deflate_jobs_launch(Ctx* c, const uint8_t* d_base, uint64_t span, uin
 {
     const LevelCfg& cfg = P.cfg;
     const uint64_t nblocks = (uint64_t)nchunks * kBlocksPerChunk;
-    const uint32_t hdr_len = P.wrap == ZB200_WRAP_ZLIB ? 2 : P.wrap == ZB200_WRAP_GZIP ? 10 : 0;
-    const uint32_t trailer_len = P.wrap == ZB200_WRAP_ZLIB ? 4 : P.wrap == ZB200_WRAP_GZIP ? 8 : 0;
+    const uint32_t hdr_len = P.wrap == ZB200_WRAP_ZLIB ? 2 : P.wrap == ZB200_WRAP_GZIP ? 10 : P.wrap == kWrapBgzf ? kBgzfHeader : 0;
+    const uint32_t trailer_len = P.wrap == ZB200_WRAP_ZLIB ? 4 : (P.wrap == ZB200_WRAP_GZIP || P.wrap == kWrapBgzf) ? 8 : 0;
     int rc;
     if ((rc = c->ws[2].ensure((uint64_t)(nchunks + 1) * sizeof(ChunkMeta))) != 0) return rc;
     ChunkMeta* d_chunks = c->ws[2].as<ChunkMeta>();
@@ -2054,9 +2059,16 @@ ZB_API int zb200_deflate_batch(const void* src, const uint64_t* src_off, size_t 
                                uint64_t* dst_len, uint32_t* crc, uint32_t* adler, int32_t* status, int level, int wrap,
                                void* stream)
 {
+    if (wrap < 0 || wrap > 2) { set_error("zb200_deflate_batch: bad argument"); return ZB_STREAM_ERROR; }
+    return zb::deflate_batch(src, src_off, n, dst, dst_off, dst_len, crc, adler, status, level, wrap, stream);
+}
+
+int zb::deflate_batch(const void* src, const uint64_t* src_off, size_t n, void* dst, const uint64_t* dst_off, uint64_t* dst_len,
+                      uint32_t* crc, uint32_t* adler, int32_t* status, int level, int wrap, void* stream)
+{
     int rc = ensure_init();
     if (rc) return rc;
-    if (level < -1 || level > 9 || wrap < 0 || wrap > 2 || (n && (!src_off || !dst_off || !dst || !dst_len))) {
+    if (level < -1 || level > 9 || (n && (!src_off || !dst_off || !dst || !dst_len))) {
         set_error("zb200_deflate_batch: bad argument");
         return ZB_STREAM_ERROR;
     }

@@ -14,6 +14,15 @@ constexpr uint32_t kHdrWords = 144;              // dynamic-block header, <= 449
 constexpr uint32_t kTooFar = 4096;               // deflate.c:108-110
 constexpr uint32_t kSlabChunks = 888;            // chunks per pipeline slab (2 waves of 3 link CTAs on 148 SMs)
 
+// Job-mode framing beyond the public ZB200_WRAP_* values: a BGZF block (SAM/BAM specification 4.1), a gzip member whose
+// 18-byte header carries the 'BC' extra subfield with BSIZE = member length - 1.  Only zb200_bgzf_compress asks for it.
+constexpr int kWrapBgzf = 4;
+constexpr uint32_t kBgzfHeader = 18;
+
+// zb200_deflate_batch with any job-mode framing, kWrapBgzf included (zb200_deflate_batch itself takes the public ones).
+int deflate_batch(const void* src, const uint64_t* src_off, size_t n, void* dst, const uint64_t* dst_off, uint64_t* dst_len,
+                  uint32_t* crc, uint32_t* adler, int32_t* status, int level, int wrap, void* stream);
+
 // configuration_table of the reference (deflate.c:137-149); kind 0 stored, 1 greedy, 2 lazy
 struct LevelCfg { uint16_t good, lazy, nice, chain; int kind; };
 

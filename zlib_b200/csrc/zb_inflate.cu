@@ -710,7 +710,8 @@ __global__ void __launch_bounds__(kInfWarps * 32)
 k_inflate_batch(const uint8_t* __restrict__ src, const uint64_t* __restrict__ src_off, uint64_t n,
                 uint8_t* __restrict__ dst, const uint64_t* __restrict__ dst_off,
                 uint64_t* __restrict__ dst_len, int32_t* __restrict__ status, int wrap, uint32_t* __restrict__ expect,
-                const uint32_t* __restrict__ ids, const uint64_t* __restrict__ src_end, const uint64_t* __restrict__ dst_end)
+                const uint32_t* __restrict__ ids, const uint64_t* __restrict__ src_end, const uint64_t* __restrict__ dst_end,
+                uint64_t* __restrict__ in_used)
 {
     __shared__ WarpTables s_tab[kInfWarps];
     __shared__ InfState s_state[kInfWarps];
@@ -726,7 +727,7 @@ k_inflate_batch(const uint8_t* __restrict__ src, const uint64_t* __restrict__ sr
     if (lane == 0) st->wrap = wrap;
     __syncwarp();
     const uint64_t a = src_off[i], e = ids ? src_end[i] : src_off[i + 1], oa = dst_off[i], oe = ids ? dst_end[i] : dst_off[i + 1];
-    inflate_warp(src + a, e - a, dst + oa, oe - oa, false, st, &s_tab[warp], &dst_len[i], nullptr, &status[i], nullptr);
+    inflate_warp(src + a, e - a, dst + oa, oe - oa, false, st, &s_tab[warp], &dst_len[i], in_used ? &in_used[i] : nullptr, &status[i], nullptr);
     __syncwarp();
     if (expect && lane == 0) {                                  // gzip members: {crc32, isize, 1} for the check that follows
         const bool gz = (st->flags & kFlagGzipTrailer) != 0;
@@ -754,7 +755,7 @@ int inflate_batch_launch(const uint8_t* d_src, const uint64_t* d_src_off, size_t
     if (gz && !d_expect) { set_error("inflate batch: gzip needs check scratch"); return ZB_STREAM_ERROR; }
     const unsigned blocks = (unsigned)((n + kInfWarps - 1) / kInfWarps);
     ZB_LAUNCH(k_inflate_batch, blocks, kInfWarps * 32, 0, s, d_src, d_src_off, (uint64_t)n, d_dst, d_dst_off, d_dst_len, d_status, wrap,
-              gz ? d_expect : nullptr, (const uint32_t*)nullptr, (const uint64_t*)nullptr, (const uint64_t*)nullptr);
+              gz ? d_expect : nullptr, (const uint32_t*)nullptr, (const uint64_t*)nullptr, (const uint64_t*)nullptr, (uint64_t*)nullptr);
     ZB_CHECK_LAUNCH();
     // gzip trailer (inflate.c:1099-1112): CRC-32 and length of what was produced, for every member that decoded
     if (gz) return checksum_batch_launch(d_dst, d_dst_off, d_dst_len, n, nullptr, nullptr, d_expect, d_status, s);
@@ -763,11 +764,11 @@ int inflate_batch_launch(const uint8_t* d_src, const uint64_t* d_src_off, size_t
 
 int inflate_members_launch(const uint8_t* d_src, const uint64_t* d_beg, const uint64_t* d_end, uint8_t* d_dst, const uint64_t* d_dst_beg,
                            const uint64_t* d_dst_end, const uint32_t* d_ids, size_t nids, uint64_t* d_dst_len, int32_t* d_status,
-                           cudaStream_t s)
+                           cudaStream_t s, uint64_t* d_in_used)
 {
     if (nids == 0) return 0;
     ZB_LAUNCH(k_inflate_batch, (unsigned)((nids + kInfWarps - 1) / kInfWarps), kInfWarps * 32, 0, s, d_src, d_beg, (uint64_t)nids, d_dst,
-              d_dst_beg, d_dst_len, d_status, (int)ZB200_WRAP_RAW, (uint32_t*)nullptr, d_ids, d_end, d_dst_end);
+              d_dst_beg, d_dst_len, d_status, (int)ZB200_WRAP_RAW, (uint32_t*)nullptr, d_ids, d_end, d_dst_end, d_in_used);
     ZB_CHECK_LAUNCH();
     return 0;
 }
@@ -1506,7 +1507,7 @@ static int emit_segments(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_
 // (no usable boundaries, output that does not fit, damaged data), negative on CUDA errors.
 int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_dst, uint64_t cap, int wrap,
                             uint64_t* out_len, int32_t* status, cudaStream_t s, uint64_t* in_used, uint32_t* adler,
-                            int* wrap_found, void* h_dst)
+                            int* wrap_found, void* h_dst, uint64_t* need)
 {
     if (len < kParMinInput || wrap < 0 || wrap > kWrapAuto) return 1;
     uint64_t hdr = 0;
@@ -1629,7 +1630,10 @@ int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t*
         if (segs.size() < 2) segs.clear();                      // nothing gained; try the other source
     }
     if (segs.empty()) return 1;
-    if (total > cap) return 1;                                  // the serial decoder reports Z_BUF_ERROR the reference's way
+    if (total > cap) {                                          // the serial decoder reports Z_BUF_ERROR the reference's way
+        if (need) *need = total;
+        return 1;
+    }
     uint64_t used = 0;
     uint32_t check = 1;
     rc = emit_segments(c, d_src, len, d_dst, segs, total, final_end, false, wrap, s, h_dst, &total, &used, &check);
@@ -1665,7 +1669,7 @@ int find_markers_launch(const uint8_t* d_src, uint64_t first, uint64_t last, uin
 }
 
 int inflate_planned(Ctx* c, const uint8_t* d_src, uint64_t src_len, uint8_t* d_dst, const PlannedStream* ps, size_t np,
-                    const uint64_t* marks, uint8_t* ok, cudaStream_t s)
+                    const uint64_t* marks, uint8_t* ok, cudaStream_t s, bool exact_end)
 {
     int rc;
     if ((rc = c->small.ensure(256)) != 0) return rc;
@@ -1726,7 +1730,8 @@ int inflate_planned(Ctx* c, const uint8_t* d_src, uint64_t src_len, uint8_t* d_d
             for (uint32_t j = seg0[i - g0]; j < seg0[i - g0 + 1] && good; j++) {
                 const SegResult& r = res[j];
                 good = r.status == 0 && r.out_len == segs[j].out_len;
-                if (good && (segs[j].flags & kSegLast)) good = r.final != 0 && r.end_bit <= 8 * ps[i].in_end;
+                if (good && (segs[j].flags & kSegLast))
+                    good = r.final != 0 && (exact_end ? (r.end_bit + 7) / 8 == ps[i].in_end : r.end_bit <= 8 * ps[i].in_end);
             }
             ok[i] = good ? 1 : 0;
         }

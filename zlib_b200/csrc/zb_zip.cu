@@ -30,8 +30,6 @@
 
 namespace zb {
 
-struct Piece { const uint8_t* src; uint8_t* dst; uint64_t len; };
-constexpr uint32_t kPieceBytes = 256u << 10;
 constexpr int kGatherThreads = 256;
 
 // One CTA per piece: dst-aligned 4-byte stores fed by two aligned loads and a funnel shift (source and destination
@@ -67,8 +65,15 @@ static void put32(uint8_t* p, uint64_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(
 __host__ __device__ static inline uint32_t get16(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
 __host__ __device__ static inline uint32_t get32(const uint8_t* p) { return get16(p) | (get16(p + 2) << 16); }
 
+int gather_launch(const Piece* d_pieces, size_t n, cudaStream_t s)
+{
+    if (n == 0) return 0;
+    ZB_LAUNCH(k_zip_gather, (unsigned)n, kGatherThreads, 0, s, d_pieces);
+    ZB_CHECK_LAUNCH();
+    return 0;
+}
+
 // ---- reading ----
-enum { kZipSkip = 0, kZipStored = 1, kZipDeflated = 2 };        // where a member goes once its local header is checked
 struct ZipLoc { uint64_t data_off; int32_t route, status; };    // 16 bytes per member, read back once
 
 // One thread per member: the local header, byte by byte (headers sit at any alignment), against the directory the way
@@ -80,7 +85,7 @@ __global__ void k_zip_locate(const uint8_t* __restrict__ arc, uint64_t arc_len, 
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const zb200_zip_entry e = ent[i];
-    ZipLoc r{0, kZipSkip, ZB_OK};
+    ZipLoc r{0, kMemberSkip, ZB_OK};
     const uint64_t lo = e.local_off;
     if (lo > arc_len || arc_len - lo < 30) r.status = ZB200_UNZ_BADZIPFILE;
     else {
@@ -96,24 +101,198 @@ __global__ void k_zip_locate(const uint8_t* __restrict__ arc, uint64_t arc_len, 
             else if (e.method == 0 && e.comp_len != e.raw_len) r.status = ZB200_UNZ_BADZIPFILE;
             else if (r.data_off > arc_len || arc_len - r.data_off < e.comp_len) r.status = ZB200_UNZ_BADZIPFILE;
             else if (dst_off[i + 1] - dst_off[i] < e.raw_len) r.status = ZB_BUF_ERROR;
-            else r.route = e.method == 0 ? kZipStored : kZipDeflated;
+            else r.route = e.method == 0 ? kMemberStored : kMemberDeflated;
         }
     }
     loc[i] = r;
 }
 
-// The last word on every member that reached a decoder: any decoder failure is invalid data, then the length, then the
-// CRC-32 (crc[slot[i]], computed from the output) against the directory.
-__global__ void k_zip_verdict(const zb200_zip_entry* __restrict__ ent, const ZipLoc* __restrict__ loc, const uint32_t* __restrict__ crc,
-                              const uint32_t* __restrict__ slot, const uint64_t* __restrict__ len, int32_t* __restrict__ status, uint32_t n)
+// The last word on every member that reached a decoder: any decoder failure is invalid data, then where the data ended
+// (members that must end exactly at their span's end), then the length, then the CRC-32 (crc[slot[i]], computed from the
+// output) against what the container states.
+__global__ void k_zip_verdict(const MemberSpan* __restrict__ m, const uint32_t* __restrict__ crc, const uint32_t* __restrict__ slot,
+                              const uint64_t* __restrict__ len, const uint64_t* __restrict__ used, int32_t* __restrict__ status, uint32_t n)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || loc[i].route == kZipSkip) return;
+    if (i >= n || m[i].route == kMemberSkip) return;
     int32_t st = status[i];
     if (st != ZB_OK) st = ZB_DATA_ERROR;                        // (the batch's Z_BUF_ERROR: more output than raw_len)
-    else if (len[i] != ent[i].raw_len) st = ZB_DATA_ERROR;
-    else if (crc[slot[i]] != ent[i].crc32) st = ZB200_UNZ_CRCERROR;
+    else if (m[i].exact_end && used[i] != m[i].end - m[i].beg) st = ZB_DATA_ERROR;
+    else if (len[i] != m[i].raw_len) st = ZB_DATA_ERROR;
+    else if (crc[slot[i]] != m[i].crc32) st = ZB200_UNZ_CRCERROR;
     status[i] = st;
+}
+
+// ---- the members' routes (shared by zb200_zip_extract and zb200_gunzip) ----
+constexpr uint64_t kShortMember = ZB200_CHUNK;                  // members with at most one chunk of output: a warp each in the batch
+
+int decode_members(Ctx* c, const uint8_t* d_arc, uint64_t arc_len, uint8_t* d_dst, const MemberSpan* m, size_t n, cudaStream_t s)
+{
+    int rc = 0;
+    const uint32_t nn = (uint32_t)n;
+    // per-member tables, uploaded in one piece: [spans] [len][status, 8 bytes each][used][beg][end][dst beg][dst end]
+    // [crc off][crc len] [slot][ids] | written on the device: [crc][adler]
+    const size_t per = sizeof(MemberSpan) + 9 * 8 + 2 * 4;
+    if ((rc = c->ws[7].ensure(n * (per + 8) + 64)) != 0) return rc;
+    uint8_t* up = c->ws[7].as<uint8_t>();
+    MemberSpan* d_m = (MemberSpan*)up;
+    uint64_t* d_len = (uint64_t*)(d_m + n);
+    int32_t* d_st = (int32_t*)(d_len + n);                      // right behind the lengths: the results come back in one copy
+    uint64_t* d_used = d_len + 2 * n;
+    uint64_t* d_beg = d_used + n;
+    uint64_t* d_end = d_beg + n;
+    uint64_t* d_dbeg = d_end + n;
+    uint64_t* d_dend = d_dbeg + n;
+    uint64_t* d_coff = d_dend + n;
+    uint64_t* d_clen = d_coff + n;
+    uint32_t* d_slot = (uint32_t*)(d_clen + n);
+    uint32_t* d_ids = d_slot + n;
+    uint32_t* d_crc = d_ids + n;
+    uint32_t* d_adl = d_crc + n;
+    const size_t up_bytes = (size_t)((uint8_t*)d_crc - up);
+
+    std::vector<uint8_t> hup(up_bytes, 0);
+    memcpy(hup.data(), m, n * sizeof(MemberSpan));
+    uint64_t* h_len = (uint64_t*)(hup.data() + n * sizeof(MemberSpan));
+    int32_t* h_st = (int32_t*)(h_len + n);
+    uint64_t* h_used = h_len + 2 * n;
+    uint64_t* h_beg = h_used + n;
+    uint64_t* h_end = h_beg + n;
+    uint64_t* h_dbeg = h_end + n;
+    uint64_t* h_dend = h_dbeg + n;
+    uint64_t* h_coff = h_dend + n;
+    uint64_t* h_clen = h_coff + n;
+    uint32_t* h_slot = (uint32_t*)(h_clen + n);
+    uint32_t* h_ids = h_slot + n;
+    std::vector<Piece> pieces;
+    std::vector<uint32_t> large, batch, one_crc, chunk_crc;  // members by route; CRC by one CTA / by chunks
+    for (uint32_t i = 0; i < nn; i++) {
+        h_st[i] = m[i].status;
+        h_beg[i] = m[i].beg; h_end[i] = m[i].end;
+        h_dbeg[i] = m[i].dst; h_dend[i] = m[i].dst + m[i].raw_len;
+        if (m[i].route == kMemberStored) {
+            for (uint64_t o = 0; o < m[i].raw_len; o += kPieceBytes)
+                pieces.push_back(Piece{d_arc + m[i].beg + o, d_dst + m[i].dst + o, std::min<uint64_t>(kPieceBytes, m[i].raw_len - o)});
+            h_len[i] = m[i].raw_len;
+            h_used[i] = m[i].end - m[i].beg;
+            one_crc.push_back(i);
+        } else if (m[i].route == kMemberDeflated) {
+            if (m[i].raw_len > kShortMember) large.push_back(i); else batch.push_back(i);
+        }
+    }
+    cudaError_t e = cudaSuccess;
+    // ---- long members: markers in their data, then the planned segment decode of all that fit the plan ----
+    std::vector<uint32_t> fallback;
+    if (!large.empty()) {
+        std::sort(large.begin(), large.end(), [&](uint32_t a, uint32_t b) { return m[a].beg < m[b].beg; });
+        uint64_t lo = ~0ull, hi = 0;
+        for (uint32_t i : large) { lo = std::min(lo, h_beg[i]); hi = std::max(hi, h_end[i]); }
+        const uint32_t cap = (uint32_t)std::min<uint64_t>((hi - lo) / 32 + 4096, 1u << 26);
+        if ((rc = c->small.ensure(256)) != 0) return rc;
+        if ((rc = c->ws[9].ensure((size_t)cap * 8 + 64)) != 0) return rc;
+        uint32_t* d_count = c->small.as<uint32_t>() + 24;
+        uint32_t nmark = 0;
+        std::vector<uint64_t> mk;
+        e = cudaMemsetAsync(d_count, 0, 4, s);
+        if (e == cudaSuccess && (rc = find_markers_launch(d_arc, lo, hi, d_count, c->ws[9].as<uint64_t>(), cap, s)) != 0) return rc;
+        if (e == cudaSuccess) e = cudaMemcpyAsync(&nmark, d_count, 4, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e == cudaSuccess && nmark <= cap && nmark) {
+            mk.resize(nmark);
+            e = cudaMemcpyAsync(mk.data(), c->ws[9].p, (size_t)nmark * 8, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+            std::sort(mk.begin(), mk.end());
+        }
+        if (e != cudaSuccess) { set_error("member decode: marker search failed: %s", cudaGetErrorString(e)); return ZB_STREAM_ERROR; }
+        std::vector<PlannedStream> plan;
+        std::vector<uint64_t> marks;
+        std::vector<uint32_t> planned;
+        bool exact = false;
+        for (uint32_t i : large) {
+            // a marker ends a chunk and the next one starts behind it: strictly inside the member's data
+            const auto a = std::upper_bound(mk.begin(), mk.end(), h_beg[i]), b = std::lower_bound(mk.begin(), mk.end(), h_end[i]);
+            const uint64_t have = (uint64_t)(b - a), want = (m[i].raw_len + ZB200_CHUNK - 1) / ZB200_CHUNK - 1;
+            if (nmark > cap || have != want) { fallback.push_back(i); continue; }
+            plan.push_back(PlannedStream{h_beg[i], h_end[i], m[i].dst, m[i].raw_len, (uint32_t)marks.size(), (uint32_t)have});
+            marks.insert(marks.end(), a, b);
+            planned.push_back(i);
+            exact = exact || m[i].exact_end;                    // one container per call: every member or none
+        }
+        std::vector<uint8_t> ok(plan.size(), 0);
+        if (!plan.empty() && (rc = inflate_planned(c, d_arc, arc_len, d_dst, plan.data(), plan.size(), marks.data(), ok.data(), s, exact)) != 0)
+            return rc;
+        for (size_t k = 0; k < planned.size(); k++) {
+            if (ok[k]) { h_len[planned[k]] = m[planned[k]].raw_len; h_used[planned[k]] = h_end[planned[k]] - h_beg[planned[k]]; chunk_crc.push_back(planned[k]); }
+            else fallback.push_back(planned[k]);
+        }
+        // ---- what does not fit the plan: the one-stream decoder (counting pass, block finder), else the batch ----
+        for (uint32_t i : fallback) {
+            uint64_t got = 0, used = 0;
+            int32_t st = ZB_OK;
+            const int pr = inflate_single_parallel(c, d_arc + h_beg[i], h_end[i] - h_beg[i], d_dst + m[i].dst, m[i].raw_len,
+                                                   ZB200_WRAP_RAW, &got, &st, s, &used);
+            if (pr < 0) return pr;
+            if (pr == 0) { h_len[i] = got; h_st[i] = st; h_used[i] = used; chunk_crc.push_back(i); }
+            else batch.push_back(i);
+        }
+    }
+    // ---- short members (and declined long ones): one batch launch; stored members: one gather launch ----
+    for (size_t k = 0; k < batch.size(); k++) { h_ids[k] = batch[k]; one_crc.push_back(batch[k]); }
+    for (size_t k = 0; k < one_crc.size(); k++) { h_slot[one_crc[k]] = (uint32_t)k; h_coff[k] = m[one_crc[k]].dst; h_clen[k] = m[one_crc[k]].raw_len; }
+    // long members by output position (ChunkDesc positions are 32-bit: one checksum launch per window below 4 GiB)
+    std::sort(chunk_crc.begin(), chunk_crc.end(), [&](uint32_t a, uint32_t b) { return m[a].dst < m[b].dst; });
+    for (size_t k = 0; k < chunk_crc.size(); k++) h_slot[chunk_crc[k]] = (uint32_t)(one_crc.size() + k);
+    e = cudaMemcpyAsync(up, hup.data(), up_bytes, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess && !pieces.empty()) {
+        if ((rc = c->ws[10].ensure(pieces.size() * sizeof(Piece))) != 0) return rc;
+        e = cudaMemcpyAsync(c->ws[10].p, pieces.data(), pieces.size() * sizeof(Piece), cudaMemcpyHostToDevice, s);
+        if (e == cudaSuccess && (rc = gather_launch(c->ws[10].as<const Piece>(), pieces.size(), s)) != 0) return rc;
+    }
+    if (e != cudaSuccess) { set_error("member decode: upload failed: %s", cudaGetErrorString(e)); return ZB_STREAM_ERROR; }
+    if ((rc = inflate_members_launch(d_arc, d_beg, d_end, d_dst, d_dbeg, d_dend, d_ids, batch.size(), d_len, d_st, s, d_used)) != 0) return rc;
+    // ---- CRC-32 of every decoded member: one CTA per short member, per 128 KiB chunk (joined) for long ones ----
+    if ((rc = checksum_batch_launch(d_dst, d_coff, d_clen, one_crc.size(), d_crc, d_adl, nullptr, nullptr, s)) != 0) return rc;
+    if (!chunk_crc.empty()) {
+        std::vector<ChunkDesc> cd;
+        std::vector<JobDesc> jobs;
+        for (size_t k0 = 0; k0 < chunk_crc.size();) {
+            const uint64_t base = m[chunk_crc[k0]].dst;
+            size_t k1 = k0;
+            cd.clear(); jobs.clear();
+            // the first member always (its ChunkDesc positions must stay below 4 GiB), further ones while the window stays below 3 GiB
+            while (k1 < chunk_crc.size() && (k1 == k0 || m[chunk_crc[k1]].dst + m[chunk_crc[k1]].raw_len - base < (3ull << 30))) {
+                const uint32_t i = chunk_crc[k1];
+                JobDesc jd{};
+                jd.first_chunk = (uint32_t)cd.size();
+                for (uint64_t o = 0; o < m[i].raw_len; o += ZB200_CHUNK) {
+                    ChunkDesc d{};
+                    d.beg = (uint32_t)(m[i].dst - base + o);
+                    d.len = (uint32_t)std::min<uint64_t>(ZB200_CHUNK, m[i].raw_len - o);
+                    cd.push_back(d);
+                }
+                jd.nchunks = (uint32_t)cd.size() - jd.first_chunk;
+                jobs.push_back(jd);
+                k1++;
+            }
+            const size_t cd_bytes = cd.size() * sizeof(ChunkDesc), jb_bytes = jobs.size() * sizeof(JobDesc);
+            if ((rc = c->ws[8].ensure(cd_bytes + jb_bytes + jobs.size() * 4 + 64)) != 0) return rc;
+            uint8_t* d8 = c->ws[8].as<uint8_t>();
+            uint32_t* d_jadl = (uint32_t*)(d8 + cd_bytes + jb_bytes);
+            e = cudaMemcpyAsync(d8, cd.data(), cd_bytes, cudaMemcpyHostToDevice, s);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(d8 + cd_bytes, jobs.data(), jb_bytes, cudaMemcpyHostToDevice, s);
+            if (e != cudaSuccess) { set_error("member decode: upload failed: %s", cudaGetErrorString(e)); return ZB_STREAM_ERROR; }
+            uint32_t* d_wcrc = d_crc + one_crc.size() + k0;         // this window's slots are consecutive
+            if ((rc = checksum_jobs_launch(c, d_dst + base, (const ChunkDesc*)d8, (uint32_t)cd.size(), (const JobDesc*)(d8 + cd_bytes),
+                                           (uint32_t)jobs.size(), d_wcrc, d_jadl, s)) != 0) return rc;
+            k0 = k1;
+        }
+    }
+    ZB_LAUNCH(k_zip_verdict, (nn + 255) / 256, 256, 0, s, d_m, d_crc, d_slot, d_len, d_used, d_st, nn);
+    if ((rc = c->ensure_pinned(n * 12 + 16)) != 0) return rc;
+    e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(c->pinned, d_len, n * 12, cudaMemcpyDeviceToHost, s);
+    if (e != cudaSuccess) { set_error("member decode failed: %s", cudaGetErrorString(e)); return ZB_STREAM_ERROR; }
+    return 0;
 }
 
 }  // namespace zb
@@ -331,8 +510,6 @@ ZB_API int zb200_zip_list(const void* archive, size_t arc_len, zb200_zip_entry* 
 }
 
 // ---- reading: the members ----
-constexpr uint64_t kZipShortMax = ZB200_CHUNK;                  // members with at most one chunk of output: a warp each in the batch
-
 ZB_API int zb200_zip_extract(const void* archive, size_t arc_len, const zb200_zip_entry* entries, size_t n, void* dst,
                              const uint64_t* dst_off, uint64_t* dst_len, int32_t* status, void* stream)
 {
@@ -360,28 +537,13 @@ ZB_API int zb200_zip_extract(const void* archive, size_t arc_len, const zb200_zi
             if ((rc = c->out.ensure(dst_span + 16)) != 0) break;
             d_dst = c->out.as<uint8_t>() - dst_base;
         }
-        // per-member tables: [entries][dst_off n+1][loc] | [len][status, 8 bytes each][beg][end][dst beg][dst end][crc off][crc len]
-        // [slot][ids] | [crc][adler]
-        const size_t tab = n * sizeof(zb200_zip_entry) + (n + 1) * 8 + n * sizeof(ZipLoc), per = 8 * 8 + 4 * 4;
-        if ((rc = c->ws[7].ensure(tab + n * per + 64)) != 0) break;
-        uint8_t* w = c->ws[7].as<uint8_t>();
+        // the directory's view of every member, for k_zip_locate (ws[0]: decode_members keeps its tables elsewhere)
+        const size_t tab = n * sizeof(zb200_zip_entry) + (n + 1) * 8 + n * sizeof(ZipLoc);
+        if ((rc = c->ws[0].ensure(tab + 64)) != 0) break;
+        uint8_t* w = c->ws[0].as<uint8_t>();
         zb200_zip_entry* d_ent = (zb200_zip_entry*)w;
         uint64_t* d_doff = (uint64_t*)(w + n * sizeof(zb200_zip_entry));
         ZipLoc* d_loc = (ZipLoc*)(d_doff + n + 1);
-        uint8_t* up = (uint8_t*)(d_loc + n);                    // everything from here on is uploaded in one piece after the routing
-        uint64_t* d_len = (uint64_t*)up;
-        int32_t* d_st = (int32_t*)(d_len + n);                  // right behind the lengths: the results come back in one copy
-        uint64_t* d_beg = d_len + 2 * n;
-        uint64_t* d_end = d_beg + n;
-        uint64_t* d_dbeg = d_end + n;
-        uint64_t* d_dend = d_dbeg + n;
-        uint64_t* d_coff = d_dend + n;
-        uint64_t* d_clen = d_coff + n;
-        uint32_t* d_slot = (uint32_t*)(d_clen + n);
-        uint32_t* d_ids = d_slot + n;
-        uint32_t* d_crc = d_ids + n;
-        uint32_t* d_adl = d_crc + n;
-        const size_t up_bytes = (size_t)((uint8_t*)d_crc - up);
         cudaError_t e = cudaMemcpyAsync(d_ent, entries, n * sizeof(zb200_zip_entry), cudaMemcpyHostToDevice, s);
         if (e == cudaSuccess) e = cudaMemcpyAsync(d_doff, dst_off, (n + 1) * 8, cudaMemcpyHostToDevice, s);
         if (e != cudaSuccess) { set_error("zb200_zip_extract: table upload failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
@@ -391,146 +553,13 @@ ZB_API int zb200_zip_extract(const void* archive, size_t arc_len, const zb200_zi
         if (e == cudaSuccess) e = cudaMemcpyAsync(loc.data(), d_loc, n * sizeof(ZipLoc), cudaMemcpyDeviceToHost, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) { set_error("zb200_zip_extract: locate failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
-
-        // ---- routes ----
-        std::vector<uint8_t> hup(up_bytes, 0);
-        uint64_t* h_len = (uint64_t*)hup.data();
-        int32_t* h_st = (int32_t*)(h_len + n);
-        uint64_t* h_beg = h_len + 2 * n;
-        uint64_t* h_end = h_beg + n;
-        uint64_t* h_dbeg = h_end + n;
-        uint64_t* h_dend = h_dbeg + n;
-        uint64_t* h_coff = h_dend + n;
-        uint64_t* h_clen = h_coff + n;
-        uint32_t* h_slot = (uint32_t*)(h_clen + n);
-        uint32_t* h_ids = h_slot + n;
-        std::vector<Piece> pieces;
-        std::vector<uint32_t> large, batch, one_crc, chunk_crc;  // members by route; CRC by one CTA / by chunks
-        for (uint32_t i = 0; i < nn; i++) {
-            const zb200_zip_entry& z = entries[i];
-            h_st[i] = loc[i].status;
-            h_beg[i] = loc[i].data_off; h_end[i] = loc[i].data_off + z.comp_len;
-            h_dbeg[i] = dst_off[i]; h_dend[i] = dst_off[i] + z.raw_len;
-            if (loc[i].route == kZipStored) {
-                for (uint64_t o = 0; o < z.raw_len; o += kPieceBytes)
-                    pieces.push_back(Piece{d_arc + loc[i].data_off + o, d_dst + dst_off[i] + o, std::min<uint64_t>(kPieceBytes, z.raw_len - o)});
-                h_len[i] = z.raw_len;
-                one_crc.push_back(i);
-            } else if (loc[i].route == kZipDeflated) {
-                if (z.raw_len > kZipShortMax) large.push_back(i); else batch.push_back(i);
-            }
-        }
-        // ---- long members: markers in their data, then the planned segment decode of all that fit the plan ----
-        std::vector<uint32_t> fallback;
-        if (!large.empty()) {
-            std::sort(large.begin(), large.end(), [&](uint32_t a, uint32_t b) { return loc[a].data_off < loc[b].data_off; });
-            uint64_t lo = ~0ull, hi = 0;
-            for (uint32_t i : large) { lo = std::min(lo, h_beg[i]); hi = std::max(hi, h_end[i]); }
-            const uint32_t cap = (uint32_t)std::min<uint64_t>((hi - lo) / 32 + 4096, 1u << 26);
-            if ((rc = c->small.ensure(256)) != 0) break;
-            if ((rc = c->ws[9].ensure((size_t)cap * 8 + 64)) != 0) break;
-            uint32_t* d_count = c->small.as<uint32_t>() + 24;
-            uint32_t nmark = 0;
-            std::vector<uint64_t> mk;
-            e = cudaMemsetAsync(d_count, 0, 4, s);
-            if (e == cudaSuccess && (rc = find_markers_launch(d_arc, lo, hi, d_count, c->ws[9].as<uint64_t>(), cap, s)) != 0) break;
-            if (e == cudaSuccess) e = cudaMemcpyAsync(&nmark, d_count, 4, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            if (e == cudaSuccess && nmark <= cap && nmark) {
-                mk.resize(nmark);
-                e = cudaMemcpyAsync(mk.data(), c->ws[9].p, (size_t)nmark * 8, cudaMemcpyDeviceToHost, s);
-                if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-                std::sort(mk.begin(), mk.end());
-            }
-            if (e != cudaSuccess) { set_error("zb200_zip_extract: marker search failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
-            std::vector<PlannedStream> plan;
-            std::vector<uint64_t> marks;
-            std::vector<uint32_t> planned;
-            for (uint32_t i : large) {
-                // a marker ends a chunk and the next one starts behind it: strictly inside the member's data
-                const auto a = std::upper_bound(mk.begin(), mk.end(), h_beg[i]), b = std::lower_bound(mk.begin(), mk.end(), h_end[i]);
-                const uint64_t have = (uint64_t)(b - a), want = (entries[i].raw_len + ZB200_CHUNK - 1) / ZB200_CHUNK - 1;
-                if (nmark > cap || have != want) { fallback.push_back(i); continue; }
-                plan.push_back(PlannedStream{h_beg[i], h_end[i], dst_off[i], entries[i].raw_len, (uint32_t)marks.size(), (uint32_t)have});
-                marks.insert(marks.end(), a, b);
-                planned.push_back(i);
-            }
-            std::vector<uint8_t> ok(plan.size(), 0);
-            if (!plan.empty() && (rc = inflate_planned(c, d_arc, arc_len, d_dst, plan.data(), plan.size(), marks.data(), ok.data(), s)) != 0) break;
-            for (size_t k = 0; k < planned.size(); k++) {
-                if (ok[k]) { h_len[planned[k]] = entries[planned[k]].raw_len; chunk_crc.push_back(planned[k]); }
-                else fallback.push_back(planned[k]);
-            }
-            // ---- what does not fit the plan: the one-stream decoder (counting pass, block finder), else the batch ----
-            for (uint32_t i : fallback) {
-                uint64_t got = 0;
-                int32_t st = ZB_OK;
-                const int pr = inflate_single_parallel(c, d_arc + h_beg[i], entries[i].comp_len, d_dst + dst_off[i], entries[i].raw_len,
-                                                       ZB200_WRAP_RAW, &got, &st, s);
-                if (pr < 0) { rc = pr; break; }
-                if (pr == 0) { h_len[i] = got; h_st[i] = st; chunk_crc.push_back(i); }
-                else batch.push_back(i);
-            }
-            if (rc) break;
-        }
-        // ---- short members (and declined long ones): one batch launch; stored members: one gather launch ----
-        for (size_t k = 0; k < batch.size(); k++) { h_ids[k] = batch[k]; one_crc.push_back(batch[k]); }
-        for (size_t k = 0; k < one_crc.size(); k++) { h_slot[one_crc[k]] = (uint32_t)k; h_coff[k] = dst_off[one_crc[k]]; h_clen[k] = entries[one_crc[k]].raw_len; }
-        // long members by output position (ChunkDesc positions are 32-bit: one checksum launch per window below 4 GiB)
-        std::sort(chunk_crc.begin(), chunk_crc.end(), [&](uint32_t a, uint32_t b) { return dst_off[a] < dst_off[b]; });
-        for (size_t k = 0; k < chunk_crc.size(); k++) h_slot[chunk_crc[k]] = (uint32_t)(one_crc.size() + k);
-        e = cudaMemcpyAsync(up, hup.data(), up_bytes, cudaMemcpyHostToDevice, s);
-        if (e == cudaSuccess && !pieces.empty()) {
-            if ((rc = c->ws[10].ensure(pieces.size() * sizeof(Piece))) != 0) break;
-            e = cudaMemcpyAsync(c->ws[10].p, pieces.data(), pieces.size() * sizeof(Piece), cudaMemcpyHostToDevice, s);
-            if (e == cudaSuccess) ZB_LAUNCH(k_zip_gather, (unsigned)pieces.size(), kGatherThreads, 0, s, c->ws[10].as<const Piece>());
-        }
-        if (e != cudaSuccess) { set_error("zb200_zip_extract: upload failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
-        if ((rc = inflate_members_launch(d_arc, d_beg, d_end, d_dst, d_dbeg, d_dend, d_ids, batch.size(), d_len, d_st, s)) != 0) break;
-        // ---- CRC-32 of every decoded member: one CTA per short member, per 128 KiB chunk (joined) for long ones ----
-        if ((rc = checksum_batch_launch(d_dst, d_coff, d_clen, one_crc.size(), d_crc, d_adl, nullptr, nullptr, s)) != 0) break;
-        if (!chunk_crc.empty()) {
-            std::vector<ChunkDesc> cd;
-            std::vector<JobDesc> jobs;
-            for (size_t k0 = 0; k0 < chunk_crc.size() && !rc;) {
-                const uint64_t base = dst_off[chunk_crc[k0]];
-                size_t k1 = k0;
-                cd.clear(); jobs.clear();
-                // the first member always (one ZIP32 member is below 4 GiB), further ones while the window stays below 3 GiB
-                while (k1 < chunk_crc.size() && (k1 == k0 || dst_off[chunk_crc[k1]] + entries[chunk_crc[k1]].raw_len - base < (3ull << 30))) {
-                    const uint32_t i = chunk_crc[k1];
-                    JobDesc jd{};
-                    jd.first_chunk = (uint32_t)cd.size();
-                    for (uint64_t o = 0; o < entries[i].raw_len; o += ZB200_CHUNK) {
-                        ChunkDesc d{};
-                        d.beg = (uint32_t)(dst_off[i] - base + o);
-                        d.len = (uint32_t)std::min<uint64_t>(ZB200_CHUNK, entries[i].raw_len - o);
-                        cd.push_back(d);
-                    }
-                    jd.nchunks = (uint32_t)cd.size() - jd.first_chunk;
-                    jobs.push_back(jd);
-                    k1++;
-                }
-                const size_t cd_bytes = cd.size() * sizeof(ChunkDesc), jb_bytes = jobs.size() * sizeof(JobDesc);
-                if ((rc = c->ws[8].ensure(cd_bytes + jb_bytes + jobs.size() * 4 + 64)) != 0) break;
-                uint8_t* d8 = c->ws[8].as<uint8_t>();
-                uint32_t* d_jadl = (uint32_t*)(d8 + cd_bytes + jb_bytes);
-                e = cudaMemcpyAsync(d8, cd.data(), cd_bytes, cudaMemcpyHostToDevice, s);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(d8 + cd_bytes, jobs.data(), jb_bytes, cudaMemcpyHostToDevice, s);
-                if (e != cudaSuccess) { set_error("zb200_zip_extract: upload failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
-                uint32_t* d_wcrc = d_crc + one_crc.size() + k0;         // this window's slots are consecutive
-                if ((rc = checksum_jobs_launch(c, d_dst + base, (const ChunkDesc*)d8, (uint32_t)cd.size(), (const JobDesc*)(d8 + cd_bytes),
-                                               (uint32_t)jobs.size(), d_wcrc, d_jadl, s)) != 0) break;
-                k0 = k1;
-            }
-            if (rc) break;
-        }
-        ZB_LAUNCH(k_zip_verdict, (nn + 255) / 256, 256, 0, s, d_ent, d_loc, d_crc, d_slot, d_len, d_st, nn);
-        if ((rc = c->ensure_pinned(n * 12 + 16)) != 0) break;
+        std::vector<MemberSpan> ms(n);
+        for (size_t i = 0; i < n; i++)
+            ms[i] = MemberSpan{loc[i].data_off, loc[i].data_off + entries[i].comp_len, dst_off[i], entries[i].raw_len, entries[i].crc32,
+                               loc[i].route, loc[i].status, 0};
+        if ((rc = decode_members(c, d_arc, arc_len, d_dst, ms.data(), n, s)) != 0) break;
         uint64_t* p_len = (uint64_t*)c->pinned;
         int32_t* p_st = (int32_t*)(p_len + n);
-        e = cudaGetLastError();
-        if (e == cudaSuccess) e = cudaMemcpyAsync(p_len, d_len, n * 12, cudaMemcpyDeviceToHost, s);
         uint8_t* h_span = (uint8_t*)dst + dst_base;
         const bool drain_threads = dst_on_host && dst_span >= HostStager::kMinBytes && classify(dst) == kHostPageable;
         if (e == cudaSuccess && dst_on_host && !drain_threads && dst_span)
