@@ -28,7 +28,6 @@
 //
 // Roofline: HBM.  Algorithmic bytes = len (read once), 8 bytes written.
 #include "zb_deflate.cuh"
-#include <stdlib.h>
 
 namespace zb {
 
@@ -126,15 +125,10 @@ int checksum_setup()
 // constant (PRMT), instead of extract + scale + add.  The kernel is instruction bound, so this is what moves it.
 // The image itself arrives by TMA: one thread issues two 64 KiB bulk copies (cp.async.bulk, SASS UBLKCP) from the
 // ready-made image in global memory and everybody waits on the mbarrier -- 32 scattered stores per thread before.
-// kTma: the DATA also comes through shared memory -- every warp keeps a private ring of kTmaSlots x 512 bytes that its
-// lane 0 refills with bulk copies (one mbarrier per slot), so the loads leave the instruction stream and registers no
-// longer cap the bytes in flight.  The ring lives in the shared memory the 64 KiB alignment of the image leaves unused.
 // The combine tree runs in the same launch: the last CTA to publish its record folds all of them (see fold_records).
 constexpr uint32_t kPrefetchAhead = 16;                          // iterations (512 B each) between an L2 prefetch and its use
 constexpr uint32_t kTabImage = 2 * 65536;                       // bytes of the table image
-constexpr int kTmaSlots = 5;                                    // 512-byte pieces in flight per warp (kTma)
-constexpr uint32_t kRingLow = 3, kRingHigh = kTmaSlots - kRingLow;   // slots below / above the image (16 KiB per slot and CTA)
-constexpr size_t kMainSmem = 65536 + kTabImage + kRingHigh * 16384;   // 64 KiB of alignment room (hosting the low slots) + image + high slots
+constexpr size_t kMainSmem = 65536 + kTabImage;                 // 64 KiB of alignment room + image
 
 struct FoldArgs {                                               // per-launch constants of the combine, computed on the host
     uint32_t pw_stride[10];                                     // x^(8 * S * 2^k), S = bytes one CTA covers
@@ -150,13 +144,6 @@ __device__ __forceinline__ uint32_t lds32(uint32_t saddr)
 {
     uint32_t v;
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(saddr));
-    return v;
-}
-
-__device__ __forceinline__ uint4 lds128(uint32_t saddr)
-{
-    uint4 v;
-    asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(saddr));
     return v;
 }
 
@@ -300,7 +287,6 @@ __device__ void fold_records(const Partial* __restrict__ parts, uint32_t n_parts
     }
 }
 
-template <bool kTma>
 __global__ void __launch_bounds__(kMainThreads, 1)
 k_checksum_main(const uint8_t* __restrict__ base, uint64_t n_units, uint32_t iters_per_warp,
                 uint64_t base_off, Partial* __restrict__ parts, const uint8_t* __restrict__ buf, uint64_t len,
@@ -308,17 +294,15 @@ k_checksum_main(const uint8_t* __restrict__ base, uint64_t n_units, uint32_t ite
 {
     extern __shared__ __align__(128) uint8_t s_raw[];
     __shared__ Partial s_part[kMainWarps];
-    __shared__ __align__(8) uint64_t s_bar[1 + kMainWarps * kTmaSlots];   // [0] table image, then one per warp and slot
+    __shared__ __align__(8) uint64_t s_bar;                   // the table image has landed
     __shared__ uint32_t s_x[64];
     __shared__ uint32_t s_last;
     const uint32_t raw = (uint32_t)__cvta_generic_to_shared(s_raw);
     const uint32_t img = (raw + 65535u) & ~65535u;              // shared address of the image
-    const uint32_t bar0 = (uint32_t)__cvta_generic_to_shared(s_bar);
+    const uint32_t bar0 = (uint32_t)__cvta_generic_to_shared(&s_bar);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    if (kTma && img - raw < kRingLow * 16384u) __trap();       // the low ring slots live in the alignment room in front of the image
     if (threadIdx.x == 0) {
         mbar_init(bar0, 1);
-        if (kTma) for (int i = 0; i < kMainWarps * kTmaSlots; i++) mbar_init(bar0 + 8 + 8 * i, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         mbar_expect_tx(bar0, kTabImage);
@@ -332,17 +316,6 @@ k_checksum_main(const uint8_t* __restrict__ base, uint64_t n_units, uint32_t ite
     Partial mine{0, 0, 0, 0, 0};
     const uint32_t iters = u0 < n_units ? (uint32_t)min((uint64_t)iters_per_warp, n_units - u0) : 0u;
     const uint8_t* seg = base + u0 * kStride;
-    // ring slot s of this warp: 512 bytes at (slot base) + wid * 512; slots 0..kRingLow-1 below the image, the rest above
-    auto slot_addr = [&](uint32_t sl) -> uint32_t {
-        return (sl < kRingLow ? img - (kRingLow - sl) * 16384u : img + kTabImage + (sl - kRingLow) * 16384u) + (uint32_t)wid * 512u;
-    };
-    const uint32_t wbar = bar0 + 8 + 8 * (uint32_t)(wid * kTmaSlots);
-    if (kTma && lane == 0) {
-        for (uint32_t j = 0; j < (uint32_t)kTmaSlots && j < iters; j++) {
-            mbar_expect_tx(wbar + 8 * j, kStride);
-            bulk_g2s(slot_addr(j), seg + (size_t)j * kStride, kStride, wbar + 8 * j);
-        }
-    }
     mbar_wait(bar0, 0);                                         // the table image has landed
 
     if (iters) {
@@ -350,36 +323,20 @@ k_checksum_main(const uint8_t* __restrict__ base, uint64_t n_units, uint32_t ite
         const uint32_t k0 = img + lane * 4, k1 = k0 + 128, k2 = k0 + 65536, k3 = k2 + 128;
         uint32_t c0 = 0, c1 = 0, c2 = 0, c3 = 0;
         uint32_t s_a = 0, s_j = 0, s_b = 0;    // sum, iteration-weighted sum, in-piece weighted sum
-        if (kTma) {
-            uint32_t sl = 0, par = 0;
-            for (uint32_t j = 0; j < iters; ++j) {
-                mbar_wait(wbar + 8 * sl, par);
-                const uint4 w0 = lds128(slot_addr(sl) + lane * 16);
-                __syncwarp();                                   // every lane has its 16 bytes: the slot can be refilled
-                if (lane == 0 && j + kTmaSlots < iters) {
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    mbar_expect_tx(wbar + 8 * sl, kStride);
-                    bulk_g2s(slot_addr(sl), seg + (size_t)(j + kTmaSlots) * kStride, kStride, wbar + 8 * sl);
-                }
-                ZB_CK_STEP(w0, j);
-                if (++sl == (uint32_t)kTmaSlots) { sl = 0; par ^= 1u; }
-            }
-        } else {
-            uint32_t j = 0;
-            // two loads in flight per lane
-            for (; j + 2 <= iters; j += 2) {
-                // two iterations use 1 KiB per warp; ask L2 for the 1 KiB that is kPrefetchAhead iterations away (registers cap
-                // the loads in flight at two per lane, which alone does not cover the HBM latency-bandwidth product)
-                if (lane < 8) asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const uint8_t*>(p - lane) + (size_t)min(j + kPrefetchAhead, iters - 2) * kStride + (lane * 128) % 1024));
-                const uint4 w0 = ld_stream(p + (size_t)j * 32);
-                const uint4 w1 = ld_stream(p + (size_t)(j + 1) * 32);
-                ZB_CK_STEP(w0, j);
-                ZB_CK_STEP(w1, j + 1);
-            }
-            for (; j < iters; ++j) {
-                const uint4 w0 = ld_stream(p + (size_t)j * 32);
-                ZB_CK_STEP(w0, j);
-            }
+        uint32_t j = 0;
+        // two loads in flight per lane
+        for (; j + 2 <= iters; j += 2) {
+            // two iterations use 1 KiB per warp; ask L2 for the 1 KiB that is kPrefetchAhead iterations away (registers cap
+            // the loads in flight at two per lane, which alone does not cover the HBM latency-bandwidth product)
+            if (lane < 8) asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const uint8_t*>(p - lane) + (size_t)min(j + kPrefetchAhead, iters - 2) * kStride + (lane * 128) % 1024));
+            const uint4 w0 = ld_stream(p + (size_t)j * 32);
+            const uint4 w1 = ld_stream(p + (size_t)(j + 1) * 32);
+            ZB_CK_STEP(w0, j);
+            ZB_CK_STEP(w1, j + 1);
+        }
+        for (; j < iters; ++j) {
+            const uint4 w0 = ld_stream(p + (size_t)j * 32);
+            ZB_CK_STEP(w0, j);
         }
 
         // Move the four lane registers to the end of the segment and reduce across the warp.
@@ -653,8 +610,7 @@ int checksum_jobs_launch(Ctx* c, const uint8_t* d_base, const ChunkDesc* d_cd, u
 
 int checksum_attr_setup()                                      // once per device, from ensure_init
 {
-    ZB_CUDA(cudaFuncSetAttribute(k_checksum_main<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMainSmem));
-    ZB_CUDA(cudaFuncSetAttribute(k_checksum_main<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMainSmem));
+    ZB_CUDA(cudaFuncSetAttribute(k_checksum_main, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMainSmem));
     return 0;
 }
 
@@ -708,13 +664,8 @@ int checksum_launch(Ctx* c, const uint8_t* d_buf, size_t len, uint32_t* d_out2, 
     fa.pw_tail = host_pow8(len - tail_begin);
     fa.pw_head = host_pow8(len - head);
     fa.pw_len = host_pow8(len);
-    static const bool tma = getenv("ZB200_CKSUM_TMA") ? atoi(getenv("ZB200_CKSUM_TMA")) != 0 : false;
-    if (tma)
-        ZB_LAUNCH(k_checksum_main<true>, blocks, kMainThreads, kMainSmem, s, d_buf + head, n_units, iters, head, c->ws[0].as<Partial>(),
-                  d_buf, (uint64_t)len, tail_begin, fa, d_out2, done);
-    else
-        ZB_LAUNCH(k_checksum_main<false>, blocks, kMainThreads, kMainSmem, s, d_buf + head, n_units, iters, head, c->ws[0].as<Partial>(),
-                  d_buf, (uint64_t)len, tail_begin, fa, d_out2, done);
+    ZB_LAUNCH(k_checksum_main, blocks, kMainThreads, kMainSmem, s, d_buf + head, n_units, iters, head, c->ws[0].as<Partial>(),
+              d_buf, (uint64_t)len, tail_begin, fa, d_out2, done);
     ZB_CHECK_LAUNCH();
     return 0;
 }

@@ -7,11 +7,11 @@
 // The reference interleaves these per input byte inside one sequential loop.  Here the same
 // decisions are taken in passes over HBM-resident arrays, each with its own parallel axis:
 //
-//   K1a link   one CTA (8 warps) per 128 KiB segment shares a 15-bit hash -> last position table in
+//   K1a link   one CTA (8 warps) per 256 KiB segment shares a 15-bit hash -> last position table in
 //              shared memory (the reference's head[]).  The warps take 128-position tiles round robin; only
 //              the table accesses of a tile are serial and the turn is handed from warp to warp with named
 //              barriers.  Output: for every position the distance to the previous position with the same
-//              3-byte hash (the reference's prev[] chain, stored as deltas so chains cross chunk boundaries
+//              4-byte hash (the reference's prev[] chain, stored as deltas so chains cross chunk boundaries
 //              and the 32 KiB of history in front of a chunk needs no copy -- it is simply there).
 //   K1b walk   one CTA per 32 KiB block, window staged in shared memory, one thread per 64-byte sub-unit
 //              running the reference's own search-emit-skip loop (deflate_fast, or deflate_slow with max_lazy,
@@ -64,7 +64,7 @@ constexpr int kHashBits = 15;
 // ------------------------------------------------------------------------------------------
 // K1a: hash-chain links
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t hash3(uint32_t v, uint32_t mask) { return ((v & mask) * 0x9E3779B1u) >> (32 - kHashBits); }   // mask: three bytes (deflate.c UPDATE_HASH covers MIN_MATCH bytes), or four
+__device__ __forceinline__ uint32_t hash4(uint32_t v) { return (v * 0x9E3779B1u) >> (32 - kHashBits); }   // four bytes, see h_levels
 
 // Ring version: kLinkWarps warps share one segment and one head[] table.  Warp w owns tiles
 // w, w+W, w+2W, ... (a tile = 128 consecutive positions).  Everything that does not touch head[]
@@ -73,6 +73,9 @@ __device__ __forceinline__ uint32_t hash3(uint32_t v, uint32_t mask) { return ((
 // passed from warp to warp in position order with named barriers (producer bar.arrive, consumer
 // bar.sync, 64 threads each).  The links are exactly those of the one-warp version.
 constexpr int kLinkWarps = 8;
+// Stream mode: one CTA links two chunks.  The 32 KiB of priming in front of a segment is redundant work; 1 / 2 / 4 chunks per
+// segment measured 13.50 / 13.31 / 13.56 ms per step.
+constexpr uint32_t kLinkSegBytes = 2 * kChunk;
 
 __device__ __forceinline__ void ring_wait(int id) { asm volatile("bar.sync %0, 64;" ::"r"(id) : "memory"); }
 __device__ __forceinline__ void ring_pass(int id) { asm volatile("bar.arrive %0, 64;" ::"r"(id) : "memory"); }
@@ -114,7 +117,7 @@ __device__ __noinline__ uint2 ring_turn(uint32_t a0, uint32_t a1, uint32_t a2, u
 
 template <bool kExact>
 __global__ void __launch_bounds__(kLinkWarps * 32)
-k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict__ dist16, const ChunkDesc* __restrict__ cd, uint32_t seg_bytes, uint32_t hash_mask)
+k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict__ dist16, const ChunkDesc* __restrict__ cd)
 {
     extern __shared__ uint16_t s_head[];                       // 2^15 entries: low 16 bits of the last position
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -129,8 +132,8 @@ k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict_
         seg_beg = d.beg; seg_end = (uint64_t)d.beg + d.len; origin = d.job_beg; lim = d.job_end;
         prime_beg = seg_beg - origin > kWindow ? seg_beg - kWindow : origin;
     } else {
-        seg_beg = (uint64_t)blockIdx.x * seg_bytes;             // stream mode: a CTA links seg_bytes (a few chunks: the 32 KiB of priming
-        seg_end = min(total, seg_beg + seg_bytes);              // in front of a segment is redundant work)
+        seg_beg = (uint64_t)blockIdx.x * kLinkSegBytes;         // stream mode: a CTA links kLinkSegBytes
+        seg_end = min(total, seg_beg + kLinkSegBytes);
         prime_beg = seg_beg > kWindow ? seg_beg - kWindow : 0;
         origin = 0; lim = total;
     }
@@ -143,8 +146,8 @@ k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict_
     const uint32_t nwords = (uint32_t)min((uint64_t)0x7fffffffu, ((mis + total + 3) >> 2) - tile_beg * 32);
     uint16_t* dout = dist16 + q0 - mis;                         // dout[q - q0] = link of position q - mis (never dereferenced below q_seg)
     const int q_lo = (int)(prime_beg + mis - q0);               // first position to insert
-    const uint32_t hbytes = hash_mask == 0xffffffffu ? 4u : 3u; // a position is entered only if all the bytes of its hash are the stream's own
-    const int q_hi = (int)(min(seg_end, lim >= origin + hbytes - 1 ? lim - (hbytes - 1) : origin) + mis) - (int)q0;   // one past the last hashable position
+    // one past the last hashable position: a position is entered only if all four bytes of its hash are the stream's own
+    const int q_hi = (int)(min(seg_end, lim >= origin + 3 ? lim - 3 : origin) + mis) - (int)q0;
     const int q_seg = (int)(seg_beg + mis - q0), q_end = (int)(seg_end + mis - q0);   // positions whose link is stored
     const int p_cap = (int)min((uint64_t)0x40000000u, q0 - mis + 128 - origin) - 128;   // stream position of q0, saturated (only "dd > p" uses it)
     const uint32_t ntiles = (uint32_t)(tile_end - tile_beg);
@@ -170,7 +173,7 @@ k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict_
             if (j == 31) wb = ext;
             const uint32_t v = __funnelshift_r(wa, wb, (li & 3) * 8);
             const bool valid = li >= lo && li < hi;
-            h[k] = valid ? hash3(v, hash_mask) : (0x10000u + lane);
+            h[k] = valid ? hash4(v) : (0x10000u + lane);
             if (kExact) {
                 const uint32_t grp = __match_any_sync(kFullMask, h[k]);
                 const uint32_t lower = grp & lt;
@@ -316,7 +319,7 @@ __global__ void __launch_bounds__(kT, kSmemLinks ? 1 : 3)
 k_lz_walk(const uint8_t* __restrict__ buf, uint32_t total, uint32_t dict, const uint16_t* __restrict__ dist16,
           uint32_t* __restrict__ tok_tmp, uint32_t* __restrict__ tok, uint32_t* __restrict__ blk_ntok,
           uint32_t* __restrict__ blk_hist, int kind, int max_chain, uint32_t nice, uint32_t max_lazy, uint32_t good,
-          int strategy, uint32_t max_dist, const ChunkDesc* __restrict__ cd, uint32_t nblocks, uint32_t* __restrict__ next_block, int flat_lazy)
+          int strategy, uint32_t max_dist, const ChunkDesc* __restrict__ cd, uint32_t nblocks, uint32_t* __restrict__ next_block)
 {
     extern __shared__ __align__(16) uint8_t s_mem[];
     __shared__ uint32_t s_hist[kHistSize];
@@ -327,28 +330,23 @@ k_lz_walk(const uint8_t* __restrict__ buf, uint32_t total, uint32_t dict, const 
     __shared__ uint32_t s_first[kT];
     __shared__ uint32_t s_wsum[kT / 32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    // Persistent CTAs (next_block != nullptr): the grid is one CTA per resident slot and every CTA takes the next
-    // unclaimed block from a device counter.  The private token regions are then indexed by SLOT, not by block: a few
-    // tens of MB that are rewritten every ~100 us and stay in L2, instead of one region per block of the slab (half a
-    // GB per slab that went out to HBM and came back).
+    // Persistent CTAs: the grid is one CTA per resident slot and every CTA takes the next unclaimed block from a device
+    // counter.  The private token regions are indexed by SLOT, not by block: a few tens of MB that are rewritten every
+    // ~100 us and stay in L2, instead of one region per block of the slab (half a GB per slab that went out to HBM and
+    // came back).
     __shared__ uint32_t s_claim;
     const uint32_t slot = blockIdx.x;
   for (;;) {
-    uint32_t b;
-    if (next_block) {
-        __syncthreads();                                        // the previous block's shared memory is no longer read
-        if (tid == 0) s_claim = atomicAdd(next_block, 1u);
-        __syncthreads();
-        b = s_claim;
-        if (b >= nblocks) return;
-    } else {
-        b = blockIdx.x;
-    }
+    __syncthreads();                                            // the previous block's shared memory is no longer read
+    if (tid == 0) s_claim = atomicAdd(next_block, 1u);
+    __syncthreads();
+    const uint32_t b = s_claim;
+    if (b >= nblocks) return;
     uint32_t blk_beg, blk_end, win_beg;                         // absolute positions in buf
     if (cd) {                                                   // job mode: block b is the (b % 4)-th block of a chunk of some job
         const ChunkDesc d = cd[b / kBlocksPerChunk];
         const uint32_t rel = (b % kBlocksPerChunk) * kBlockBytes;
-        if (rel >= d.len) { if (next_block) continue; return; } // short chunk: this block slot is unused (nobody reads it)
+        if (rel >= d.len) continue;                             // short chunk: this block slot is unused (nobody reads it)
         blk_beg = d.beg + rel;
         blk_end = d.beg + min(d.len, rel + kBlockBytes);
         win_beg = blk_beg - d.job_beg > kWindow ? blk_beg - kWindow : d.job_beg;
@@ -388,7 +386,7 @@ k_lz_walk(const uint8_t* __restrict__ buf, uint32_t total, uint32_t dict, const 
 
     // ---- walk this thread's sub-unit ----
     const uint32_t s0 = blk_beg + tid * kSub, s1 = min(s0 + kSub, blk_end);
-    uint32_t* mine = tok_tmp + (size_t)(next_block ? slot : b) * kTmpPerBlock + (size_t)tid * kSubSlots + kFront;
+    uint32_t* mine = tok_tmp + (size_t)slot * kTmpPerBlock + (size_t)tid * kSubSlots + kFront;
     uint32_t ntok = 0, pos = s0;
     if (s0 < blk_end) {
         if (kind == 1) {                                        // deflate_fast, deflate.c:1448-1546
@@ -429,105 +427,6 @@ k_lz_walk(const uint8_t* __restrict__ buf, uint32_t total, uint32_t dict, const 
                 if (ph > 0) mine[at] = held0;
                 if (ph > 1) mine[at + 1] = held1;
                 if (ph > 2) mine[at + 2] = held2;
-            }
-        } else if (kSmemLinks && flat_lazy && strategy != 3) {  // deflate_slow, deflate.c:1554-1674, as a flat state machine
-            // The nested form (search loop inside the token loop, compare loop inside the search loop) leaves 5 of 32 lanes
-            // active at level 6: a warp stays in the search loop until its longest chain is done (ncu, r2_l6walk).  Here a
-            // lane is in ONE of three states and every trip of the single loop advances it by one step -- one chain
-            // candidate (link + quick reject on the word a longer match must reach), four bytes of a comparison, or the
-            // parse decision between two searches -- so lanes with short chains move on to their next position instead
-            // of waiting.  Same decisions, same tokens as the nested form.
-            enum { kStNext = 0, kStCand = 1, kStCmp = 2, kStDone = 3 };
-            uint32_t prev_len = kMinMatch - 1, prev_dist = 0;
-            bool avail = false, started = false;
-            uint32_t st = kStNext;
-            uint32_t o = 0, acc = 0, best_len = kMinMatch - 1, best_dist = 0, qoff = 0, qmask = 0, hq = 0, maxlen = 0, nice_eff = 0;
-            uint32_t cmp_len = 0, d_next = 0;
-            int chain = 0;
-            while (st != kStDone) {
-                bool cand_done = false;
-                uint32_t len = 0;
-                if (st == kStCmp) {
-                    const uint32_t co = o - acc;
-                    const uint32_t y = lds32u(s_mem, o + cmp_len) ^ lds32u(s_mem, co + cmp_len);
-                    if (y) { len = cmp_len + ((uint32_t)(__ffs(y) - 1) >> 3); cand_done = true; }
-                    else { cmp_len += 4; len = cmp_len; cand_done = cmp_len >= maxlen; }
-                } else if (st == kStCand) {
-                    const uint32_t co = o - acc;
-                    d_next = links[(pos - win_beg) - acc];
-                    const uint32_t x = lds32u(s_mem, co + qoff) ^ hq;
-                    if ((x & qmask) == 0) {
-                        if (qoff == 0 && x != 0) { len = 3; cand_done = true; }     // first three agree, the fourth does not
-                        else {
-                            cmp_len = qoff == 0 ? 4u : 0u;
-                            if (cmp_len >= maxlen) { len = maxlen; cand_done = true; }
-                            else st = kStCmp;
-                        }
-                    } else {
-                        cand_done = true;                       // rejected: len 0 never beats best_len
-                    }
-                }
-                if (cand_done) {                                // this candidate is settled: keep it if longer, move down the chain
-                    len = min(len, maxlen);
-                    bool stop = false;
-                    if (len > best_len) {
-                        best_len = len; best_dist = acc;
-                        if (len >= nice_eff) stop = true;
-                        else {
-                            qoff = len >= 4 ? len - 3 : 0u;
-                            qmask = 0xffffffffu;
-                            hq = lds32u(s_mem, o + qoff);
-                        }
-                    }
-                    if (stop || d_next == 0) st = kStNext;
-                    else {
-                        acc += d_next;
-                        st = (--chain <= 0 || acc > max_dist) ? kStNext : kStCand;
-                    }
-                }
-                if (st == kStNext) {
-                    for (;;) {
-                        if (started) {                          // the position's result is in (best_len, best_dist): the lazy decision
-                            uint32_t flen = best_dist ? best_len : kMinMatch - 1;
-                            const uint32_t fdist = best_dist;
-                            if (flen <= 5 && (strategy == 1 || (flen == kMinMatch && fdist > kTooFar))) flen = kMinMatch - 1;   // Z_FILTERED, TOO_FAR
-                            if (prev_len >= kMinMatch && flen <= prev_len) {            // the pending match wins
-                                mine[ntok++] = (prev_dist << 16) | (prev_len - kMinMatch);
-                                pos += prev_len - 1;
-                                avail = false; prev_len = kMinMatch - 1;
-                            } else if (avail) {                                         // pending literal goes out, the new match waits
-                                mine[ntok++] = byte_at(pos - 1);
-                                prev_len = flen; prev_dist = fdist;
-                                pos++;
-                            } else {
-                                avail = true;
-                                prev_len = flen; prev_dist = fdist;
-                                pos++;
-                            }
-                        }
-                        started = true;
-                        if (!avail && pos >= s1) { st = kStDone; break; }
-                        if (avail && pos - 1 >= s1) { pos--; st = kStDone; break; }   // the pending position belongs to the next sub-unit
-                        best_len = kMinMatch - 1; best_dist = 0;
-                        if (pos < blk_end) {
-                            maxlen = blk_end - pos < kMaxMatch ? blk_end - pos : kMaxMatch;
-                            if (maxlen >= kMinMatch && prev_len < max_lazy) {
-                                if (prev_len > best_len) best_len = prev_len;           // only a longer match is of interest
-                                acc = links[pos - win_beg];
-                                if (acc != 0 && best_len < maxlen && acc <= max_dist) {
-                                    chain = prev_len >= good ? max(max_chain >> 2, 1) : max_chain;
-                                    o = sm_off + pos - win_beg;
-                                    nice_eff = min(nice, maxlen);
-                                    qoff = best_len >= 4 ? best_len - 3 : 0u;
-                                    qmask = best_len >= 3 ? 0xffffffffu : 0xffffffu;
-                                    hq = lds32u(s_mem, o + qoff);
-                                    st = kStCand;
-                                    break;
-                                }
-                            }
-                        }
-                    }
-                }
             }
         } else {                                                // deflate_slow, deflate.c:1554-1674
             uint32_t prev_len = kMinMatch - 1, prev_dist = 0;
@@ -615,7 +514,7 @@ k_lz_walk(const uint8_t* __restrict__ buf, uint32_t total, uint32_t dict, const 
     __syncthreads();
     // ---- each warp moves its 32 regions, coalesced, and tallies ----
     uint32_t* out = tok + (size_t)b * kBlockBytes;
-    const uint32_t* tmp_blk = tok_tmp + (size_t)(next_block ? slot : b) * kTmpPerBlock;
+    const uint32_t* tmp_blk = tok_tmp + (size_t)slot * kTmpPerBlock;
     auto tally = [&](uint32_t v) {
         const bool is_match = (v >> 16) != 0;
         atomicAdd(&s_hist[is_match ? 257 + len_code(v & 0xffffu) : v], 1u);
@@ -643,7 +542,6 @@ k_lz_walk(const uint8_t* __restrict__ buf, uint32_t total, uint32_t dict, const 
     __syncthreads();
     for (int i = tid; i < (int)kHistSize; i += kT) blk_hist[(size_t)b * kHistSize + i] = s_hist[i];
     if (tid == 0) blk_ntok[b] = all;
-    if (!next_block) return;
   }
 }
 
@@ -1126,7 +1024,46 @@ __global__ void __launch_bounds__(1024) k_scan_jobs(uint32_t nchunks, ChunkMeta*
     }
 }
 
-// Job mode: header and trailer of every stream of the slab (deflate.c:577-650, 832-850), one thread per job.
+// ------------------------------------------------------------------------------------------
+// stream framing: header and trailer (deflate.c:577-650, 832-850)
+// ------------------------------------------------------------------------------------------
+__host__ __device__ constexpr uint32_t frame_header_len(int wrap)
+{
+    return wrap == ZB200_WRAP_ZLIB ? 2 : wrap == ZB200_WRAP_GZIP ? 10 : wrap == kWrapBgzf ? kBgzfHeader : 0;
+}
+__host__ __device__ constexpr uint32_t frame_trailer_len(int wrap)
+{
+    return wrap == ZB200_WRAP_ZLIB ? 4 : (wrap == ZB200_WRAP_GZIP || wrap == kWrapBgzf) ? 8 : 0;
+}
+
+// zlib or gzip header (BGZF's is written by k_frame_jobs); Z_HUFFMAN_ONLY and above report the fastest level
+__device__ __forceinline__ void write_frame_header(uint8_t* o, int wrap, int level, int strat)
+{
+    if (wrap == ZB200_WRAP_ZLIB) {
+        const uint32_t fl = (level < 2 || strat >= 2) ? 0 : level < 6 ? 1 : level == 6 ? 2 : 3;   // deflate.c:628-636
+        uint32_t h = (0x78u << 8) | (fl << 6);
+        h += 31 - h % 31;
+        o[0] = h >> 8; o[1] = h;
+    } else if (wrap == ZB200_WRAP_GZIP) {
+        const uint8_t g[10] = {31, 139, 8, 0, 0, 0, 0, 0, (uint8_t)(level == 9 ? 2 : (level < 2 || strat >= 2) ? 4 : 0), 3};   // deflate.c:590-593
+        for (int i = 0; i < 10; i++) o[i] = g[i];
+    }
+}
+
+// The trailer in front of `end`.  zlib: big-endian Adler-32; gzip and BGZF: CRC-32, then the input length mod 2^32.
+__device__ __forceinline__ void write_frame_trailer(uint8_t* end, int wrap, uint32_t crc, uint32_t adler, uint64_t len)
+{
+    if (wrap == ZB200_WRAP_ZLIB) {
+        uint8_t* t = end - 4;
+        t[0] = adler >> 24; t[1] = adler >> 16; t[2] = adler >> 8; t[3] = adler;
+    } else if (wrap == ZB200_WRAP_GZIP || wrap == kWrapBgzf) {
+        uint8_t* t = end - 8;
+        for (int i = 0; i < 4; i++) t[i] = crc >> (8 * i);
+        for (int i = 0; i < 4; i++) t[4 + i] = (uint8_t)(len >> (8 * i));
+    }
+}
+
+// Job mode: header and trailer of every stream of the slab, one thread per job.
 __global__ void k_frame_jobs(uint8_t* __restrict__ out, const JobDesc* __restrict__ jobs, uint32_t njobs,
                              const uint32_t* __restrict__ crc, const uint32_t* __restrict__ adler, int level, int wrap,
                              int strat, JobResult* __restrict__ jres)
@@ -1139,31 +1076,15 @@ __global__ void k_frame_jobs(uint8_t* __restrict__ out, const JobDesc* __restric
     const uint64_t total = jres[j].total;
     if (total > jd.dst_cap) return;
     uint8_t* o = out + jd.dst_off;
-    uint32_t hl = 0;
-    if (wrap == ZB200_WRAP_ZLIB) {
-        const uint32_t fl = (level < 2 || strat >= 2) ? 0 : level < 6 ? 1 : level == 6 ? 2 : 3;   // deflate.c:628-636
-        uint32_t h = (0x78u << 8) | (fl << 6);
-        h += 31 - h % 31;
-        o[0] = h >> 8; o[1] = h; hl = 2;
-    } else if (wrap == ZB200_WRAP_GZIP) {
-        const uint8_t g[10] = {31, 139, 8, 0, 0, 0, 0, 0, (uint8_t)(level == 9 ? 2 : (level < 2 || strat >= 2) ? 4 : 0), 3};   // deflate.c:590-593
-        for (int i = 0; i < 10; i++) o[i] = g[i];
-        hl = 10;
-    } else if (wrap == kWrapBgzf) {                             // htslib's bgzf.c header bytes; BSIZE is known only here
+    if (wrap == kWrapBgzf) {                                    // htslib's bgzf.c header bytes; BSIZE is known only here
         const uint8_t g[16] = {31, 139, 8, 4, 0, 0, 0, 0, 0, 255, 6, 0, 'B', 'C', 2, 0};
         for (int i = 0; i < 16; i++) o[i] = g[i];
         o[16] = (uint8_t)(total - 1); o[17] = (uint8_t)((total - 1) >> 8);   // total > 65536 is refused by the caller
-        hl = kBgzfHeader;
+    } else {
+        write_frame_header(o, wrap, level, strat);
     }
-    if (jd.nchunks == 0) { o[hl] = 3; o[hl + 1] = 0; }
-    if (wrap == ZB200_WRAP_ZLIB) {
-        uint8_t* t = o + total - 4;
-        t[0] = ad >> 24; t[1] = ad >> 16; t[2] = ad >> 8; t[3] = ad;
-    } else if (wrap == ZB200_WRAP_GZIP || wrap == kWrapBgzf) {
-        uint8_t* t = o + total - 8;
-        for (int i = 0; i < 4; i++) t[i] = cr >> (8 * i);
-        for (int i = 0; i < 4; i++) t[4 + i] = (uint8_t)(jd.src_len >> (8 * i));
-    }
+    if (jd.nchunks == 0) { const uint32_t hl = frame_header_len(wrap); o[hl] = 3; o[hl + 1] = 0; }
+    write_frame_trailer(o + total, wrap, cr, ad, jd.src_len);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1441,41 +1362,18 @@ k_huff_pack(const uint8_t* __restrict__ src, uint64_t n, const uint32_t* __restr
     if (threadIdx.x == 0 && (pk.bytepos != cm.bytes || pk.carry_bits != 0)) atomicAdd(err, 1u);
 }
 
-// ------------------------------------------------------------------------------------------
-// stream framing: header and trailer (deflate.c:577-650, 832-850)
-// ------------------------------------------------------------------------------------------
+// One stream: header and trailer around the payload that ends at d_end[0].
 __global__ void k_frame(uint8_t* __restrict__ out, uint64_t cap, uint64_t hdr_len, const uint64_t* __restrict__ d_end,
                         const uint32_t* __restrict__ sums, uint64_t n, int level, int wrap, int flags, uint64_t* __restrict__ total_out)
 {
     if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    const int strat = (flags >> 8) & 7;                         // Z_HUFFMAN_ONLY and above report the fastest level
-    uint64_t pos = d_end[0];                                    // header + every slab's payload
-    uint8_t trailer[8]; int tl = 0;
-    if (!(flags & (ZB200_DEFLATE_NO_TRAILER | ZB200_DEFLATE_NOT_LAST))) {
-        if (wrap == ZB200_WRAP_ZLIB) {
-            const uint32_t a = sums[1];
-            trailer[0] = a >> 24; trailer[1] = a >> 16; trailer[2] = a >> 8; trailer[3] = a; tl = 4;
-        } else if (wrap == ZB200_WRAP_GZIP) {
-            const uint32_t cr = sums[0];
-            for (int i = 0; i < 4; i++) trailer[i] = cr >> (8 * i);
-            for (int i = 0; i < 4; i++) trailer[4 + i] = (uint8_t)(n >> (8 * i));
-            tl = 8;
-        }
-    }
+    const uint64_t pos = d_end[0];                              // header + every slab's payload
+    const uint32_t tl = (flags & (ZB200_DEFLATE_NO_TRAILER | ZB200_DEFLATE_NOT_LAST)) ? 0 : frame_trailer_len(wrap);
+    const uint32_t crc = sums[0], adler = sums[1];
     total_out[0] = pos + tl;
     if (pos + tl > cap) return;
-    if (hdr_len) {
-        if (wrap == ZB200_WRAP_ZLIB) {
-            const uint32_t fl = (level < 2 || strat >= 2) ? 0 : level < 6 ? 1 : level == 6 ? 2 : 3;   // deflate.c:628-636
-            uint32_t h = (0x78u << 8) | (fl << 6);
-            h += 31 - h % 31;
-            out[0] = h >> 8; out[1] = h;
-        } else if (wrap == ZB200_WRAP_GZIP) {
-            const uint8_t g[10] = {31, 139, 8, 0, 0, 0, 0, 0, (uint8_t)(level == 9 ? 2 : (level < 2 || strat >= 2) ? 4 : 0), 3};   // deflate.c:590-593
-            for (int i = 0; i < 10; i++) out[i] = g[i];
-        }
-    }
-    for (int i = 0; i < tl; i++) out[pos + i] = trailer[i];
+    if (hdr_len) write_frame_header(out, wrap, level, (flags >> 8) & 7);
+    if (tl) write_frame_trailer(out + pos + tl, wrap, crc, adler, n);
 }
 
 // empty input: a lone final fixed block with just the end-of-block code = 03 00 (what the reference emits)
@@ -1499,38 +1397,66 @@ struct DeflateParams {
     uint32_t max_dist;                                          // kWindow, or the reference's MAX_DIST of a smaller windowBits
 };
 
-// Development knobs (read once): ZB200_WALK_PERSIST=0 restores one CTA per block; ZB200_L1_CHAIN / ZB200_L1_NICE override
-// the level-1 search budget for sweeps.  None of them is part of the interface.
-static int env_int(const char* name, int dflt)
-{
-    const char* v = getenv(name);
-    return (v && *v) ? atoi(v) : dflt;
-}
-// The flat state machine of the lazy walk pays where chains are long (levels 7..9: up to 1.19 x); below that its longer
-// trip costs more than the idle lanes of the nested loops (level 6: 0.85 .. 0.96 x, level 4: 0.65 x; profiles/r2_sweeps.md).
-static int walk_flat_lazy(int chain) { static const int force = env_int("ZB200_LAZY_FLAT", -1); return force >= 0 ? force : (chain >= 256 ? 1 : 0); }
 // exact intra-step links (MATCH.ANY, 8.4 ms per GiB) for the levels that search long chains; levels 1..6 take the relaxed
 // links (3.1 ms per GiB, ~0.1 % larger output)
-static bool link_exact(int level, int strategy) { static const int force = env_int("ZB200_LINK_EXACT", -1); return force >= 0 ? force != 0 : (level >= 7 || (level >= 4 && strategy == 4)); }
-// lazy levels whose chain budget is at most this run in the greedy shape (links from L2, 3 CTAs per SM); development knob
-static uint32_t link_hash_mask(int level)                       // four hashed bytes from this level on (development: 10 = the reference's three everywhere)
-{
-    static const int from = env_int("ZB200_HASH4_FROM", 1);
-    return level >= from ? 0xffffffffu : 0xffffffu;
-}
+static bool link_exact(int level, int strategy) { return level >= 7 || (level >= 4 && strategy == 4); }
 // Lazy levels whose chain budget is at most this run in the greedy shape (links from L2, 64-byte sub-units, 3 CTAs per SM): with
 // the short budgets of the four-byte chains the few link loads per search no longer pay for staging the links in shared memory
 // (levels 4..7: 5 to 12 % faster and 0.1 % smaller, profiles/r2_sweeps.md).  Longer chains (levels 8, 9) keep the shared-memory links.
-static int lazy_global_max() { static const int v = env_int("ZB200_LAZY_GLOBAL_MAX", 16); return v; }
-static bool walk_persistent() { static const bool on = env_int("ZB200_WALK_PERSIST", 1) != 0; return on; }
-static unsigned walk_grid(uint64_t nblocks, bool lazy_shape)
+constexpr uint32_t kLazyGlobalMax = 16;
+constexpr uint64_t kWalkCtasPerSm = 3;                          // greedy shape: three fit (the lazy shape: one)
+
+struct BlockBufs {                                              // what k_plan and k_huff_pack read (all null at level 0)
+    BlockMeta* blk = nullptr;
+    uint32_t *tok = nullptr, *ntok = nullptr, *codes = nullptr, *hdr = nullptr;
+};
+
+// Link, walk and code construction of nblocks blocks: the scratch, then the kernels on s.  Stream mode (d_cd null): d_buf =
+// [dict][source], total = dict + source bytes, blocks from d_buf + dict on.  Job mode: d_buf[0, total) holds the jobs of
+// the chunk table d_cd, dict = 0, four block slots per chunk.
+static int deflate_blocks_launch(Ctx* c, const uint8_t* d_buf, uint64_t total, uint64_t dict, uint64_t nblocks,
+                                 const ChunkDesc* d_cd, const DeflateParams& P, cudaStream_t s, BlockBufs* out)
 {
-    if (!walk_persistent()) return (unsigned)nblocks;
-    static const int per_sm = std::min(3, std::max(1, env_int("ZB200_WALK_CTAS_PER_SM", 3)));   // greedy shape: three fit; fewer leave room for the other slab's kernels
-    const uint64_t slots = (uint64_t)device_sms() * (lazy_shape ? 1 : per_sm);
-    return (unsigned)std::min<uint64_t>(nblocks, slots);
+    const LevelCfg& cfg = P.cfg;
+    if (cfg.kind == 0 || nblocks == 0) return 0;
+    const uint64_t slots = std::min<uint64_t>(nblocks, (uint64_t)device_sms() * kWalkCtasPerSm);   // persistent walk CTAs
+    int rc;
+    if ((rc = c->ws[3].ensure(total * 2 + 64)) != 0) return rc;                          // dist16
+    if ((rc = c->ws[4].ensure(slots * kTmpPerBlock * 4 + 64)) != 0) return rc;           // private token regions
+    if ((rc = c->ws[5].ensure(nblocks * kBlockBytes * 4 + 64)) != 0) return rc;          // tokens, contiguous per block
+    if ((rc = c->ws[6].ensure(nblocks * sizeof(BlockMeta))) != 0) return rc;
+    if ((rc = c->ws[7].ensure(nblocks * kHistSize * 4)) != 0) return rc;
+    if ((rc = c->ws[8].ensure(nblocks * kHistSize * 4)) != 0) return rc;
+    if ((rc = c->ws[9].ensure(nblocks * kHdrWords * 4)) != 0) return rc;
+    if ((rc = c->ws[10].ensure(nblocks * 4 + 16)) != 0) return rc;
+    uint16_t* d_dist = c->ws[3].as<uint16_t>();
+    uint32_t* d_tmp = c->ws[4].as<uint32_t>();
+    uint32_t* d_hist = c->ws[7].as<uint32_t>();
+    out->tok = c->ws[5].as<uint32_t>();
+    out->blk = c->ws[6].as<BlockMeta>();
+    out->codes = c->ws[8].as<uint32_t>(); out->hdr = c->ws[9].as<uint32_t>();
+    out->ntok = c->ws[10].as<uint32_t>();
+    uint32_t* d_next = out->ntok + nblocks;                     // the walk kernel's block counter
+    if (cfg.chain != 0 && P.strategy != 3) {                    // Z_RLE needs no chains
+        const unsigned nseg = (unsigned)(d_cd ? nblocks / kBlocksPerChunk : (total + kLinkSegBytes - 1) / kLinkSegBytes);
+        // levels 1-6 trade the exact intra-step links for speed, like the reference's fast levels trade ratio
+        if (link_exact(P.level, P.strategy)) ZB_LAUNCH(k_lz_link<true>, nseg, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_buf, total, d_dist, d_cd);
+        else ZB_LAUNCH(k_lz_link<false>, nseg, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_buf, total, d_dist, d_cd);
+    }
+    ZB_CUDA(cudaMemsetAsync(d_next, 0, 4, s));
+    if (cfg.kind == 2 && cfg.chain > kLazyGlobalMax && P.strategy != 3)
+        ZB_LAUNCH((k_lz_walk<kWalkThreadsLazy, true>), (unsigned)std::min<uint64_t>(nblocks, device_sms()), kWalkThreadsLazy,
+                  kWalkSmem + kWalkLinkSmem, s, d_buf, (uint32_t)total, (uint32_t)dict, d_dist, d_tmp, out->tok, out->ntok, d_hist,
+                  cfg.kind, (int)cfg.chain, (uint32_t)cfg.nice, (uint32_t)cfg.lazy, (uint32_t)cfg.good, P.strategy, P.max_dist, d_cd,
+                  (uint32_t)nblocks, d_next);
+    else
+        ZB_LAUNCH((k_lz_walk<kWalkThreadsFast, false>), (unsigned)slots, kWalkThreadsFast, kWalkSmem, s, d_buf, (uint32_t)total,
+                  (uint32_t)dict, d_dist, d_tmp, out->tok, out->ntok, d_hist, cfg.kind, (int)cfg.chain, (uint32_t)cfg.nice,
+                  (uint32_t)cfg.lazy, (uint32_t)cfg.good, P.strategy, P.max_dist, d_cd, (uint32_t)nblocks, d_next);
+    ZB_LAUNCH(k_huff_build, (unsigned)((nblocks + kCodeWarps - 1) / kCodeWarps), kCodeWarps * 32, 0, s, total - dict, out->blk, d_hist,
+              out->codes, out->hdr, P.strategy == 4 ? 1 : 0, d_cd, nblocks);
+    return 0;
 }
-static uint64_t walk_slots(uint64_t nblocks) { return walk_persistent() ? std::min<uint64_t>(nblocks, (uint64_t)device_sms() * 3) : nblocks; }
 
 // One slab: d_buf = [dict bytes][n source bytes], contiguous in device memory.  The slab's payload starts at
 // out[(*d_start or 0) + start_add]; *d_end receives where the next slab starts.  Everything is asynchronous on s.
@@ -1539,60 +1465,20 @@ static int deflate_slab_launch(Ctx* c, const uint8_t* d_buf, uint64_t dict, uint
                                uint64_t start_add, uint64_t* d_end, uint32_t* d_err, cudaStream_t s,
                                cudaEvent_t prev_scanned = nullptr, cudaEvent_t scanned = nullptr, uint32_t bitmode = 0, uint32_t prime_val = 0)
 {
-    const LevelCfg& cfg = P.cfg;
-    const uint64_t total = dict + n;
     const uint64_t nchunks = (n + kChunk - 1) / kChunk;
     const uint64_t nblocks = (n + kBlockBytes - 1) / kBlockBytes;
-    const uint8_t* d_src = d_buf + dict;
     int rc;
     if ((rc = c->ws[2].ensure(nchunks * sizeof(ChunkMeta))) != 0) return rc;
     ChunkMeta* d_chunks = c->ws[2].as<ChunkMeta>();
-    BlockMeta* d_blk = nullptr;
-    uint32_t *d_hist = nullptr, *d_codes = nullptr, *d_hdr = nullptr, *d_tok = nullptr, *d_ntok = nullptr;
-    if (cfg.kind != 0) {
-        if ((rc = c->ws[3].ensure(total * 2 + 64)) != 0) return rc;          // dist16
-        if ((rc = c->ws[4].ensure((uint64_t)walk_slots(nblocks) * kTmpPerBlock * 4 + 64)) != 0) return rc;               // private token regions
-        if ((rc = c->ws[5].ensure(nblocks * kBlockBytes * 4 + 64)) != 0) return rc;               // tokens, contiguous per block
-        if ((rc = c->ws[6].ensure(nblocks * sizeof(BlockMeta))) != 0) return rc;
-        if ((rc = c->ws[7].ensure(nblocks * kHistSize * 4)) != 0) return rc;
-        if ((rc = c->ws[8].ensure(nblocks * kHistSize * 4)) != 0) return rc;
-        if ((rc = c->ws[9].ensure(nblocks * kHdrWords * 4)) != 0) return rc;
-        if ((rc = c->ws[10].ensure(nblocks * 4 + 16)) != 0) return rc;
-        uint16_t* d_dist = c->ws[3].as<uint16_t>();
-        uint32_t* d_tmp = c->ws[4].as<uint32_t>();
-        d_tok = c->ws[5].as<uint32_t>();
-        d_blk = c->ws[6].as<BlockMeta>();
-        d_hist = c->ws[7].as<uint32_t>(); d_codes = c->ws[8].as<uint32_t>(); d_hdr = c->ws[9].as<uint32_t>();
-        d_ntok = c->ws[10].as<uint32_t>();
-        uint32_t* d_next = walk_persistent() ? d_ntok + nblocks : nullptr;   // the walk kernel's block counter
-        static const uint32_t link_seg = kChunk * (uint32_t)std::max(1, env_int("ZB200_LINK_SEG_CHUNKS", 2));
-        const unsigned nseg = (unsigned)((total + link_seg - 1) / link_seg);
-        if (cfg.chain != 0 && P.strategy != 3) {                // Z_RLE needs no chains
-            // levels 1-6 trade the exact intra-step links for speed, like the reference's fast levels trade ratio
-            if (link_exact(P.level, P.strategy)) ZB_LAUNCH(k_lz_link<true>, nseg, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_buf, total, d_dist, (const ChunkDesc*)nullptr, link_seg, link_hash_mask(P.level));
-            else ZB_LAUNCH(k_lz_link<false>, nseg, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_buf, total, d_dist, (const ChunkDesc*)nullptr, link_seg, link_hash_mask(P.level));
-        }
-        const bool lazy_shape = cfg.kind == 2 && cfg.chain != 0 && P.strategy != 3 && (int)cfg.chain > lazy_global_max();
-        const unsigned wgrid = walk_grid(nblocks, lazy_shape);
-        if (d_next) ZB_CUDA(cudaMemsetAsync(d_next, 0, 4, s));
-        if (lazy_shape)
-            ZB_LAUNCH((k_lz_walk<kWalkThreadsLazy, true>), wgrid, kWalkThreadsLazy, kWalkSmem + kWalkLinkSmem, s, d_buf, (uint32_t)total,
-                      (uint32_t)dict, d_dist, d_tmp, d_tok, d_ntok, d_hist, cfg.kind, (int)cfg.chain, (uint32_t)cfg.nice, (uint32_t)cfg.lazy,
-                      (uint32_t)cfg.good, P.strategy, P.max_dist, (const ChunkDesc*)nullptr, (uint32_t)nblocks, d_next, walk_flat_lazy((int)cfg.chain));
-        else
-            ZB_LAUNCH((k_lz_walk<kWalkThreadsFast, false>), wgrid, kWalkThreadsFast, kWalkSmem, s, d_buf, (uint32_t)total,
-                      (uint32_t)dict, d_dist, d_tmp, d_tok, d_ntok, d_hist, cfg.kind, (int)cfg.chain, (uint32_t)cfg.nice, (uint32_t)cfg.lazy,
-                      (uint32_t)cfg.good, P.strategy, P.max_dist, (const ChunkDesc*)nullptr, (uint32_t)nblocks, d_next, walk_flat_lazy((int)cfg.chain));
-        ZB_LAUNCH(k_huff_build, (unsigned)((nblocks + kCodeWarps - 1) / kCodeWarps), kCodeWarps * 32, 0, s, n, d_blk, d_hist,
-                  d_codes, d_hdr, P.strategy == 4 ? 1 : 0, (const ChunkDesc*)nullptr, (uint64_t)0);
-    }
-    ZB_LAUNCH(k_plan, (unsigned)((nchunks + 255) / 256), 256, 0, s, nchunks, n, d_chunks, d_blk, last_is_final, cfg.kind == 0 ? 1 : 0, force_mark, (const ChunkDesc*)nullptr, bitmode);
+    BlockBufs bb;
+    if ((rc = deflate_blocks_launch(c, d_buf, dict + n, dict, nblocks, nullptr, P, s, &bb)) != 0) return rc;
+    ZB_LAUNCH(k_plan, (unsigned)((nchunks + 255) / 256), 256, 0, s, nchunks, n, d_chunks, bb.blk, last_is_final, P.cfg.kind == 0 ? 1 : 0, force_mark, (const ChunkDesc*)nullptr, bitmode);
     // Slabs alternate between two streams; only the running output offset links them: this slab's offsets need the
     // end of the previous slab, everything before this point (link, walk, codes, plan) does not.
     if (prev_scanned) ZB_CUDA(cudaStreamWaitEvent(s, prev_scanned, 0));
     ZB_LAUNCH(k_scan, 1, 1024, 0, s, nchunks, d_chunks, d_start, start_add, d_end);
     if (scanned) ZB_CUDA(cudaEventRecord(scanned, s));
-    ZB_LAUNCH(k_huff_pack, (unsigned)nchunks, kPackThreads, 0, s, d_src, n, d_tok, d_ntok, d_blk, d_codes, d_hdr, d_chunks, d_out, cap,
+    ZB_LAUNCH(k_huff_pack, (unsigned)nchunks, kPackThreads, 0, s, d_buf + dict, n, bb.tok, bb.ntok, bb.blk, bb.codes, bb.hdr, d_chunks, d_out, cap,
               last_is_final, force_mark, d_err, (const ChunkDesc*)nullptr, (const JobDesc*)nullptr, (JobResult*)nullptr, bitmode, prime_val, d_err + 1);
     ZB_CHECK_LAUNCH();
     return 0;
@@ -1604,54 +1490,16 @@ static int deflate_jobs_launch(Ctx* c, const uint8_t* d_base, uint64_t span, uin
                                const ChunkDesc* d_cd, const JobDesc* d_jobs, uint8_t* d_out,
                                const DeflateParams& P, uint32_t* d_crc, uint32_t* d_adler, JobResult* d_jres, cudaStream_t s)
 {
-    const LevelCfg& cfg = P.cfg;
-    const uint64_t nblocks = (uint64_t)nchunks * kBlocksPerChunk;
-    const uint32_t hdr_len = P.wrap == ZB200_WRAP_ZLIB ? 2 : P.wrap == ZB200_WRAP_GZIP ? 10 : P.wrap == kWrapBgzf ? kBgzfHeader : 0;
-    const uint32_t trailer_len = P.wrap == ZB200_WRAP_ZLIB ? 4 : (P.wrap == ZB200_WRAP_GZIP || P.wrap == kWrapBgzf) ? 8 : 0;
     int rc;
     if ((rc = c->ws[2].ensure((uint64_t)(nchunks + 1) * sizeof(ChunkMeta))) != 0) return rc;
     ChunkMeta* d_chunks = c->ws[2].as<ChunkMeta>();
-    BlockMeta* d_blk = nullptr;
-    uint32_t *d_hist = nullptr, *d_codes = nullptr, *d_hdr = nullptr, *d_tok = nullptr, *d_ntok = nullptr;
-    if (nchunks && cfg.kind != 0) {
-        if ((rc = c->ws[3].ensure(span * 2 + 64)) != 0) return rc;
-        if ((rc = c->ws[4].ensure((uint64_t)walk_slots(nblocks) * kTmpPerBlock * 4 + 64)) != 0) return rc;
-        if ((rc = c->ws[5].ensure(nblocks * kBlockBytes * 4 + 64)) != 0) return rc;
-        if ((rc = c->ws[6].ensure(nblocks * sizeof(BlockMeta))) != 0) return rc;
-        if ((rc = c->ws[7].ensure(nblocks * kHistSize * 4)) != 0) return rc;
-        if ((rc = c->ws[8].ensure(nblocks * kHistSize * 4)) != 0) return rc;
-        if ((rc = c->ws[9].ensure(nblocks * kHdrWords * 4)) != 0) return rc;
-        if ((rc = c->ws[10].ensure(nblocks * 4 + 16)) != 0) return rc;
-        uint16_t* d_dist = c->ws[3].as<uint16_t>();
-        uint32_t* d_tmp = c->ws[4].as<uint32_t>();
-        d_tok = c->ws[5].as<uint32_t>();
-        d_blk = c->ws[6].as<BlockMeta>();
-        d_hist = c->ws[7].as<uint32_t>(); d_codes = c->ws[8].as<uint32_t>(); d_hdr = c->ws[9].as<uint32_t>();
-        d_ntok = c->ws[10].as<uint32_t>();
-        uint32_t* d_next = walk_persistent() ? d_ntok + nblocks : nullptr;   // the walk kernel's block counter
-        if (cfg.chain != 0 && P.strategy != 3) {
-            if (link_exact(P.level, P.strategy)) ZB_LAUNCH(k_lz_link<true>, nchunks, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_base, span, d_dist, d_cd, kChunk, link_hash_mask(P.level));
-            else ZB_LAUNCH(k_lz_link<false>, nchunks, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_base, span, d_dist, d_cd, kChunk, link_hash_mask(P.level));
-        }
-        const bool lazy_shape = cfg.kind == 2 && cfg.chain != 0 && P.strategy != 3 && (int)cfg.chain > lazy_global_max();
-        const unsigned wgrid = walk_grid(nblocks, lazy_shape);
-        if (d_next) ZB_CUDA(cudaMemsetAsync(d_next, 0, 4, s));
-        if (lazy_shape)
-            ZB_LAUNCH((k_lz_walk<kWalkThreadsLazy, true>), wgrid, kWalkThreadsLazy, kWalkSmem + kWalkLinkSmem, s, d_base, (uint32_t)span,
-                      0u, d_dist, d_tmp, d_tok, d_ntok, d_hist, cfg.kind, (int)cfg.chain, (uint32_t)cfg.nice, (uint32_t)cfg.lazy,
-                      (uint32_t)cfg.good, P.strategy, P.max_dist, d_cd, (uint32_t)nblocks, d_next, walk_flat_lazy((int)cfg.chain));
-        else
-            ZB_LAUNCH((k_lz_walk<kWalkThreadsFast, false>), wgrid, kWalkThreadsFast, kWalkSmem, s, d_base, (uint32_t)span,
-                      0u, d_dist, d_tmp, d_tok, d_ntok, d_hist, cfg.kind, (int)cfg.chain, (uint32_t)cfg.nice, (uint32_t)cfg.lazy,
-                      (uint32_t)cfg.good, P.strategy, P.max_dist, d_cd, (uint32_t)nblocks, d_next, walk_flat_lazy((int)cfg.chain));
-        ZB_LAUNCH(k_huff_build, (unsigned)((nblocks + kCodeWarps - 1) / kCodeWarps), kCodeWarps * 32, 0, s, span, d_blk, d_hist,
-                  d_codes, d_hdr, P.strategy == 4 ? 1 : 0, d_cd, nblocks);
-    }
+    BlockBufs bb;
+    if ((rc = deflate_blocks_launch(c, d_base, span, 0, (uint64_t)nchunks * kBlocksPerChunk, d_cd, P, s, &bb)) != 0) return rc;
     if (nchunks)
-        ZB_LAUNCH(k_plan, (nchunks + 255) / 256, 256, 0, s, (uint64_t)nchunks, span, d_chunks, d_blk, 1, cfg.kind == 0 ? 1 : 0, 0, d_cd, 0u);
-    ZB_LAUNCH(k_scan_jobs, 1, 1024, 0, s, nchunks, d_chunks, d_cd, d_jobs, njobs, hdr_len, trailer_len, d_jres);
+        ZB_LAUNCH(k_plan, (nchunks + 255) / 256, 256, 0, s, (uint64_t)nchunks, span, d_chunks, bb.blk, 1, P.cfg.kind == 0 ? 1 : 0, 0, d_cd, 0u);
+    ZB_LAUNCH(k_scan_jobs, 1, 1024, 0, s, nchunks, d_chunks, d_cd, d_jobs, njobs, frame_header_len(P.wrap), frame_trailer_len(P.wrap), d_jres);
     if (nchunks)
-        ZB_LAUNCH(k_huff_pack, nchunks, kPackThreads, 0, s, d_base, span, d_tok, d_ntok, d_blk, d_codes, d_hdr, d_chunks, d_out, (uint64_t)0,
+        ZB_LAUNCH(k_huff_pack, nchunks, kPackThreads, 0, s, d_base, span, bb.tok, bb.ntok, bb.blk, bb.codes, bb.hdr, d_chunks, d_out, (uint64_t)0,
                   1, 0, (uint32_t*)nullptr, d_cd, d_jobs, d_jres, 0u, 0u, (uint32_t*)nullptr);
     if ((rc = checksum_jobs_launch(c, d_base, d_cd, nchunks, d_jobs, njobs, d_crc, d_adler, s)) != 0) return rc;
     ZB_LAUNCH(k_frame_jobs, (njobs + 127) / 128, 128, 0, s, d_out, d_jobs, njobs, d_crc, d_adler, P.level, P.wrap, P.strategy, d_jres);
@@ -1691,7 +1539,7 @@ static int deflate_enqueue_dev(Ctx* c, cudaStream_t s, const uint8_t* d_buf, uin
 {
     const int force_mark = (P.flags & ZB200I_DEFLATE_FORCE_MARK) ? 1 : 0;
     const int last_is_final = (P.flags & ZB200_DEFLATE_NOT_LAST) ? 0 : 1;
-    const uint64_t hdr_len = (P.flags & ZB200_DEFLATE_NO_HEADER) ? 0 : P.wrap == ZB200_WRAP_ZLIB ? 2 : P.wrap == ZB200_WRAP_GZIP ? 10 : 0;
+    const uint64_t hdr_len = (P.flags & ZB200_DEFLATE_NO_HEADER) ? 0 : frame_header_len(P.wrap);
     std::vector<uint64_t> cut;
     plan_slabs(n, false, cut);
     const uint64_t nslabs = cut.size() - 1;
@@ -1730,21 +1578,7 @@ static int deflate_params(DeflateParams& P, int level, int wrap, int flags)
 {
     if (level < 0) level = 6;
     P.cfg = h_levels[level]; P.level = level; P.wrap = wrap; P.flags = flags;
-    if (level == 1) {
-        static const int chain1 = env_int("ZB200_L1_CHAIN", 0), nice1 = env_int("ZB200_L1_NICE", 0);
-        if (chain1 > 0) P.cfg.chain = (uint16_t)chain1;
-        if (nice1 > 0) P.cfg.nice = (uint16_t)nice1;
-    }
     P.strategy = (flags >> 8) & 7;                              // Z_FILTERED 1, Z_HUFFMAN_ONLY 2, Z_RLE 3, Z_FIXED 4
-    {
-        static const int chain = env_int("ZB200_CHAIN", 0), nice = env_int("ZB200_NICE", 0);   // development: whichever level runs
-        if (chain > 0) P.cfg.chain = (uint16_t)chain;
-        if (nice > 0) P.cfg.nice = (uint16_t)nice;
-    }
-    if (level == 6) {
-        static const int chain6 = env_int("ZB200_L6_CHAIN", 0);
-        if (chain6 > 0) P.cfg.chain = (uint16_t)chain6;
-    }
     const int wbits = (flags >> 12) & 15;                       // 0 = 15; deflate.c:270-279, h/deflate.h:276
     P.max_dist = (wbits >= 9 && wbits < 15) ? (1u << wbits) - 262u : kWindow;
     if (P.strategy == 2 && P.cfg.kind != 0) { P.cfg.chain = 0; P.cfg.kind = 1; }   // literals only (deflate.c:1490)
@@ -1798,7 +1632,7 @@ static int shard_begin(ShardJob* J, const void* src, size_t src_len, const void*
     level = P.level;
     const int force_mark = (flags & ZB200I_DEFLATE_FORCE_MARK) ? 1 : 0;
     const int last_is_final = (flags & ZB200_DEFLATE_NOT_LAST) ? 0 : 1;
-    const uint64_t hdr_len = (flags & ZB200_DEFLATE_NO_HEADER) ? 0 : wrap == ZB200_WRAP_ZLIB ? 2 : wrap == ZB200_WRAP_GZIP ? 10 : 0;
+    const uint64_t hdr_len = (flags & ZB200_DEFLATE_NO_HEADER) ? 0 : frame_header_len(wrap);
     const uint64_t n = src_len;
     if ((prime_bits || partial_end) && (P.cfg.kind == 0 || n == 0 || prime_bits > 7 || hdr_len)) {
         set_error("zb200: pending bits need a raw shard with input at level 1..9");   // the shim handles the other cases on the host
