@@ -38,6 +38,7 @@
 #include "zb200_internal.h"
 #include <stdlib.h>
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 namespace zb {
@@ -67,7 +68,7 @@ constexpr int kHashBits = 15;
 __device__ __forceinline__ uint32_t hash4(uint32_t v) { return (v * 0x9E3779B1u) >> (32 - kHashBits); }   // four bytes, see h_levels
 
 // Ring version: kLinkWarps warps share one segment and one head[] table.  Warp w owns tiles
-// w, w+W, w+2W, ... (a tile = 128 consecutive positions).  Everything that does not touch head[]
+// w, w+W, w+2W, ... (a tile = kLinkSteps steps of 32 consecutive positions).  Everything that does not touch head[]
 // -- loads, hashes, the intra-step same-hash groups, the dist16 stores -- runs concurrently in all
 // warps; only the short "read head[], then write head[]" section of a tile is serial, and it is
 // passed from warp to warp in position order with named barriers (producer bar.arrive, consumer
@@ -76,47 +77,46 @@ constexpr int kLinkWarps = 8;
 // Stream mode: one CTA links two chunks.  The 32 KiB of priming in front of a segment is redundant work; 1 / 2 / 4 chunks per
 // segment measured 13.50 / 13.31 / 13.56 ms per step.
 constexpr uint32_t kLinkSegBytes = 2 * kChunk;
+// A segment's CTA is one serial chain of ring turns, and the kernel runs as one wave, so its time is turns per segment x
+// the latency of a turn.  A hand-off costs far more than a step's read and write of head[], so a turn takes many steps.
+constexpr int kLinkSteps = 16;
+constexpr int kLinkTile = 32 * kLinkSteps;                      // positions per tile
+constexpr int kLinkRegs = kLinkSteps / 4;                       // words of the tile per lane (a step covers eight)
+// head[], then one slot per lane that positions whose hash is not entered read and write instead
+constexpr uint32_t kLinkSmem = (1u << kHashBits) * 2 + 32 * 2;
 
 __device__ __forceinline__ void ring_wait(int id) { asm volatile("bar.sync %0, 64;" ::"r"(id) : "memory"); }
 __device__ __forceinline__ void ring_pass(int id) { asm volatile("bar.arrive %0, 64;" ::"r"(id) : "memory"); }
 
-// One warp's turn: wait for the token, then for each of the tile's four 32-position steps read head[] (every lane, the
-// caller ignores what it does not need) and let the step's group leaders write their position; pass the token on.
-// Shared-memory accesses of one warp execute in program order, which is all the steps need from each other.
-__device__ __noinline__ uint2 ring_turn(uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t q, uint32_t wmask,
-                                        int bar_in, int bar_out)
+struct LinkAddrs { uint32_t a[kLinkSteps]; };                   // per step: the shared-memory address of the lane's head[] slot
+struct LinkHeads { uint32_t h[kLinkSteps]; };                   // per step: what that slot held before the step
+
+// One warp's turn: wait for the token, then for each of the tile's steps read head[] (every lane, the caller ignores what
+// it does not need) and write the lane's position -- in exact mode only where bit k of wmask is set: the step's group
+// leaders; pass the token on.  Each step is one warp-wide read and one warp-wide write, so same-hash positions of a
+// relaxed step resolve within one store instruction.  Shared-memory accesses of one warp execute in program order, which
+// is all the steps need from each other.  A real call, so that the compiler schedules nothing else between the barriers.
+template <bool kExact>
+__device__ __noinline__ LinkHeads ring_turn(LinkAddrs a, uint32_t q, uint32_t wmask, int bar_in, int bar_out)
 {
-    uint32_t lo, hi;
-    asm volatile(
-        "{\n"
-        ".reg .pred w0, w1, w2, w3;\n"
-        ".reg .b16 t0, t1, t2, t3, s0, s1, s2, s3;\n"
-        ".reg .b32 x;\n"
-        "and.b32 x, %8, 1; setp.ne.u32 w0, x, 0;\n"
-        "and.b32 x, %8, 2; setp.ne.u32 w1, x, 0;\n"
-        "and.b32 x, %8, 4; setp.ne.u32 w2, x, 0;\n"
-        "and.b32 x, %8, 8; setp.ne.u32 w3, x, 0;\n"
-        "cvt.u16.u32 s0, %6; add.u32 x, %6, 32; cvt.u16.u32 s1, x; add.u32 x, %6, 64; cvt.u16.u32 s2, x; add.u32 x, %6, 96; cvt.u16.u32 s3, x;\n"
-        "bar.sync %9, 64;\n"
-        "ld.shared.u16 t0, [%2];\n"
-        "@w0 st.shared.u16 [%2], s0;\n"
-        "ld.shared.u16 t1, [%3];\n"
-        "@w1 st.shared.u16 [%3], s1;\n"
-        "ld.shared.u16 t2, [%4];\n"
-        "@w2 st.shared.u16 [%4], s2;\n"
-        "ld.shared.u16 t3, [%5];\n"
-        "@w3 st.shared.u16 [%5], s3;\n"
-        "bar.arrive %7, 64;\n"
-        "mov.b32 %0, {t0, t1}; mov.b32 %1, {t2, t3};\n"
-        "}\n"
-        : "=r"(lo), "=r"(hi)
-        : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(q), "r"(bar_out), "r"(wmask), "r"(bar_in)
-        : "memory");
-    return make_uint2(lo, hi);
+    LinkHeads t;
+    asm volatile("bar.sync %0, 64;" ::"r"(bar_in) : "memory");
+#pragma unroll
+    for (int k = 0; k < kLinkSteps; ++k) {
+        if (kExact)
+            asm volatile("{\n.reg .pred w;\n.reg .b32 x;\nand.b32 x, %3, %4; setp.ne.u32 w, x, 0;\n"
+                         "ld.shared.u16 %0, [%1];\n@w st.shared.u16 [%1], %2;\n}"
+                         : "=r"(t.h[k]) : "r"(a.a[k]), "r"(q + 32 * k), "r"(wmask), "r"(1u << k) : "memory");
+        else
+            asm volatile("ld.shared.u16 %0, [%1];\nst.shared.u16 [%1], %2;"
+                         : "=r"(t.h[k]) : "r"(a.a[k]), "r"(q + 32 * k) : "memory");
+    }
+    asm volatile("bar.arrive %0, 64;" ::"r"(bar_out) : "memory");
+    return t;
 }
 
 template <bool kExact>
-__global__ void __launch_bounds__(kLinkWarps * 32)
+__global__ void __launch_bounds__(kLinkWarps * 32, 3)          // 3 CTAs per SM: the 64 KiB head[] tables fill shared memory
 k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict__ dist16, const ChunkDesc* __restrict__ cd)
 {
     extern __shared__ uint16_t s_head[];                       // 2^15 entries: low 16 bits of the last position
@@ -138,9 +138,9 @@ k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict_
         origin = 0; lim = total;
     }
     const uint32_t mis = (uint32_t)((uintptr_t)buf & 3);
-    // q = p + mis indexes bytes from the 4-byte aligned base; a tile is 128 consecutive q.  Everything below is
-    // relative to the first tile of this segment, so it fits 32 bits (a segment spans <= 160 KiB + 128).
-    const uint64_t tile_beg = (prime_beg + mis) >> 7, tile_end = (seg_end + mis + 127) >> 7;
+    // q = p + mis indexes bytes from the 4-byte aligned base; tiles start at q0, the 128-aligned q in front of the first
+    // position to insert.  Everything below is relative to q0, so it fits 32 bits (a segment spans <= 288 KiB + 128).
+    const uint64_t tile_beg = (prime_beg + mis) >> 7;
     const uint64_t q0 = tile_beg * 128;
     const uint32_t* words = reinterpret_cast<const uint32_t*>(buf - mis) + tile_beg * 32;
     const uint32_t nwords = (uint32_t)min((uint64_t)0x7fffffffu, ((mis + total + 3) >> 2) - tile_beg * 32);
@@ -150,63 +150,93 @@ k_lz_link(const uint8_t* __restrict__ buf, uint64_t total, uint16_t* __restrict_
     const int q_hi = (int)(min(seg_end, lim >= origin + 3 ? lim - 3 : origin) + mis) - (int)q0;
     const int q_seg = (int)(seg_beg + mis - q0), q_end = (int)(seg_end + mis - q0);   // positions whose link is stored
     const int p_cap = (int)min((uint64_t)0x40000000u, q0 - mis + 128 - origin) - 128;   // stream position of q0, saturated (only "dd > p" uses it)
-    const uint32_t ntiles = (uint32_t)(tile_end - tile_beg);
+    const uint32_t ntiles = (uint32_t)((q_end + kLinkTile - 1) / kLinkTile);
     const uint32_t iters = (ntiles + kLinkWarps - 1) / kLinkWarps;
     const uint32_t head_base = (uint32_t)__cvta_generic_to_shared(s_head);
+    const uint32_t spare = head_base + (1u << kHashBits) * 2 + lane * 2;   // the slot of a position that is not entered
     const int bar_in = 1 + warp, bar_out = 1 + (warp + 1) % kLinkWarps;
-    auto ldw = [&](uint32_t t) { const uint32_t w = t * 32 + lane; return w < nwords ? __ldg(words + w) : 0u; };
-    auto ldx = [&](uint32_t t) { const uint32_t w = (t + 1) * 32; return w < nwords ? __ldg(words + w) : 0u; };
+    // A tile's 8 * kLinkSteps words: word 32 i + lane of the tile in w[i], the word behind the tile in e (every lane).
+    auto load = [&](uint32_t t, uint32_t (&w)[kLinkRegs], uint32_t& e) {
+        const uint32_t w0 = t * (kLinkTile / 4);
+#pragma unroll
+        for (int i = 0; i < kLinkRegs; ++i) w[i] = w0 + 32 * i + lane < nwords ? __ldg(words + w0 + 32 * i + lane) : 0u;
+        e = w0 + kLinkTile / 4 < nwords ? __ldg(words + w0 + kLinkTile / 4) : 0u;
+    };
+    // Step k's position 32 k + lane hashes the four bytes that start in word 8 k + lane / 4: that word (from lane
+    // 8 (k % 4) + lane / 4 of w[k / 4]) and the next one (from the next lane, where lane 0 stands for the following
+    // register, which only the last lanes of every fourth step read).
+    const uint32_t src = lane >> 2, shift = (lane & 3) * 8;
 
     if (warp == kLinkWarps - 1) ring_pass(bar_out);            // lets warp 0 take the first turn
     uint32_t tile = warp;
-    uint32_t cur = ldw(tile), ext = ldx(tile);
+    uint32_t cur[kLinkRegs], ext;
+    load(tile, cur, ext);
     for (uint32_t it = 0; it < iters; ++it, tile += kLinkWarps) {
-        const uint32_t cur_n = ldw(tile + kLinkWarps), ext_n = ldx(tile + kLinkWarps);
-        const int qb = (int)(tile * 128);
-        const int lo = min(max(q_lo - qb, 0), 128), hi = min(max(q_hi - qb, 0), 128);
-        uint32_t h[4], d[4], hv[4], ha[4], rd[4], wr[4];
+        uint32_t nxt[kLinkRegs], ext_n;
+        load(tile + kLinkWarps, nxt, ext_n);
+        const int qb = (int)tile * kLinkTile;
+        uint32_t v[kLinkSteps];                                  // the four bytes at each of the lane's positions
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int li = 32 * k + lane, j = li >> 2;
-            const uint32_t wa = __shfl_sync(kFullMask, cur, j);
-            uint32_t wb = __shfl_sync(kFullMask, cur, (j + 1) & 31);
-            if (j == 31) wb = ext;
-            const uint32_t v = __funnelshift_r(wa, wb, (li & 3) * 8);
-            const bool valid = li >= lo && li < hi;
-            h[k] = valid ? hash4(v) : (0x10000u + lane);
-            if (kExact) {
-                const uint32_t grp = __match_any_sync(kFullMask, h[k]);
-                const uint32_t lower = grp & lt;
-                wr[k] = (valid && (grp >> lane) == 1u) ? 1u : 0u;    // highest lane of its group writes head[]
-                rd[k] = (valid && lower == 0) ? 1u : 0u;             // lowest lane of its group reads head[]
-                d[k] = (valid && lower) ? (uint32_t)(lane - (31 - __clz(lower))) : 0u;
-            } else {
-                // Relaxed: positions of one 32-wide step that share a hash all link to the entry from before the
-                // step (a valid, merely older, chain member) and the table keeps whichever of them the hardware
-                // writes last.  No cross-lane grouping (MATCH.ANY saturates the ADU pipe), ~0.1 % larger output.
-                wr[k] = rd[k] = valid ? 1u : 0u;
-                d[k] = 0;
-            }
-            ha[k] = head_base + (h[k] & 0x7fffu) * 2;
-        }
-        // ---- serial section: this warp's turn on head[] (a real call, so that the compiler cannot schedule
-        // unrelated work between the two barriers) ----
-        const uint32_t wmask = wr[0] | (wr[1] << 1) | (wr[2] << 2) | (wr[3] << 3);
-        const uint2 got = ring_turn(ha[0], ha[1], ha[2], ha[3], (uint32_t)qb + lane, wmask, bar_in, bar_out);
-        hv[0] = got.x & 0xffffu; hv[1] = got.x >> 16; hv[2] = got.y & 0xffffu; hv[3] = got.y >> 16;
-        // ---- links out ----
-        const int slo = min(max(q_seg - qb, 0), 128), shi = min(max(q_end - qb, 0), 128);
+        for (int i = 0; i < kLinkRegs; ++i) {
+            const uint32_t succ = lane == 0 ? (i + 1 < kLinkRegs ? cur[i + 1] : ext) : cur[i];
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int li = 32 * k + lane;
-            if (rd[k]) {
-                uint32_t dd = ((uint32_t)(qb + li) - hv[k]) & 0xffffu;
-                if (dd == 0) dd = 0x10000u;
-                d[k] = (dd > kWindow || (int)dd > p_cap + qb + li) ? 0u : dd;
+            for (int r = 0; r < 4; ++r) {
+                const uint32_t wa = __shfl_sync(kFullMask, cur[i], src + 8 * r);
+                const uint32_t wb = __shfl_sync(kFullMask, succ, (src + 8 * r + 1) & 31);
+                v[4 * i + r] = __funnelshift_r(wa, wb, shift);
             }
-            if (li >= slo && li < shi) dout[qb + li] = (uint16_t)d[k];
         }
-        cur = cur_n; ext = ext_n;
+        // Most tiles lie inside [q_lo, q_hi), are not cut by q_seg, and are more than a window from the stream's start:
+        // every position is entered, all or none are stored, and no link can reach in front of the stream.
+        const bool inner = qb >= q_lo && qb + kLinkTile <= q_hi &&
+                           (qb + kLinkTile <= q_seg || (qb >= q_seg && p_cap + qb >= (int)kWindow));
+        auto link = [&](auto edge_tag) {
+            constexpr bool kEdge = decltype(edge_tag)::value;
+            LinkAddrs ha;
+            uint32_t d[kLinkSteps], rd = 0, wmask = 0;
+#pragma unroll
+            for (int k = 0; k < kLinkSteps; ++k) {
+                const int q = qb + 32 * k + lane;
+                const bool valid = !kEdge || (q >= q_lo && q < q_hi);
+                const uint32_t h = hash4(v[k]);
+                ha.a[k] = valid ? head_base + h * 2 : spare;
+                if (kExact) {
+                    const uint32_t grp = __match_any_sync(kFullMask, valid ? h : 0x10000u + lane);
+                    const uint32_t lower = grp & lt;
+                    wmask |= (valid && (grp >> lane) == 1u) ? 1u << k : 0u;    // highest lane of its group writes head[]
+                    rd |= (valid && lower == 0) ? 1u << k : 0u;                // lowest lane of its group reads head[]
+                    d[k] = (valid && lower) ? (uint32_t)(lane - (31 - __clz(lower))) : 0u;
+                } else {
+                    // Relaxed: positions of one 32-wide step that share a hash all link to the entry from before the
+                    // step (a valid, merely older, chain member) and the table keeps whichever of them the hardware
+                    // writes last.  No cross-lane grouping (MATCH.ANY saturates the ADU pipe), ~0.1 % larger output.
+                    rd |= valid ? 1u << k : 0u;
+                    d[k] = 0;
+                }
+            }
+            const LinkHeads hv = ring_turn<kExact>(ha, (uint32_t)(qb + lane), wmask, bar_in, bar_out);
+            if (!kEdge && qb < q_seg) return;                    // priming: nothing to store
+#pragma unroll
+            for (int k = 0; k < kLinkSteps; ++k) {
+                const int q = qb + 32 * k + lane;
+                if (rd >> k & 1) {
+                    if (kEdge) {
+                        uint32_t dd = ((uint32_t)q - hv.h[k]) & 0xffffu;
+                        if (dd == 0) dd = 0x10000u;
+                        d[k] = (dd > kWindow || (int)dd > p_cap + q) ? 0u : dd;
+                    } else {                                     // the same test: (dd - 1) mod 2^16 < kWindow
+                        const uint32_t dd = (uint32_t)q - hv.h[k];
+                        d[k] = (dd - 1u) & kWindow ? 0u : dd;
+                    }
+                }
+                if (!kEdge || (q >= q_seg && q < q_end)) dout[q] = (uint16_t)d[k];
+            }
+        };
+        if (inner) link(std::false_type{});
+        else link(std::true_type{});
+#pragma unroll
+        for (int i = 0; i < kLinkRegs; ++i) cur[i] = nxt[i];
+        ext = ext_n;
     }
     if (warp == 0) ring_wait(bar_in);                            // absorb the last hand-off
 }
@@ -1440,8 +1470,8 @@ static int deflate_blocks_launch(Ctx* c, const uint8_t* d_buf, uint64_t total, u
     if (cfg.chain != 0 && P.strategy != 3) {                    // Z_RLE needs no chains
         const unsigned nseg = (unsigned)(d_cd ? nblocks / kBlocksPerChunk : (total + kLinkSegBytes - 1) / kLinkSegBytes);
         // levels 1-6 trade the exact intra-step links for speed, like the reference's fast levels trade ratio
-        if (link_exact(P.level, P.strategy)) ZB_LAUNCH(k_lz_link<true>, nseg, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_buf, total, d_dist, d_cd);
-        else ZB_LAUNCH(k_lz_link<false>, nseg, kLinkWarps * 32, (1 << kHashBits) * 2, s, d_buf, total, d_dist, d_cd);
+        if (link_exact(P.level, P.strategy)) ZB_LAUNCH(k_lz_link<true>, nseg, kLinkWarps * 32, kLinkSmem, s, d_buf, total, d_dist, d_cd);
+        else ZB_LAUNCH(k_lz_link<false>, nseg, kLinkWarps * 32, kLinkSmem, s, d_buf, total, d_dist, d_cd);
     }
     ZB_CUDA(cudaMemsetAsync(d_next, 0, 4, s));
     if (cfg.kind == 2 && cfg.chain > kLazyGlobalMax && P.strategy != 3)
@@ -1567,8 +1597,8 @@ static int deflate_enqueue_dev(Ctx* c, cudaStream_t s, const uint8_t* d_buf, uin
 
 int deflate_setup()                                             // once per device, from ensure_init (under its lock)
 {
-    ZB_CUDA(cudaFuncSetAttribute(k_lz_link<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (1 << kHashBits) * 2));
-    ZB_CUDA(cudaFuncSetAttribute(k_lz_link<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (1 << kHashBits) * 2));
+    ZB_CUDA(cudaFuncSetAttribute(k_lz_link<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLinkSmem));
+    ZB_CUDA(cudaFuncSetAttribute(k_lz_link<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLinkSmem));
     ZB_CUDA(cudaFuncSetAttribute(k_lz_walk<kWalkThreadsFast, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWalkSmem));
     ZB_CUDA(cudaFuncSetAttribute(k_lz_walk<kWalkThreadsLazy, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWalkSmem + kWalkLinkSmem));
     return 0;
