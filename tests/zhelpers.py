@@ -207,3 +207,52 @@ def corpus(kind, n, seed=0):
     if kind == 4:
         return bytes(rng.choice(b"ab") for _ in range(n))
     raise ValueError(kind)
+
+
+# ---- CRC-32 / Adler-32 algebra in plain Python: references for checksums of buffers too long to hold on the host ----
+# Reflected CRC-32 polynomial arithmetic as RFC 1952 defines the CRC; independent of every library under test.
+CRC_POLY = 0xEDB88320
+ADLER_BASE = 65521
+
+
+def _gf2_mul(a, b):
+    """a * b mod P, both in the reflected representation (bit 31 = x^0)."""
+    p = 0
+    for i in range(31, -1, -1):
+        if (a >> i) & 1:
+            p ^= b
+        b = (b >> 1) ^ CRC_POLY if b & 1 else b >> 1
+    return p
+
+
+def _x8n(n):
+    """x^(8 n) mod P by square and multiply."""
+    acc, sq = 1 << 31, 1 << 23                   # x^0, x^8
+    while n:
+        if n & 1:
+            acc = _gf2_mul(acc, sq)
+        sq = _gf2_mul(sq, sq)
+        n >>= 1
+    return acc
+
+
+def crc32_cat(c1, c2, len2):
+    """CRC-32 of A || B from crc(A), crc(B) and len(B)."""
+    return _gf2_mul(c1, _x8n(len2)) ^ c2
+
+
+def crc32_drop_prefix(c12, c1, len2):
+    """CRC-32 of B from crc(A || B), crc(A) and len(B)."""
+    return c12 ^ _gf2_mul(c1, _x8n(len2))
+
+
+def adler32_cat(a1, a2, len2):
+    s1 = ((a1 & 0xFFFF) + (a2 & 0xFFFF) - 1) % ADLER_BASE
+    s2 = ((a1 >> 16) + (a2 >> 16) + len2 * ((a1 & 0xFFFF) - 1)) % ADLER_BASE
+    return (s2 << 16) | s1
+
+
+def adler32_drop_prefix(a12, a1, len2):
+    s1 = ((a12 & 0xFFFF) - (a1 & 0xFFFF) + 1) % ADLER_BASE
+    s2 = ((a12 >> 16) - (a1 >> 16) - len2 * ((a1 & 0xFFFF) - 1)) % ADLER_BASE
+    return (s2 << 16) | s1

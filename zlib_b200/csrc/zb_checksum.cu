@@ -131,7 +131,9 @@ constexpr uint32_t kTabImage = 2 * 65536;                       // bytes of the 
 constexpr size_t kMainSmem = 65536 + kTabImage;                 // 64 KiB of alignment room + image
 
 struct FoldArgs {                                               // per-launch constants of the combine, computed on the host
-    uint32_t pw_stride[10];                                     // x^(8 * S * 2^k), S = bytes one CTA covers
+    uint32_t pw_stride[10];                                     // x^(8 * S * G * 2^k), S = bytes one CTA covers, G = group
+    uint32_t pw_cta;                                            // X = x^(8 * S)
+    uint32_t group;                                             // G: records one fold thread takes before the tree
     uint32_t pw_warp[5];                                        // x^(8 * W * 2^k), W = bytes one warp covers
     uint32_t pw_last;                                           // x^(8 * D): from the end of the last full CTA to the end of the last CTA
     uint32_t pw_tail;                                           // x^(8 * (len - aligned end)): over the ragged tail
@@ -198,8 +200,10 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
 // so with q counted from the back over the first n - 1 records the register at the aligned end is
 //   ( sum_q u_q X^q ) * x^(8 D)  xor  u_last,      X = x^(8 S),
 // a polynomial in X evaluated by pairing neighbours: ten levels of ONE modular multiply per thread with the host's
-// X^(2^k), instead of one modular power per record.  Head and tail bytes, the pre-conditioning and the Adler sums
-// (closed form per record) are folded in the same pass.
+// X^(2^k), instead of one modular power per record.  With more than 1024 + 1 records (seven rounds of resident warps
+// and more: from 13.875 GiB with 148 SMs) thread t first folds records q = tG .. tG + G - 1 by Horner's rule in X, and the tree
+// then runs in X^G.  Head and tail bytes, the pre-conditioning and the Adler sums (closed form per record) are folded
+// in the same pass.
 __device__ void fold_records(const Partial* __restrict__ parts, uint32_t n_parts, const uint8_t* __restrict__ buf, uint64_t len,
                              uint64_t head, uint64_t tail_begin, const FoldArgs& fa, uint32_t* __restrict__ out2, uint32_t* s_x)
 {
@@ -218,7 +222,14 @@ __device__ void fold_records(const Partial* __restrict__ parts, uint32_t n_parts
         b = (b + pb + (uint32_t)((suffix % kAdlerBase) * pa % kAdlerBase)) % kAdlerBase;
         a %= kAdlerBase;
     }
-    if ((uint32_t)tid < m) u = ((const volatile Partial*)(parts + (m - 1 - tid)))->reg;
+    if (fa.group == 1) {
+        if ((uint32_t)tid < m) u = ((const volatile Partial*)(parts + (m - 1 - tid)))->reg;
+    } else {
+        for (uint32_t i = fa.group; i-- > 0;) {                 // u = sum_i u_(tG + i) X^i
+            const uint64_t q = (uint64_t)tid * fa.group + i;
+            if (q < m) u = gf2_mul(u, fa.pw_cta) ^ ((const volatile Partial*)(parts + (m - 1 - q)))->reg;
+        }
+    }
 #pragma unroll
     for (int k = 0; k < 5; k++) {                               // levels inside a warp: lane q takes lane q + 2^k
         const uint32_t hi = __shfl_down_sync(0xffffffffu, u, 1u << k);
@@ -647,17 +658,16 @@ int checksum_launch(Ctx* c, const uint8_t* d_buf, size_t len, uint32_t* d_out2, 
     uint64_t n_parts = blocks;                                  // one record per CTA
     int rc = c->ws[0].ensure(n_parts * sizeof(Partial));
     if (rc) return rc;
-    if (blocks > 1025) {                                        // beyond the in-kernel combine (2.5 TB): not reachable with 64-bit lengths in 180 GB
-        set_error("checksum: %u CTAs exceed the combine tree", blocks);
-        return ZB_STREAM_ERROR;
-    }
     if ((rc = c->ensure_flags()) != 0) return rc;
     unsigned int* done = c->flags.as<unsigned int>();            // zero between launches (the last CTA resets it)
     // constants of the combine (fold_records): powers of x for the uniform spacing of the CTA records and for the edges
     FoldArgs fa;
     const uint64_t S = (uint64_t)kMainWarps * iters * kStride;
     fa.cta_bytes = S;
-    for (int k = 0; k < 10; k++) fa.pw_stride[k] = host_pow8(S << k);
+    fa.group = (uint32_t)((blocks - 1 + 1023) / 1024);             // the tree pairs 1024 values; rounds past 6 give it more records
+    if (fa.group == 0) fa.group = 1;
+    fa.pw_cta = host_pow8(S);
+    for (int k = 0; k < 10; k++) fa.pw_stride[k] = host_pow8((S * fa.group) << k);
     for (int k = 0; k < 5; k++) fa.pw_warp[k] = host_pow8(((uint64_t)iters * kStride) << k);
     const uint64_t aligned = n_units * kStride;
     fa.pw_last = host_pow8(aligned - (uint64_t)(blocks - 1) * S);

@@ -88,8 +88,8 @@ struct WarpTables {
 };
 
 struct Bits {
-    const uint32_t* words;                       // 4-byte aligned base covering the stream
-    uint32_t nwords, nextw;
+    const uint32_t* words;                       // 4-byte aligned base at the last seek (see seek_bits)
+    uint32_t nwords, nextw;                      // words from that base to the end of the stream (at most 2^32 - 1) / next to load
     uint64_t buf;
     int cnt;
     uint64_t used, total;                        // bits consumed so far / bits in the stream
@@ -108,12 +108,19 @@ __device__ __forceinline__ uint32_t peek(const Bits& b, int n) { return (uint32_
 __device__ __forceinline__ void drop(Bits& b, int n) { b.buf >>= n; b.cnt -= n; b.used += n; }
 __device__ __forceinline__ bool have(const Bits& b, int n) { return b.used + (uint64_t)n <= b.total; }
 
+// Every seek moves the word base to the word holding `bitpos`, so the 32-bit word indices (nextw here, wi in the lean
+// loops) count from a recent seek, not from the start of the stream: a stream of 2^32 words (16 GiB) or more would wrap
+// them.  The lean loops seek whenever they stop, and they stop before nwords, so no index wraps between two seeks.
 __device__ void seek_bits(Bits& b, const uint8_t* in, uint64_t bitpos)
 {
     const uintptr_t a = (uintptr_t)in + (bitpos >> 3);
-    const uintptr_t base = (uintptr_t)b.words;
-    const int skip = (int)(((a - base) & 3) * 8 + (bitpos & 7));
-    b.nextw = (uint32_t)((a - base) >> 2);
+    const uintptr_t base = a & ~(uintptr_t)3;
+    const uintptr_t end = ((uintptr_t)in + (b.total >> 3) + 3) & ~(uintptr_t)3;
+    const uint64_t left = end > base ? (end - base) >> 2 : 0;
+    const int skip = (int)((a & 3) * 8 + (bitpos & 7));
+    b.words = reinterpret_cast<const uint32_t*>(base);
+    b.nwords = left > 0xffffffffu ? 0xffffffffu : (uint32_t)left;
+    b.nextw = 0;
     b.buf = 0; b.cnt = 0;
     refill(b);
     b.buf >>= skip; b.cnt -= skip;
@@ -428,8 +435,6 @@ __device__ void inflate_warp(const uint8_t* in, uint64_t in_len, uint8_t* out, u
 {
     const int lane = threadIdx.x & 31;
     Bits b;
-    b.words = reinterpret_cast<const uint32_t*>((uintptr_t)in & ~(uintptr_t)3);
-    b.nwords = (uint32_t)(((((uintptr_t)in + in_len + 3) & ~(uintptr_t)3) - (uintptr_t)b.words) >> 2);
     b.total = in_len * 8;
     seek_bits(b, in, st->bit_off);
     Out o{out, 0, out_cap, st->hist};
@@ -993,8 +998,6 @@ __device__ void seg_decode(const uint8_t* in, uint64_t in_len, const SegDesc sd,
 {
     const int lane = threadIdx.x & 31;
     Bits b;
-    b.words = reinterpret_cast<const uint32_t*>((uintptr_t)in & ~(uintptr_t)3);
-    b.nwords = (uint32_t)(((((uintptr_t)in + in_len + 3) & ~(uintptr_t)3) - (uintptr_t)b.words) >> 2);
     b.total = in_len * 8;
     seek_bits(b, in, sd.start);
     uint16_t* out = kEmit ? sym + sd.sym_off : nullptr;
@@ -1378,8 +1381,6 @@ k_find_blocks_check(const uint8_t* __restrict__ in, uint64_t in_len, const uint6
     if (j >= nprobe) return;
     WarpTables* t = &s_tab[threadIdx.x >> 5];
     Bits b;
-    b.words = reinterpret_cast<const uint32_t*>((uintptr_t)in & ~(uintptr_t)3);
-    b.nwords = (uint32_t)(((((uintptr_t)in + in_len + 3) & ~(uintptr_t)3) - (uintptr_t)b.words) >> 2);
     b.total = in_len * 8;
     seek_bits(b, in, probe[j]);
     refill(b);
