@@ -414,43 +414,108 @@ k_lz_walk(const uint8_t* __restrict__ buf, uint32_t total, uint32_t dict, const 
     }
     auto byte_at = [&](uint32_t q) { return (uint32_t)s_mem[smap(sm_off + q - win_beg)]; };   // buf[q]
 
+    // ---- level 1: screen every position of the block for a match start ----
+    // With a chain budget of one, the search at p is a pure function of p: the head dist16[p] and one 3-byte test.  Four
+    // tokens in five are literals at level 1, and in the walk below every lane of a warp pays for the search whenever one
+    // lane needs it.  So each warp first tests the 2048 positions of its own 32 sub-units, 32 consecutive positions per
+    // ballot (coalesced head loads, every lane busy), and bit r of a thread's 64-bit word is set exactly where the search
+    // at s0 + r finds a match.  The walk then emits the literals in front of the next set bit without searching.
+    const bool screened = !kSmemLinks && kind == 1 && max_chain == 1 && strategy != 3;
+    if constexpr (!kSmemLinks) {
+        static_assert(kSub == 64, "one 64-bit word of match starts per sub-unit");
+        if (screened) {
+            constexpr uint32_t kBatch = 8;                      // head loads in flight per lane
+            const uint32_t wbeg = blk_beg + (uint32_t)warp * 32u * kSub;
+            for (uint32_t k = 0; k < kSub; k += kBatch) {
+                uint32_t hd[kBatch];
+#pragma unroll
+                for (uint32_t j = 0; j < kBatch; j++) {
+                    const uint32_t p = wbeg + 32u * (k + j) + lane;
+                    hd[j] = p + kMinMatch <= blk_end ? __ldg(dist16 + p) : 0u;
+                }
+#pragma unroll
+                for (uint32_t j = 0; j < kBatch; j++) {
+                    const uint32_t o = sm_off + wbeg + 32u * (k + j) + lane - win_beg;
+                    const uint32_t d = hd[j] <= max_dist ? hd[j] : 0u;
+                    const bool hit = d != 0 && ((lds32u(s_mem, o) ^ lds32u(s_mem, o - d)) & 0xffffffu) == 0;
+                    const uint32_t word = __ballot_sync(kFullMask, hit);
+                    if (lane == 0) {                            // the bitmap borrows s_end / s_cnt, idle until the frontier
+                        const uint32_t t = warp * 32 + (k + j) / 2;
+                        ((k + j) & 1 ? s_cnt : s_end)[t] = word;     // thread t: positions s0..s0+31 in s_end, the rest in s_cnt
+                    }
+                }
+            }
+            __syncwarp();
+        }
+    }
+
     // ---- walk this thread's sub-unit ----
     const uint32_t s0 = blk_beg + tid * kSub, s1 = min(s0 + kSub, blk_end);
     uint32_t* mine = tok_tmp + (size_t)slot * kTmpPerBlock + (size_t)tid * kSubSlots + kFront;
     uint32_t ntok = 0, pos = s0;
     if (s0 < blk_end) {
         if (kind == 1) {                                        // deflate_fast, deflate.c:1448-1546
-            // Chain heads of neighbouring positions share a 32-byte sector that L1 (3 % hits: the window image leaves it
-            // ~30 KB) has lost by the time the next token starts.  Four of them are kept per thread in the shared arrays of
-            // the later phases, which are idle during the walk: one 8-byte load serves up to four token starts.
-            s_first[tid] = 0xffffffffu;
-            auto head_of = [&](uint32_t q) -> uint32_t {            // dist16[q]
-                const uint32_t g = q >> 2;
-                if (s_first[tid] != g) {
-                    const uint2 v = __ldg(reinterpret_cast<const uint2*>(dist16) + g);
-                    s_end[tid] = v.x; s_cnt[tid] = v.y; s_first[tid] = g;
-                }
-                const uint32_t w = (q & 2u) ? s_cnt[tid] : s_end[tid];
-                return (q & 1u) ? w >> 16 : w & 0xffffu;
-            };
             uint32_t held0 = 0, held1 = 0, held2 = 0;           // tokens waiting for the fourth of their group
-            while (pos < s1) {
-                const uint32_t maxlen = min(kMaxMatch, blk_end - pos);
-                Found f{0, 0};
-                if (maxlen >= kMinMatch && max_chain > 0) {
-                    if (strategy == 3) f = walk_search_rle(s_mem, sm_off + pos - win_beg, pos > win_beg, maxlen, 0);
-                    else f = walk_search<!kSmemLinks>(s_mem, sm_off + pos - win_beg, links + (pos - win_beg), kSmemLinks ? links[pos - win_beg] : head_of(pos), maxlen, max_chain, min(nice, maxlen), 0, max_dist);
-                }
-                // tokens leave four at a time (the private region is 16-byte aligned): a quarter of the store requests to L2
-                uint32_t tk;
-                if (f.len >= kMinMatch) { tk = (f.dist << 16) | (f.len - kMinMatch); pos += f.len; }
-                else { tk = byte_at(pos); pos++; }
+            // tokens leave four at a time (the private region is 16-byte aligned): a quarter of the store requests to L2
+            // (selects, not branches: the lanes of a warp are at different phases)
+            auto put = [&](uint32_t tk) {
                 const uint32_t ph = ntok & 3u;
                 if (ph == 3u) *reinterpret_cast<uint4*>(mine + ntok - 3) = make_uint4(held0, held1, held2, tk);
-                else if (ph == 2u) held2 = tk;
-                else if (ph == 1u) held1 = tk;
-                else held0 = tk;
+                held0 = ph == 0u ? tk : held0;
+                held1 = ph == 1u ? tk : held1;
+                held2 = ph == 2u ? tk : held2;
                 ntok++;
+            };
+            if (screened) {
+                // One turn per match: the literals up to the next match start, then the match.  The head of that start is
+                // loaded before the literals go out, so its trip to L2 overlaps them.  The screen had that head in a register
+                // of another lane; reloading it (0.08 loads per byte) is deliberate: keeping it needs room the 40 registers
+                // of three CTAs per SM do not leave.
+                const uint32_t n = s1 - s0;
+                auto next_start = [&](uint32_t r) -> uint32_t {    // first match start at or after offset r, else n
+                    const uint64_t m = r < 64u ? ((uint64_t)s_cnt[tid] << 32 | s_end[tid]) >> r : 0u;
+                    return m ? r + (uint32_t)__ffsll((long long)m) - 1u : n;
+                };
+                uint32_t r = 0, q = next_start(0);
+                while (r < n) {
+                    const uint32_t head = q < n ? __ldg(dist16 + s0 + q) : 0u;
+#pragma unroll 1                                        // unrolled, the literal loop makes the kernel spill
+                    for (; r < q; r++) put(byte_at(s0 + r));
+                    if (q >= n) break;
+                    const uint32_t at = s0 + q, maxlen = min(kMaxMatch, blk_end - at);
+                    const Found f = walk_search<true>(s_mem, sm_off + at - win_beg, links + (at - win_beg), head, maxlen, 1,
+                                                      min(nice, maxlen), 0, max_dist);
+                    put((f.dist << 16) | (f.len - kMinMatch));
+                    r = q + f.len;
+                    q = next_start(r);
+                }
+                pos = s0 + r;
+            } else {
+                // Chain heads of neighbouring positions share a 32-byte sector that L1 (3 % hits: the window image leaves it
+                // ~30 KB) has lost by the time the next token starts.  Four of them are kept per thread in the shared arrays
+                // of the later phases, which are idle during the walk: one 8-byte load serves up to four token starts.
+                s_first[tid] = 0xffffffffu;
+                auto head_of = [&](uint32_t q) -> uint32_t {        // dist16[q]
+                    const uint32_t g = q >> 2;
+                    if (s_first[tid] != g) {
+                        const uint2 v = __ldg(reinterpret_cast<const uint2*>(dist16) + g);
+                        s_end[tid] = v.x; s_cnt[tid] = v.y; s_first[tid] = g;
+                    }
+                    const uint32_t w = (q & 2u) ? s_cnt[tid] : s_end[tid];
+                    return (q & 1u) ? w >> 16 : w & 0xffffu;
+                };
+                while (pos < s1) {
+                    const uint32_t maxlen = min(kMaxMatch, blk_end - pos);
+                    Found f{0, 0};
+                    if (maxlen >= kMinMatch && max_chain > 0) {
+                        if (strategy == 3) f = walk_search_rle(s_mem, sm_off + pos - win_beg, pos > win_beg, maxlen, 0);
+                        else f = walk_search<!kSmemLinks>(s_mem, sm_off + pos - win_beg, links + (pos - win_beg), kSmemLinks ? links[pos - win_beg] : head_of(pos), maxlen, max_chain, min(nice, maxlen), 0, max_dist);
+                    }
+                    uint32_t tk;
+                    if (f.len >= kMinMatch) { tk = (f.dist << 16) | (f.len - kMinMatch); pos += f.len; }
+                    else { tk = byte_at(pos); pos++; }
+                    put(tk);
+                }
             }
             {
                 const uint32_t ph = ntok & 3u, at = ntok - ph;
