@@ -200,6 +200,29 @@ int zb200_inflate_batch_dev(const void *d_src, const uint64_t *d_src_off, size_t
                             void *d_dst, const uint64_t *d_dst_off, uint64_t *d_dst_len,
                             int32_t *d_status, int wrap, void *stream);
 
+/* ---- sizing: what zb200_inflate_batch would produce, without producing it ----
+ * Stream i = src[src_off[i] .. src_off[i+1]), as in zb200_inflate_batch (same wrap values, RAW / ZLIB / GZIP / AUTO).
+ * out_len[i]  = the bytes zb200_inflate_batch writes for that stream into a slot of unlimited size (or of `limit` bytes).
+ * src_used[i] = input bytes the stream occupies, through its trailer (may be NULL): where the next thing in the buffer starts.
+ * status[i]   = what zb200_inflate_batch would return for it, with one exception: the zlib Adler-32 and the gzip CRC-32
+ *               are NOT verified (they need the output bytes); a stream whose only fault is a wrong check value is Z_OK.
+ *               The gzip ISIZE is verified (against out_len mod 2^32), and so is FHCRC.
+ * limit: 0 = none; otherwise counting stops at `limit` bytes and a stream with input left reports Z_BUF_ERROR and
+ *        out_len = limit, exactly what zb200_inflate_batch reports for a slot of `limit` bytes (a bound on hostile input).
+ * src: host (pageable or pinned) or device memory; the results land in host arrays (the call synchronises its stream).
+ * Feeding out_len back as slot sizes makes zb200_inflate_batch reproduce the same lengths and statuses (but for the
+ * check values).  Long streams are sized by the counting pass of the segment decoder (see DESIGN.md), all others by a
+ * count-only form of the batch kernel: no output is stored, so a 5 MB stream may stand for 5 GiB. */
+int zb200_inflate_batch_size(const void *src, const uint64_t *src_off, size_t n, uint64_t *out_len, uint64_t *src_used,
+                             int32_t *status, int wrap, uint64_t limit, void *stream);
+
+/* Device-resident form: every pointer is device memory, nothing is copied, nothing synchronises (so, like
+ * zb200_inflate_batch_dev, every stream is counted by one warp however long it is).  d_dst_off (may be NULL; n + 1
+ * entries) receives the exclusive prefix sum of d_out_len, i.e. a ready d_dst_off for zb200_inflate_batch_dev. */
+int zb200_inflate_batch_size_dev(const void *d_src, const uint64_t *d_src_off, size_t n, uint64_t *d_out_len,
+                                 uint64_t *d_src_used, int32_t *d_status, uint64_t *d_dst_off, int wrap, uint64_t limit,
+                                 void *stream);
+
 /* ---- all GPUs of the box behind one call (SURVEY.md 8(e)): one host thread per device inside the library ----
  * Host buffers, like zlib.h's own calls (pinned memory moves fastest).  ndev <= 0 means every visible device.
  * zb200_multi_deflate: the input is cut into chunk-aligned pieces dealt round robin over the devices; every piece is

@@ -167,6 +167,8 @@ class Lib:
             "zb200_bgzf_compress": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, vp]),
             "zb200_inflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
             "zb200_inflate_batch_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
+            "zb200_inflate_batch_size": (C.c_int, [vp, vp, sz, vp, vp, vp, C.c_int, C.c_uint64, vp]),
+            "zb200_inflate_batch_size_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, C.c_uint64, vp]),
             "zb200_multi_devices": (C.c_int, []),
             "zb200_multi_deflate": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, C.c_int, C.c_int, u32p, u32p]),
             "zb200_multi_checksum": (C.c_int, [vp, sz, C.c_int, u32p, u32p]),
@@ -479,6 +481,28 @@ class Lib:
         self._check(self.dll.zb200_inflate_batch_dev(C.c_void_p(d_src), C.c_void_p(d_src_off), n, C.c_void_p(d_dst),
                                                      C.c_void_p(d_dst_off), C.c_void_p(d_dst_len), C.c_void_p(d_status),
                                                      wrap, _stream(stream)), "zb200_inflate_batch_dev")
+
+    def inflate_batch_size(self, streams, wrap: int = WRAP_ZLIB, limit: int = 0, stream=None):
+        """zb200_inflate_batch_size over a list of bytes objects -> (out_len, src_used, status) lists: what inflate_batch
+        would produce for each stream, found without producing it (zlib Adler-32 and gzip CRC-32 are not verified)."""
+        import numpy as np
+        n = len(streams)
+        src_off = np.zeros(n + 1, dtype=np.uint64)
+        src_off[1:] = np.cumsum([len(x) for x in streams], dtype=np.uint64)
+        src = np.frombuffer(b"".join(streams) + b"\0" * 8, dtype=np.uint8)
+        out_len = np.zeros(max(n, 1), dtype=np.uint64)
+        src_used = np.zeros(max(n, 1), dtype=np.uint64)
+        status = np.full(max(n, 1), -99, dtype=np.int32)
+        self._check(self.dll.zb200_inflate_batch_size(src.ctypes.data, src_off.ctypes.data, n, out_len.ctypes.data,
+                                                      src_used.ctypes.data, status.ctypes.data, wrap, limit,
+                                                      _stream(stream)), "zb200_inflate_batch_size")
+        return [int(x) for x in out_len[:n]], [int(x) for x in src_used[:n]], [int(x) for x in status[:n]]
+
+    def decompress_batch(self, streams, wrap: int = WRAP_ZLIB, limit: int = 0, stream=None):
+        """Sizes the batch with inflate_batch_size, then decodes it into slots of exactly those sizes -> (outputs,
+        statuses).  `limit` bounds every slot (0 = none): a stream longer than that reports Z_BUF_ERROR."""
+        out_len, _, _ = self.inflate_batch_size(streams, wrap=wrap, limit=limit, stream=stream)
+        return self.inflate_batch(streams, out_len, wrap=wrap, stream=stream)
 
     # ---- streaming API driven the way example.c drives it ----------------
     def deflate_stream(self, data: bytes, level=6, wbits=15, in_chunk=1 << 16, out_chunk=1 << 16, flushes=None,

@@ -212,13 +212,16 @@ __device__ __forceinline__ void store_lens(WarpTables* t, int at, int n, uint8_t
 enum Stop { kRunning = 0, kDone, kShortIn, kShortOut, kError, kWantDict };
 
 // Output cursor: positions are relative to p; bytes at negative offsets down to -hist are history.
+// Count mode (kCount, zb200_inflate_batch_size): p is null, nothing is stored, pos only counts; cap is the caller's limit.
 struct Out { uint8_t* p; uint64_t pos, cap, hist; };
 
+template <bool kCount>
 __device__ __forceinline__ uint32_t copy_match(Out& o, uint32_t len, uint32_t dist)
 {
     const int lane = threadIdx.x & 31;
     uint32_t n = len;
     if (o.pos + n > o.cap) n = (uint32_t)(o.cap - o.pos);
+    if (kCount) { o.pos += n; return n; }
     __syncwarp();
     uint8_t* dst = o.p + o.pos;
     const uint8_t* src = dst - dist;
@@ -233,7 +236,9 @@ __device__ __forceinline__ uint32_t copy_match(Out& o, uint32_t len, uint32_t di
 }
 
 // Decodes symbols of the current block until end-of-block or a stop condition (the work of
-// inflate_fast, inffast.c:67-302, plus the careful tail of inflate.c:951-1076).
+// inflate_fast, inffast.c:67-302, plus the careful tail of inflate.c:951-1076).  Count mode decodes and checks the same
+// symbols and stops at the same ones; it only leaves out the stores.
+template <bool kCount>
 __device__ Stop decode_block(Bits& b, Out& o, const WarpTables* t, InfState* st, bool streaming, bool one)
 {
     const int lane = threadIdx.x & 31;
@@ -254,7 +259,7 @@ __device__ Stop decode_block(Bits& b, Out& o, const WarpTables* t, InfState* st,
         const uint32_t kind = ent_kind(e);
         if (kind == kLit) {
             if (o.pos >= o.cap) { if (streaming) b.used = mark; return kShortOut; }
-            if (lane == 0) o.p[o.pos] = (uint8_t)ent_val(e);
+            if (!kCount && lane == 0) o.p[o.pos] = (uint8_t)ent_val(e);
             o.pos++;
             if (one) return kRunning;
             continue;
@@ -284,7 +289,7 @@ __device__ Stop decode_block(Bits& b, Out& o, const WarpTables* t, InfState* st,
         const uint32_t dist = ent_val(de) + peek(b, xd);
         drop(b, xd);
         if ((uint64_t)dist > o.pos + o.hist) { st->msg = kMsgFar; return kError; }
-        const uint32_t done = copy_match(o, mlen, dist);
+        const uint32_t done = copy_match<kCount>(o, mlen, dist);
         if (done < mlen) {
             st->copy_len = mlen - done; st->copy_dist = dist;
             return kShortOut;
@@ -303,6 +308,9 @@ __device__ Stop decode_block(Bits& b, Out& o, const WarpTables* t, InfState* st,
 // the primary table, end of block, an invalid symbol, a distance beyond the history -- leaves the loop at the start
 // of that symbol and the careful decoder above deals with it (and produces the error, if it is one).
 // Returns kDone after an end-of-block code, kRunning otherwise.
+// Count mode is the same loop without the stores and the deferred copy: a literal is its code length and one count, a
+// match its length and distance codes, the distance check against what was counted, and one add.
+template <bool kCount>
 __device__ Stop decode_fast(Bits& b, Out& o, const WarpTables* t, const uint8_t* in)
 {
     const int lane = threadIdx.x & 31;
@@ -320,9 +328,11 @@ __device__ Stop decode_fast(Bits& b, Out& o, const WarpTables* t, const uint8_t*
     if (wi0 > w_lim) return kRunning;
     uint32_t wi = wi0, off = off0;
     uint32_t lo = __ldg(words + wi), hi = __ldg(words + wi + 1), nxt = __ldg(words + wi + 2);
-    uint8_t* p = o.p + o.pos;
-    asm volatile("" : "+l"(p));                                 // one register pair; not re-derived from its parts at every use
-    __builtin_assume(__isGlobal(p));
+    uint8_t* p = kCount ? nullptr : o.p + o.pos;
+    if constexpr (!kCount) {
+        asm volatile("" : "+l"(p));                             // one register pair; not re-derived from its parts at every use
+        __builtin_assume(__isGlobal(p));
+    }
     const uint32_t* const lit = t->lit;
     const uint32_t* const dtab = t->dist;
     uint32_t produced = 0;
@@ -345,9 +355,9 @@ __device__ Stop decode_fast(Bits& b, Out& o, const WarpTables* t, const uint8_t*
             // code.  Every lane stores the (same) byte: cheaper than electing one.
             const uint32_t e2 = lit[__funnelshift_r(win, 0u, e) & (kLitSize - 1)];
             uint8_t* q = p + produced;
-            q[0] = (uint8_t)(e >> 16);
+            if (!kCount) q[0] = (uint8_t)(e >> 16);
             off += e & 31u; produced++;
-            if ((int32_t)e2 < 0) { q[1] = (uint8_t)(e2 >> 16); off += e2 & 31u; produced++; }
+            if ((int32_t)e2 < 0) { if (!kCount) q[1] = (uint8_t)(e2 >> 16); off += e2 & 31u; produced++; }
             continue;
         }
         end_wi = wi; end_off = off;                             // start of this symbol
@@ -371,6 +381,11 @@ __device__ Stop decode_fast(Bits& b, Out& o, const WarpTables* t, const uint8_t*
         const uint32_t dist = (de >> 16) + __funnelshift_r(dwin & ((1u << dtot) - 1u), 0u, de);
         if (!(de & 0x8000u) || dist > back + produced) break;
         off += dtot;
+        if (kCount) {
+            produced += mlen;
+            if (produced > p_lim) { end_wi = wi; end_off = off; break; }
+            continue;
+        }
         uint8_t* d = p + produced + lane;
         const uint8_t* s = d - dist;
         produced += mlen;
@@ -398,7 +413,7 @@ __device__ Stop decode_fast(Bits& b, Out& o, const WarpTables* t, const uint8_t*
         }
         if (produced > p_lim) { end_wi = wi; end_off = off; break; }
     }
-    if (pend) *pend_d = (uint8_t)pend_v;
+    if (!kCount && pend) *pend_d = (uint8_t)pend_v;
     __syncwarp();
     o.pos += produced;
     seek_bits(b, in, b.used + ((uint64_t)(end_wi - wi0) * 32u + end_off - off0));
@@ -429,6 +444,10 @@ __device__ void adler_fold(uint32_t& s1, uint32_t& s2, const uint8_t* p, uint64_
 
 // Whole-stream driver for one warp.  `st` is this stream's state (shared memory for the batch
 // path, global memory for a z_stream, where it carries the position between calls).
+// kCount: the sizing pass of zb200_inflate_batch_size (never streaming, out == nullptr, out_cap = the limit).  Headers,
+// tables, symbols, distances and stops are those of the decode; stored bytes are skipped, the Adler-32 is not computed,
+// and a gzip ISIZE is compared here (the decode leaves it to the k_checksum_batch launch behind it).
+template <bool kCount>
 __device__ void inflate_warp(const uint8_t* in, uint64_t in_len, uint8_t* out, uint64_t out_cap,
                              bool streaming, InfState* st, WarpTables* t,
                              uint64_t* out_len_p, uint64_t* in_used_p, int32_t* status_p, int32_t* msg_p)
@@ -631,9 +650,11 @@ __device__ void inflate_warp(const uint8_t* in, uint64_t in_len, uint8_t* out, u
             uint64_t c = st->stored_left;
             if (c > ain) c = ain;
             if (c > aout) c = aout;
-            __syncwarp();
-            for (uint64_t i = lane; i < c; i += 32) o.p[o.pos + i] = in[bytepos + i];
-            __syncwarp();
+            if (!kCount) {
+                __syncwarp();
+                for (uint64_t i = lane; i < c; i += 32) o.p[o.pos + i] = in[bytepos + i];
+                __syncwarp();
+            }
             o.pos += c; b.used += c * 8;
             st->stored_left -= (uint32_t)c;
             if (st->stored_left == 0) { seek_bits(b, in, b.used); mode = kModeBlock; }
@@ -641,12 +662,12 @@ __device__ void inflate_warp(const uint8_t* in, uint64_t in_len, uint8_t* out, u
         } else if (mode == kModeCodes) {
             // lean loop while both buffers have room, one careful symbol whenever it stops short (it leaves at symbol
             // boundaries with the position and the output count up to date, so a z_stream fed piecewise can use it too)
-            if (decode_fast(b, o, t, in) == kDone) { mode = kModeBlock; continue; }
-            stop = decode_block(b, o, t, st, streaming, true);
+            if (decode_fast<kCount>(b, o, t, in) == kDone) { mode = kModeBlock; continue; }
+            stop = decode_block<kCount>(b, o, t, st, streaming, true);
             if (stop == kDone) { stop = kRunning; mode = kModeBlock; }
             else if (stop == kShortOut && st->copy_len) mode = kModeCopy;
         } else if (mode == kModeCopy) {
-            const uint32_t done = copy_match(o, st->copy_len, st->copy_dist);
+            const uint32_t done = copy_match<kCount>(o, st->copy_len, st->copy_dist);
             st->copy_len -= done;
             if (st->copy_len) stop = kShortOut; else mode = kModeCodes;
         } else if (mode == kModeTrailer) {
@@ -656,10 +677,12 @@ __device__ void inflate_warp(const uint8_t* in, uint64_t in_len, uint8_t* out, u
                 drop(b, pad);
                 uint32_t want = 0;
                 for (int i = 0; i < 4; i++) { refill(b); want = (want << 8) | peek(b, 8); drop(b, 8); }
-                __syncwarp();
-                adler_fold(s1, s2, o.p + folded, o.pos - folded);
-                folded = o.pos;
-                if (want != ((s2 << 16) | s1)) { st->msg = kMsgCheck; stop = kError; continue; }
+                if (!kCount) {
+                    __syncwarp();
+                    adler_fold(s1, s2, o.p + folded, o.pos - folded);
+                    folded = o.pos;
+                    if (want != ((s2 << 16) | s1)) { st->msg = kMsgCheck; stop = kError; continue; }
+                }
             } else if (wrap == ZB200_WRAP_GZIP) {     // inflate.c:1099-1112; the caller checks CRC-32 and length of the output
                 if (!have(b, pad + 64)) { stop = kShortIn; continue; }
                 drop(b, pad);
@@ -699,6 +722,11 @@ __device__ void inflate_warp(const uint8_t* in, uint64_t in_len, uint8_t* out, u
     }
     __syncwarp();
     if (lane == 0) {
+        // inflate.c:1106-1110: the length check of a gzip member (its CRC-32 would need the output); lane 0 wrote the trailer
+        if (kCount && status == ZB_OK && (st->flags & kFlagGzipTrailer) && st->isize != (uint32_t)o.pos) {
+            status = ZB_DATA_ERROR;
+            st->msg = kMsgLength;
+        }
         st->mode = mode; st->last = last; st->s1 = s1; st->s2 = s2;
         st->bit_off = (uint32_t)(b.used & 7);
         uint64_t h = st->hist + o.pos;
@@ -732,7 +760,7 @@ k_inflate_batch(const uint8_t* __restrict__ src, const uint64_t* __restrict__ sr
     if (lane == 0) st->wrap = wrap;
     __syncwarp();
     const uint64_t a = src_off[i], e = ids ? src_end[i] : src_off[i + 1], oa = dst_off[i], oe = ids ? dst_end[i] : dst_off[i + 1];
-    inflate_warp(src + a, e - a, dst + oa, oe - oa, false, st, &s_tab[warp], &dst_len[i], in_used ? &in_used[i] : nullptr, &status[i], nullptr);
+    inflate_warp<false>(src + a, e - a, dst + oa, oe - oa, false, st, &s_tab[warp], &dst_len[i], in_used ? &in_used[i] : nullptr, &status[i], nullptr);
     __syncwarp();
     if (expect && lane == 0) {                                  // gzip members: {crc32, isize, 1} for the check that follows
         const bool gz = (st->flags & kFlagGzipTrailer) != 0;
@@ -746,7 +774,80 @@ k_inflate_stream(const uint8_t* __restrict__ in, uint64_t in_len, uint8_t* __res
                  InfState* __restrict__ st, InfCallResult* __restrict__ res)
 {
     __shared__ WarpTables s_tab;
-    inflate_warp(in, in_len, out, out_cap, true, st, &s_tab, &res->out_len, &res->in_used, &res->status, &res->msg);
+    inflate_warp<false>(in, in_len, out, out_cap, true, st, &s_tab, &res->out_len, &res->in_used, &res->status, &res->msg);
+}
+
+// zb200_inflate_batch_size: k_inflate_batch's warp per stream in count mode.  limit == 0: no limit.
+__global__ void __launch_bounds__(kInfWarps * 32)
+k_inflate_count(const uint8_t* __restrict__ src, const uint64_t* __restrict__ src_off, uint64_t n, uint64_t limit,
+                uint64_t* __restrict__ out_len, uint64_t* __restrict__ src_used, int32_t* __restrict__ status, int wrap)
+{
+    __shared__ WarpTables s_tab[kInfWarps];
+    __shared__ InfState s_state[kInfWarps];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint64_t i = (uint64_t)blockIdx.x * kInfWarps + warp;
+    if (i >= n) return;
+    InfState* st = &s_state[warp];
+    for (int k = lane; k < (int)(sizeof(InfState) / 4); k += 32) reinterpret_cast<uint32_t*>(st)[k] = 0;
+    __syncwarp();
+    if (lane == 0) st->wrap = wrap;
+    __syncwarp();
+    const uint64_t a = src_off[i], e = src_off[i + 1];
+    inflate_warp<true>(src + a, e - a, nullptr, limit ? limit : ~0ull, false, st, &s_tab[warp], &out_len[i],
+                       src_used ? &src_used[i] : nullptr, &status[i], nullptr);
+}
+
+// off[i] = len[0] + ... + len[i - 1] for i = 0 .. n (a d_dst_off from the sizes).  One CTA, tiles of 4096 entries.
+__global__ void __launch_bounds__(1024) k_size_scan(const uint64_t* __restrict__ len, uint64_t n, uint64_t* __restrict__ off)
+{
+    constexpr int kPer = 4;
+    __shared__ uint64_t s_warp[32];
+    __shared__ uint64_t s_carry;
+    const int t = threadIdx.x, lane = t & 31, w = t >> 5;
+    if (t == 0) s_carry = 0;
+    __syncthreads();
+    for (uint64_t base = 0; base < n; base += 1024 * kPer) {
+        uint64_t v[kPer], sum = 0;
+#pragma unroll
+        for (int k = 0; k < kPer; k++) {
+            const uint64_t j = base + (uint64_t)t * kPer + k;
+            v[k] = j < n ? len[j] : 0;
+            sum += v[k];
+        }
+        uint64_t x = sum;                                       // inclusive scan over the warp
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) { const uint64_t y = __shfl_up_sync(kFull, x, d); if (lane >= d) x += y; }
+        if (lane == 31) s_warp[w] = x;
+        __syncthreads();
+        if (w == 0) {
+            uint64_t y = s_warp[lane];
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) { const uint64_t z = __shfl_up_sync(kFull, y, d); if (lane >= d) y += z; }
+            s_warp[lane] = y;
+        }
+        __syncthreads();
+        uint64_t ex = s_carry + (w ? s_warp[w - 1] : 0) + x - sum;
+#pragma unroll
+        for (int k = 0; k < kPer; k++) {
+            const uint64_t j = base + (uint64_t)t * kPer + k;
+            if (j < n) off[j] = ex;
+            ex += v[k];
+        }
+        __syncthreads();
+        if (t == 0) s_carry += s_warp[31];
+        __syncthreads();
+    }
+    if (t == 0) off[n] = s_carry;
+}
+
+static int inflate_count_launch(const uint8_t* d_src, const uint64_t* d_src_off, size_t n, uint64_t limit, uint64_t* d_out_len,
+                                uint64_t* d_src_used, int32_t* d_status, int wrap, cudaStream_t s)
+{
+    if (n == 0) return 0;
+    ZB_LAUNCH(k_inflate_count, (unsigned)((n + kInfWarps - 1) / kInfWarps), kInfWarps * 32, 0, s, d_src, d_src_off, (uint64_t)n, limit,
+              d_out_len, d_src_used, d_status, wrap);
+    ZB_CHECK_LAUNCH();
+    return 0;
 }
 
 // d_expect: n x 3 words of scratch, needed when wrap is gzip or auto (the CRC-32 / length check runs as a second launch)
@@ -1508,7 +1609,7 @@ static int emit_segments(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_
 // (no usable boundaries, output that does not fit, damaged data), negative on CUDA errors.
 int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_dst, uint64_t cap, int wrap,
                             uint64_t* out_len, int32_t* status, cudaStream_t s, uint64_t* in_used, uint32_t* adler,
-                            int* wrap_found, void* h_dst, uint64_t* need)
+                            int* wrap_found, void* h_dst, uint64_t* need, bool count_only)
 {
     if (len < kParMinInput || wrap < 0 || wrap > kWrapAuto) return 1;
     uint64_t hdr = 0;
@@ -1583,8 +1684,9 @@ int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t*
         if (nc < 2) continue;
         // ---- streams of this library end every ZB200_CHUNK bytes of input with a marker: assume exactly that (segment j
         // holds bytes [j, j + 1) * ZB200_CHUNK of the output) and go straight to the emit pass, which checks every
-        // segment's length and arrival; if the assumption fails anywhere, the counting pass below takes over ----
-        if (source == 0 && (uint64_t)(nc - 1) * ZB200_CHUNK < cap) {
+        // segment's length and arrival; if the assumption fails anywhere, the counting pass below takes over.  (Sizing
+        // skips this: the assumption is only checked by decoding) ----
+        if (!count_only && source == 0 && (uint64_t)(nc - 1) * ZB200_CHUNK < cap) {
             std::vector<SegDesc> guess(nc);
             for (uint32_t j = 0; j < nc; j++)
                 guess[j] = SegDesc{cand[j], j + 1 < nc ? cand[j + 1] : 0, (uint64_t)j * ZB200_CHUNK,
@@ -1625,6 +1727,9 @@ int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t*
                 segs.push_back(SegDesc{seg_start, cand[r.arrive], total, seg_out});
                 total += seg_out; seg_out = 0; seg_start = cand[r.arrive];
             }
+            // the counting pass lets a segment reach 32 KiB in front of it; where less than that lies in front, only the
+            // emit pass (or the serial decoder) can tell "too far back", so sizing leaves such a stream to the count kernel
+            if (count_only && total + seg_out < kWindow32) { ok = false; break; }
             j = r.arrive;
         }
         if (!ok) return 1;                                      // damage on the true path: the serial decoder names it
@@ -1634,6 +1739,24 @@ int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t*
     if (total > cap) {                                          // the serial decoder reports Z_BUF_ERROR the reference's way
         if (need) *need = total;
         return 1;
+    }
+    if (count_only) {
+        // the stream ends at the final block's end and its trailer; a trailer cut short, or a gzip ISIZE that differs from
+        // the count (inflate.c:1106-1110), is declined: the count kernel names it
+        const uint64_t trailer_len = wrap == ZB200_WRAP_ZLIB ? 4 : wrap == ZB200_WRAP_GZIP ? 8 : 0, trailer_at = (final_end + 7) >> 3;
+        if (trailer_at + trailer_len > len) return 1;
+        if (wrap == ZB200_WRAP_GZIP) {
+            uint8_t tr[8];
+            ZB_CUDA(cudaMemcpyAsync(tr, d_src + trailer_at, 8, cudaMemcpyDeviceToHost, s));
+            ZB_CUDA(cudaStreamSynchronize(s));
+            const uint32_t isize = (uint32_t)tr[4] | ((uint32_t)tr[5] << 8) | ((uint32_t)tr[6] << 16) | ((uint32_t)tr[7] << 24);
+            if (isize != (uint32_t)total) return 1;
+        }
+        *out_len = total;
+        *status = ZB_OK;
+        if (in_used) *in_used = trailer_at + trailer_len;
+        if (wrap_found) *wrap_found = wrap;
+        return 0;
     }
     uint64_t used = 0;
     uint32_t check = 1;
@@ -2196,4 +2319,158 @@ ZB_API int zb200_inflate_batch(const void* src, const uint64_t* src_off, size_t 
     if (c2) ctx_release(c2, c2->own_stream);
     ctx_release(c, s);
     return rc;
+}
+
+// ---- sizing: zb200_inflate_batch_size ----
+// The streams zb200_inflate_batch would send to the one-stream segment decoder (same rule) get its search and counting
+// pass alone; the rest, and whatever that pass declines, go to k_inflate_count.  Only compressed bytes travel: a host
+// arena moves in groups of about kInfGroupBytes on the copy stream while earlier groups are counted, the groups alternate
+// between two streams (one group's warps do not fill the GPU), and the results come back through the context's pinned
+// words, 20 bytes per stream.
+static int size_args(const char* who, const uint64_t* src_off, size_t n, const void* out_len, const void* status, int wrap)
+{
+    if (wrap < 0 || wrap > kWrapAuto) { set_error("%s: wrap %d not supported", who, wrap); return ZB_STREAM_ERROR; }
+    if (n && (!src_off || !out_len || !status)) { set_error("%s: src_off, out_len and status are required", who); return ZB_STREAM_ERROR; }
+    return 0;
+}
+
+ZB_API int zb200_inflate_batch_size(const void* src, const uint64_t* src_off, size_t n, uint64_t* out_len, uint64_t* src_used,
+                                    int32_t* status, int wrap, uint64_t limit, void* stream)
+{
+    int rc = size_args("zb200_inflate_batch_size", src_off, n, out_len, status, wrap);
+    if (rc) return rc;
+    for (size_t i = 0; i < n; i++)
+        if (src_off[i + 1] < src_off[i]) { set_error("zb200_inflate_batch_size: src_off must not decrease"); return ZB_STREAM_ERROR; }
+    if ((rc = ensure_init()) != 0) return rc;
+    if (n == 0) return 0;
+    Ctx* c = ctx_acquire((cudaStream_t)stream);
+    if (!c) return ZB_MEM_ERROR;
+    cudaStream_t s = pick_stream(c, stream);
+    Ctx* c2 = nullptr;
+    HostStager stager;
+    const uint64_t cap = limit ? limit : ~0ull;
+    do {
+        const size_t src_total = (size_t)src_off[n];
+        const bool src_on_host = src_total != 0 && classify(src) != kDevice;
+        const uint8_t* d_src = (const uint8_t*)src;
+        if (src_on_host || src_total == 0) {
+            if ((rc = c->in.ensure(src_total + 64)) != 0) break;
+            d_src = c->in.as<uint8_t>();
+        }
+        cudaError_t e = cudaSuccess;
+        // ---- long streams: the counting pass of the segment decoder ----
+        std::vector<uint8_t> handled(n, 0);
+        size_t nhandled = 0;
+        for (size_t i = 0; i < n && !rc; i++) {
+            const uint64_t a = src_off[i], len = src_off[i + 1] - a;
+            if (len < kParMinInput || (n > kParFewStreams && len < kParLongStream)) continue;
+            if (src_on_host && len >= HostStager::kMinBytes && classify(src) == kHostPageable) {
+                HostStager one;
+                if ((rc = one.start((const uint8_t*)src + a, (uint8_t*)d_src + a, len, s)) != 0) break;
+                if ((rc = one.wait_range(0, len, s)) != 0) break;
+                one.finish();
+            } else if (src_on_host) {
+                e = cudaMemcpyAsync((uint8_t*)d_src + a, (const uint8_t*)src + a, len, cudaMemcpyHostToDevice, s);
+                if (e != cudaSuccess) { set_error("input staging failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+            }
+            uint64_t got = 0, used = 0;
+            int32_t st = ZB_OK;
+            const int pr = inflate_single_parallel(c, d_src + a, len, nullptr, cap, wrap, &got, &st, s, &used, nullptr, nullptr, nullptr,
+                                                   nullptr, true);
+            if (pr < 0) { rc = pr; break; }
+            if (pr != 0) continue;
+            out_len[i] = got; status[i] = st;
+            if (src_used) src_used[i] = used;
+            handled[i] = 1; nhandled++;
+        }
+        if (rc) { cudaStreamSynchronize(s); break; }
+        if (nhandled == n) {
+            if (cudaStreamSynchronize(s) != cudaSuccess) { set_error("inflate size failed: %s", cudaGetErrorString(cudaGetLastError())); rc = ZB_STREAM_ERROR; }
+            break;
+        }
+        // ---- groups of consecutive streams still to do, by compressed bytes ----
+        std::vector<size_t> g0, g1;
+        for (size_t i = 0; i < n;) {
+            if (handled[i]) { i++; continue; }
+            size_t j = i + 1;
+            while (j < n && !handled[j] && !(src_on_host && src_off[j] - src_off[i] >= kInfGroupBytes)) j++;
+            g0.push_back(i); g1.push_back(j);
+            i = j;
+        }
+        const size_t ng = g0.size();
+        if (ng > 1 && (c2 = ctx_acquire_own()) == nullptr) { rc = ZB_MEM_ERROR; break; }
+        if ((rc = c->ensure_aux((int)(ng + 2))) != 0) break;
+        cudaStream_t s_in = c->aux[0];
+        // descriptors: [src_off n+1][out_len n][src_used n][status n]; results: [out_len n][src_used n][status n] pinned
+        if ((rc = c->ws[0].ensure((size_t)(3 * n + 1) * 8 + n * 4)) != 0) break;
+        uint64_t* d_src_off = c->ws[0].as<uint64_t>();
+        uint64_t* d_len = d_src_off + (n + 1);
+        uint64_t* d_used = d_len + n;
+        int32_t* d_status = (int32_t*)(d_used + n);
+        if ((rc = c->ensure_pinned(n * 20 + 16)) != 0) break;
+        uint64_t* h_len = (uint64_t*)c->pinned;
+        uint64_t* h_used = h_len + n;
+        int32_t* h_status = (int32_t*)(h_used + n);
+        e = cudaMemcpyAsync(d_src_off, src_off, (n + 1) * 8, cudaMemcpyHostToDevice, s);
+        if (e == cudaSuccess) {
+            e = cudaEventRecord(c->evs[ng], s);
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(s_in, c->evs[ng], 0);
+            if (e == cudaSuccess && c2) e = cudaStreamWaitEvent(c2->own_stream, c->evs[ng], 0);
+        }
+        if (e != cudaSuccess) { set_error("descriptor upload failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+        const bool threaded = src_on_host && src_total >= HostStager::kMinBytes && classify(src) == kHostPageable;
+        if (threaded && (rc = stager.start(src, (uint8_t*)d_src, src_total, s_in)) != 0) break;
+        cudaStream_t s_main = s;
+        for (size_t k = 0; k < ng && !rc; k++) {
+            const size_t i0 = g0[k], i1 = g1[k];
+            const uint64_t a = src_off[i0], b = src_off[i1];
+            cudaStream_t s = (c2 && (k & 1)) ? c2->own_stream : s_main;
+            if (src_on_host && b > a && threaded) {
+                if ((rc = stager.wait_range(a, b - a, s)) != 0) break;
+            } else if (src_on_host && b > a) {
+                e = cudaMemcpyAsync((uint8_t*)d_src + a, (const uint8_t*)src + a, b - a, cudaMemcpyHostToDevice, s_in);
+                if (e == cudaSuccess) e = cudaEventRecord(c->evs[k], s_in);
+                if (e == cudaSuccess) e = cudaStreamWaitEvent(s, c->evs[k], 0);
+                if (e != cudaSuccess) { set_error("input staging failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+            }
+            if ((rc = inflate_count_launch(d_src, d_src_off + i0, i1 - i0, limit, d_len + i0, src_used ? d_used + i0 : nullptr,
+                                           d_status + i0, wrap, s)) != 0) break;
+            e = cudaMemcpyAsync(h_len + i0, d_len + i0, (i1 - i0) * 8, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess && src_used) e = cudaMemcpyAsync(h_used + i0, d_used + i0, (i1 - i0) * 8, cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(h_status + i0, d_status + i0, (i1 - i0) * 4, cudaMemcpyDeviceToHost, s);
+            if (e != cudaSuccess) { set_error("result copy failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+        }
+        if (c2) {
+            cudaEventRecord(c->evs[ng + 1], c2->own_stream);
+            cudaStreamWaitEvent(s, c->evs[ng + 1], 0);
+        }
+        if (rc) { cudaStreamSynchronize(s); cudaStreamSynchronize(s_in); break; }
+        e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) { set_error("inflate size readback failed: %s", cudaGetErrorString(e)); rc = ZB_STREAM_ERROR; break; }
+        for (size_t k = 0; k < ng; k++)
+            for (size_t i = g0[k]; i < g1[k]; i++) {
+                out_len[i] = h_len[i]; status[i] = h_status[i];
+                if (src_used) src_used[i] = h_used[i];
+            }
+    } while (0);
+    stager.finish();
+    if (c2) ctx_release(c2, c2->own_stream);
+    ctx_release(c, s);
+    return rc;
+}
+
+ZB_API int zb200_inflate_batch_size_dev(const void* d_src, const uint64_t* d_src_off, size_t n, uint64_t* d_out_len,
+                                        uint64_t* d_src_used, int32_t* d_status, uint64_t* d_dst_off, int wrap, uint64_t limit,
+                                        void* stream)
+{
+    int rc = size_args("zb200_inflate_batch_size_dev", d_src_off, n, d_out_len, d_status, wrap);
+    if (rc) return rc;
+    if ((rc = ensure_init()) != 0) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = inflate_count_launch((const uint8_t*)d_src, d_src_off, n, limit, d_out_len, d_src_used, d_status, wrap, s)) != 0) return rc;
+    if (d_dst_off) {
+        ZB_LAUNCH(k_size_scan, 1, 1024, 0, s, d_out_len, (uint64_t)n, d_dst_off);
+        ZB_CHECK_LAUNCH();
+    }
+    return 0;
 }

@@ -46,8 +46,10 @@ int inflate_members_launch(const uint8_t* d_src, const uint64_t* d_beg, const ui
 // The one-stream segment decoder (counting pass, then the block finder): 0 = decoded, 1 = declined, negative = CUDA error.
 int inflate_single_parallel(Ctx* c, const uint8_t* d_src, uint64_t len, uint8_t* d_dst, uint64_t cap, int wrap,
                             uint64_t* out_len, int32_t* status, cudaStream_t s, uint64_t* in_used = nullptr, uint32_t* adler = nullptr,
-                            int* wrap_found = nullptr, void* h_dst = nullptr, uint64_t* need = nullptr);
+                            int* wrap_found = nullptr, void* h_dst = nullptr, uint64_t* need = nullptr, bool count_only = false);
 // (*need: set when the stream was declined because its output, *need bytes, does not fit cap)
+// count_only: the search and the counting pass alone (zb200_inflate_batch_size): nothing is written to d_dst, no check
+// value is computed; *out_len, *in_used and a gzip ISIZE come from the accepted path and the trailer.
 // A raw stream at d_src[in_beg .. in_end) whose output is exactly out_len bytes at d_dst + out_off, with nmarks sync markers:
 // marks[first_mark ..] are the byte positions right behind them, ascending.
 struct PlannedStream { uint64_t in_beg, in_end, out_off, out_len; uint32_t first_mark, nmarks; };
