@@ -654,7 +654,9 @@ API int zo_deflate(const uint8_t *in, size_t n, uint8_t *out, size_t cap,
 /* ------------------------------------------------------------------------ */
 
 static __thread const char *last_msg;
+static __thread size_t last_max_dist;
 API const char *zo_last_msg(void) { return last_msg; }
+API size_t zo_last_max_dist(void) { return last_max_dist; }
 
 typedef struct {
     const uint8_t *in; size_t in_len; uint64_t bitpos;   /* next unread bit */
@@ -748,6 +750,7 @@ static int inflate_codes(dec *d, const dcode *lc, const dcode *dc)    /* inflate
         if (!need(d, dist_extra[t])) return 1;
         unsigned dist = d_dist_base[t] + take(d, dist_extra[t]);
         if (dist > d->out_pos) FAIL("invalid distance too far back");
+        if (dist > last_max_dist) last_max_dist = dist;
         for (unsigned i = 0; i < len; i++) {
             if (d->out_pos >= d->out_cap) { d->short_out = 1; return 1; }
             d->out[d->out_pos] = d->out[d->out_pos - dist]; d->out_pos++;
@@ -825,6 +828,7 @@ API int zo_inflate(const uint8_t *in, size_t in_len, uint8_t *out, size_t out_ca
     dec d; memset(&d, 0, sizeof(d));
     d.in = in; d.in_len = in_len; d.out = out; d.out_cap = out_cap;
     last_msg = NULL;
+    last_max_dist = 0;
     int rc = 1;
     crc_setup();
     if (out_len) *out_len = 0;

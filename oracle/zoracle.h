@@ -52,6 +52,10 @@ int zo_inflate(const uint8_t *in, size_t in_len, uint8_t *out, size_t out_cap,
 /* Last error text of zo_inflate on this thread (same strings as strm->msg). */
 const char *zo_last_msg(void);
 
+/* Largest match distance the last zo_inflate on this thread decoded (0 if none): what a
+ * stream asks of the window its header declares. */
+size_t zo_last_max_dist(void);
+
 #ifdef __cplusplus
 }
 #endif

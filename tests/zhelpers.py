@@ -33,6 +33,7 @@ class Oracle:
         d.zo_inflate.restype = C.c_int
         d.zo_inflate.argtypes = [C.c_void_p, sz, C.c_void_p, sz, C.POINTER(sz), C.POINTER(sz), C.c_int]
         d.zo_last_msg.restype = cp
+        d.zo_last_max_dist.restype, d.zo_last_max_dist.argtypes = sz, []
 
     @staticmethod
     def _p(data):
@@ -76,6 +77,10 @@ class Oracle:
     def last_msg(self):
         m = self.dll.zo_last_msg()
         return m.decode() if m else None
+
+    def last_max_dist(self):
+        """The largest distance the last inflate() decoded."""
+        return self.dll.zo_last_max_dist()
 
 
 class Ref:

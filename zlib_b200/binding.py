@@ -73,6 +73,73 @@ class gz_header(C.Structure):
                 ("hcrc", C.c_int), ("done", C.c_int)]
 
 
+def signatures():
+    """{symbol: (restype, argtypes)} of every function of include/zlib.h and include/zb200.h."""
+    ul, ui, vp, sz = C.c_ulong, C.c_uint, C.c_void_p, C.c_size_t
+    u32p, u64p, i32p = C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), C.POINTER(C.c_int32)
+    zsp = C.POINTER(z_stream)
+    return {
+        # zlib.h
+        "zlibVersion": (C.c_char_p, []), "zlibCompileFlags": (ul, []), "zError": (C.c_char_p, [C.c_int]),
+        "get_crc_table": (C.POINTER(ul), []), "inflateSyncPoint": (C.c_int, [zsp]),
+        "deflate": (C.c_int, [zsp, C.c_int]), "deflateEnd": (C.c_int, [zsp]),
+        "deflateSetDictionary": (C.c_int, [zsp, vp, ui]), "deflateCopy": (C.c_int, [zsp, zsp]),
+        "deflateReset": (C.c_int, [zsp]), "deflateParams": (C.c_int, [zsp, C.c_int, C.c_int]),
+        "deflateTune": (C.c_int, [zsp, C.c_int, C.c_int, C.c_int, C.c_int]),
+        "deflateBound": (ul, [zsp, ul]), "deflatePrime": (C.c_int, [zsp, C.c_int, C.c_int]),
+        "deflateSetHeader": (C.c_int, [zsp, vp]),
+        "inflate": (C.c_int, [zsp, C.c_int]), "inflateEnd": (C.c_int, [zsp]),
+        "inflateSetDictionary": (C.c_int, [zsp, vp, ui]), "inflateSync": (C.c_int, [zsp]),
+        "inflateCopy": (C.c_int, [zsp, zsp]), "inflateReset": (C.c_int, [zsp]),
+        "inflatePrime": (C.c_int, [zsp, C.c_int, C.c_int]), "inflateGetHeader": (C.c_int, [zsp, vp]),
+        "compress": (C.c_int, [vp, C.POINTER(ul), vp, ul]),
+        "compress2": (C.c_int, [vp, C.POINTER(ul), vp, ul, C.c_int]),
+        "compressBound": (ul, [ul]), "uncompress": (C.c_int, [vp, C.POINTER(ul), vp, ul]),
+        "adler32": (ul, [ul, vp, ui]), "adler32_combine": (ul, [ul, ul, C.c_long]),
+        "crc32": (ul, [ul, vp, ui]), "crc32_combine": (ul, [ul, ul, C.c_long]),
+        "deflateInit_": (C.c_int, [zsp, C.c_int, C.c_char_p, C.c_int]),
+        "inflateInit_": (C.c_int, [zsp, C.c_char_p, C.c_int]),
+        "deflateInit2_": (C.c_int, [zsp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_int]),
+        "inflateInit2_": (C.c_int, [zsp, C.c_int, C.c_char_p, C.c_int]),
+        # zb200.h
+        "zb200_init": (C.c_int, [C.c_int]), "zb200_device_count": (C.c_int, []),
+        "zb200_last_error": (C.c_char_p, []), "zb200_build_info": (C.c_char_p, []),
+        "zb200_alloc_pinned": (vp, [sz]), "zb200_free_pinned": (None, [vp]),
+        "zb200_alloc_device": (vp, [sz]), "zb200_free_device": (None, [vp]),
+        "zb200_copy": (C.c_int, [vp, vp, sz, vp]), "zb200_sync": (C.c_int, [vp]),
+        "zb200_copy_async": (C.c_int, [vp, vp, sz, vp]),
+        "zb200_host_register": (C.c_int, [vp, sz]), "zb200_host_unregister": (C.c_int, [vp]),
+        "zb200_ipc_export": (C.c_int, [vp, vp]), "zb200_ipc_open": (C.c_int, [vp, C.POINTER(vp)]), "zb200_ipc_close": (C.c_int, [vp]),
+        "zb200_checksum": (C.c_int, [vp, sz, u32p, u32p, vp]),
+        "zb200_checksum_dev": (C.c_int, [vp, sz, vp, vp]),
+        "zb200_checksum_batch": (C.c_int, [vp, vp, sz, vp, vp, vp]),
+        "zb200_deflate": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, C.c_int, vp]),
+        "zb200_deflate_shard": (C.c_int, [vp, sz, vp, sz, vp, C.POINTER(sz), C.c_int, C.c_int, C.c_int, u32p, u32p, vp]),
+        "zb200_deflate_shard_begin": (C.c_int, [C.POINTER(vp), vp, sz, vp, sz, vp, sz, C.c_int, C.c_int, C.c_int, vp]),
+        "zb200_deflate_shard_end": (C.c_int, [vp, C.POINTER(sz), u32p, u32p]),
+        "zb200_deflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, vp]),
+        "zb200_zip_bound": (sz, [vp, vp, sz]),
+        "zb200_zip_build": (C.c_int, [vp, vp, vp, sz, C.c_int, C.c_uint32, vp, C.POINTER(sz)]),
+        "zb200_zip_segment": (C.c_int, [vp, vp, vp, sz, C.c_int, C.c_uint32, vp, C.POINTER(sz), vp]),
+        "zb200_zip_directory": (C.c_int, [vp, vp, sz, C.c_uint32, C.c_uint64, vp, C.POINTER(sz)]),
+        "zb200_zip_list": (C.c_int, [vp, sz, vp, C.POINTER(sz)]),
+        "zb200_zip_extract": (C.c_int, [vp, sz, vp, sz, vp, vp, vp, vp, vp]),
+        "zb200_gunzip": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.POINTER(sz), vp]),
+        "zb200_bgzf_bound": (sz, [sz]),
+        "zb200_bgzf_compress": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, vp]),
+        "zb200_inflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
+        "zb200_inflate_batch_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
+        "zb200_inflate_batch_size": (C.c_int, [vp, vp, sz, vp, vp, vp, C.c_int, C.c_uint64, vp]),
+        "zb200_inflate_batch_size_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, C.c_uint64, vp]),
+        "zb200_multi_devices": (C.c_int, []),
+        "zb200_multi_deflate": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, C.c_int, C.c_int, u32p, u32p]),
+        "zb200_multi_checksum": (C.c_int, [vp, sz, C.c_int, u32p, u32p]),
+        "zb200_multi_inflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, C.c_int]),
+        "zb200_kernel_launches": (C.c_uint64, []),
+        "zb200_profile": (None, [C.c_int]), "zb200_profile_report": (C.c_int, [C.c_char_p, sz]),
+    }
+
+
 class ZipEntry:
     """One member as zb200_zip_list reports it; `raw` is the 48-byte zb200_zip_entry record."""
     __slots__ = ("name", "local_off", "comp_len", "raw_len", "crc32", "method", "flags", "raw")
@@ -113,69 +180,7 @@ class Lib:
         self.path = path
         self.dll = C.CDLL(path, mode=os.RTLD_LOCAL | os.RTLD_DEEPBIND)
         d = self.dll
-        ul, ui, vp, sz = C.c_ulong, C.c_uint, C.c_void_p, C.c_size_t
-        u32p, u64p, i32p = C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), C.POINTER(C.c_int32)
-        zsp = C.POINTER(z_stream)
-        sig = {
-            # zlib.h
-            "zlibVersion": (C.c_char_p, []), "zlibCompileFlags": (ul, []), "zError": (C.c_char_p, [C.c_int]),
-            "get_crc_table": (C.POINTER(ul), []), "inflateSyncPoint": (C.c_int, [zsp]),
-            "deflate": (C.c_int, [zsp, C.c_int]), "deflateEnd": (C.c_int, [zsp]),
-            "deflateSetDictionary": (C.c_int, [zsp, vp, ui]), "deflateCopy": (C.c_int, [zsp, zsp]),
-            "deflateReset": (C.c_int, [zsp]), "deflateParams": (C.c_int, [zsp, C.c_int, C.c_int]),
-            "deflateTune": (C.c_int, [zsp, C.c_int, C.c_int, C.c_int, C.c_int]),
-            "deflateBound": (ul, [zsp, ul]), "deflatePrime": (C.c_int, [zsp, C.c_int, C.c_int]),
-            "deflateSetHeader": (C.c_int, [zsp, vp]),
-            "inflate": (C.c_int, [zsp, C.c_int]), "inflateEnd": (C.c_int, [zsp]),
-            "inflateSetDictionary": (C.c_int, [zsp, vp, ui]), "inflateSync": (C.c_int, [zsp]),
-            "inflateCopy": (C.c_int, [zsp, zsp]), "inflateReset": (C.c_int, [zsp]),
-            "inflatePrime": (C.c_int, [zsp, C.c_int, C.c_int]), "inflateGetHeader": (C.c_int, [zsp, vp]),
-            "compress": (C.c_int, [vp, C.POINTER(ul), vp, ul]),
-            "compress2": (C.c_int, [vp, C.POINTER(ul), vp, ul, C.c_int]),
-            "compressBound": (ul, [ul]), "uncompress": (C.c_int, [vp, C.POINTER(ul), vp, ul]),
-            "adler32": (ul, [ul, vp, ui]), "adler32_combine": (ul, [ul, ul, C.c_long]),
-            "crc32": (ul, [ul, vp, ui]), "crc32_combine": (ul, [ul, ul, C.c_long]),
-            "deflateInit_": (C.c_int, [zsp, C.c_int, C.c_char_p, C.c_int]),
-            "inflateInit_": (C.c_int, [zsp, C.c_char_p, C.c_int]),
-            "deflateInit2_": (C.c_int, [zsp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_int]),
-            "inflateInit2_": (C.c_int, [zsp, C.c_int, C.c_char_p, C.c_int]),
-            # zb200.h
-            "zb200_init": (C.c_int, [C.c_int]), "zb200_device_count": (C.c_int, []),
-            "zb200_last_error": (C.c_char_p, []), "zb200_build_info": (C.c_char_p, []),
-            "zb200_alloc_pinned": (vp, [sz]), "zb200_free_pinned": (None, [vp]),
-            "zb200_alloc_device": (vp, [sz]), "zb200_free_device": (None, [vp]),
-            "zb200_copy": (C.c_int, [vp, vp, sz, vp]), "zb200_sync": (C.c_int, [vp]),
-            "zb200_copy_async": (C.c_int, [vp, vp, sz, vp]),
-            "zb200_host_register": (C.c_int, [vp, sz]), "zb200_host_unregister": (C.c_int, [vp]),
-            "zb200_ipc_export": (C.c_int, [vp, vp]), "zb200_ipc_open": (C.c_int, [vp, C.POINTER(vp)]), "zb200_ipc_close": (C.c_int, [vp]),
-            "zb200_checksum": (C.c_int, [vp, sz, u32p, u32p, vp]),
-            "zb200_checksum_dev": (C.c_int, [vp, sz, vp, vp]),
-            "zb200_checksum_batch": (C.c_int, [vp, vp, sz, vp, vp, vp]),
-            "zb200_deflate": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, C.c_int, vp]),
-            "zb200_deflate_shard": (C.c_int, [vp, sz, vp, sz, vp, C.POINTER(sz), C.c_int, C.c_int, C.c_int, u32p, u32p, vp]),
-            "zb200_deflate_shard_begin": (C.c_int, [C.POINTER(vp), vp, sz, vp, sz, vp, sz, C.c_int, C.c_int, C.c_int, vp]),
-            "zb200_deflate_shard_end": (C.c_int, [vp, C.POINTER(sz), u32p, u32p]),
-            "zb200_deflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, vp]),
-            "zb200_zip_bound": (sz, [vp, vp, sz]),
-            "zb200_zip_build": (C.c_int, [vp, vp, vp, sz, C.c_int, C.c_uint32, vp, C.POINTER(sz)]),
-            "zb200_zip_segment": (C.c_int, [vp, vp, vp, sz, C.c_int, C.c_uint32, vp, C.POINTER(sz), vp]),
-            "zb200_zip_directory": (C.c_int, [vp, vp, sz, C.c_uint32, C.c_uint64, vp, C.POINTER(sz)]),
-            "zb200_zip_list": (C.c_int, [vp, sz, vp, C.POINTER(sz)]),
-            "zb200_zip_extract": (C.c_int, [vp, sz, vp, sz, vp, vp, vp, vp, vp]),
-            "zb200_gunzip": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.POINTER(sz), vp]),
-            "zb200_bgzf_bound": (sz, [sz]),
-            "zb200_bgzf_compress": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, vp]),
-            "zb200_inflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
-            "zb200_inflate_batch_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, vp]),
-            "zb200_inflate_batch_size": (C.c_int, [vp, vp, sz, vp, vp, vp, C.c_int, C.c_uint64, vp]),
-            "zb200_inflate_batch_size_dev": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, C.c_uint64, vp]),
-            "zb200_multi_devices": (C.c_int, []),
-            "zb200_multi_deflate": (C.c_int, [vp, sz, vp, C.POINTER(sz), C.c_int, C.c_int, C.c_int, u32p, u32p]),
-            "zb200_multi_checksum": (C.c_int, [vp, sz, C.c_int, u32p, u32p]),
-            "zb200_multi_inflate_batch": (C.c_int, [vp, vp, sz, vp, vp, vp, vp, C.c_int, C.c_int]),
-            "zb200_kernel_launches": (C.c_uint64, []),
-            "zb200_profile": (None, [C.c_int]), "zb200_profile_report": (C.c_int, [C.c_char_p, sz]),
-        }
+        sig = signatures()
         self.missing = []
         for name, (res, args) in sig.items():
             try:

@@ -44,6 +44,7 @@ struct internal_state {
     /* ---- inflate ---- */
     zb200i_inflater *inf;
     int inf_wrap, inf_done, inf_bad, inf_started;
+    int sync_on; unsigned sync_have;                   /* inflateSync under way (mode SYNC) and the marker bytes matched so far: state->have */
     uLong inf_dict_id;
     /* gzip header capture for inflateGetHeader (inflate.c:634-759): a host-side shadow of the bytes the device skips */
     gz_headerp gz_head;
@@ -202,11 +203,24 @@ ZAPI int deflateSetDictionary(z_streamp strm, const Bytef *dictionary, uInt dict
 ZAPI uLong deflateBound(z_streamp strm, uLong sourceLen)        /* deflate.c:489-517 */
 {
     zs *s;
-    uLong destLen = sourceLen + ((sourceLen + 7) >> 3) + ((sourceLen + 63) >> 6) + 11;
+    uLong destLen = sourceLen + ((sourceLen + 7) >> 3) + ((sourceLen + 63) >> 6) + 11, more = 0;
     if (strm == Z_NULL || strm->state == Z_NULL || strm->state->kind != KIND_DEFLATE) return destLen;
     s = strm->state;
-    if (s->wbits != 15 || s->mem_level != 8) return destLen;
-    return compressBound(sourceLen);
+    /* both formulas count the 6 bytes of the zlib wrapper; what a stream writes beyond them is added, as zlib 1.2.5.1
+     * and later do: the dictionary id, or the gzip wrapper (18 bytes) and the deflateSetHeader fields */
+    if ((s->wrap == 1 || s->wrap == -1) && s->dict_set) more = 4;      /* the wrap turns negative once the trailer is out */
+    else if (s->wrap == 2 || s->wrap == -2) {
+        gz_headerp g = s->gzhead;
+        more = 18 - 6;
+        if (g != Z_NULL) {
+            if (g->extra != Z_NULL) more += 2 + (g->extra_len & 0xffff);
+            if (g->name != Z_NULL) more += (uLong)strlen((const char *)g->name) + 1;
+            if (g->comment != Z_NULL) more += (uLong)strlen((const char *)g->comment) + 1;
+            if (g->hcrc) more += 2;
+        }
+    }
+    if (s->wbits != 15 || s->mem_level != 8) return destLen + more;
+    return compressBound(sourceLen) + more;
 }
 
 ZAPI int deflateTune(z_streamp strm, int good_length, int max_lazy, int nice_length, int max_chain)
@@ -528,6 +542,7 @@ ZAPI int inflateReset(z_streamp strm)                           /* inflate.c:103
     strm->msg = Z_NULL;
     strm->adler = 1;
     s->inf_done = s->inf_bad = s->inf_started = 0;
+    s->sync_on = 0; s->sync_have = 0;
     s->gz_head = Z_NULL; s->gz_st = GZ_FIXED; s->gz_have = 0;
     return zb200i_inflate_reset(s->inf, s->inf_wrap | (s->wbits << 8)) == 0 ? Z_OK : Z_STREAM_ERROR;
 }
@@ -544,10 +559,12 @@ ZAPI int inflateEnd(z_streamp strm)                             /* inflate.c:115
 
 /* Walks the gzip header as its bytes are consumed and fills the caller's gz_header the way inflate.c:634-759 does:
  * fixed fields, then FEXTRA / FNAME / FCOMMENT clipped to the caller's buffers, then FHCRC; done = 1 at the end of the
- * header, -1 if the stream turns out not to be gzip (windowBits + 32).  The device decoder validates the same bytes. */
-static void gz_capture(zs *s, const unsigned char *p, size_t n)
+ * header, -1 if the stream turns out not to be gzip (windowBits + 32).  The device decoder validates the same bytes.
+ * Returns how many of the n bytes it took to see that the magic is not gzip's, 0 if it did not see that. */
+static size_t gz_capture(zs *s, const unsigned char *p, size_t n)
 {
     gz_headerp h = s->gz_head;
+    const size_t n0 = n;
     while (n && s->gz_st != GZ_DONE) {
         const unsigned c = *p++;
         n--;
@@ -557,7 +574,7 @@ static void gz_capture(zs *s, const unsigned char *p, size_t n)
             if (s->gz_have == 2 && (s->gz_fix[0] != 0x1f || s->gz_fix[1] != 0x8b)) {      /* a zlib stream */
                 if (h != Z_NULL) h->done = -1;
                 s->gz_st = GZ_DONE;
-                break;
+                return n0 - n;
             }
             if (s->gz_have < 10) break;
             s->gz_flags = s->gz_fix[3];
@@ -610,6 +627,7 @@ static void gz_capture(zs *s, const unsigned char *p, size_t n)
             h->done = 1;
         }
     }
+    return 0;
 }
 
 ZAPI int inflate(z_streamp strm, int flush)                     /* inflate.c:554-1153 */
@@ -643,7 +661,17 @@ ZAPI int inflate(z_streamp strm, int flush)                     /* inflate.c:554
 
     rc = zb200i_inflate_run(s->inf, strm->next_in, in0, strm->next_out, out0, &in_used, &out_len, &status, &msg, &check);
     if (rc != Z_OK) { strm->msg = ERR_MSG(rc == Z_MEM_ERROR ? Z_MEM_ERROR : Z_STREAM_ERROR); return rc == Z_MEM_ERROR ? Z_MEM_ERROR : Z_STREAM_ERROR; }
-    if (s->inf_wrap >= 2 && s->gz_st != GZ_DONE) gz_capture(s, strm->next_in, in_used);
+    if (s->inf_wrap >= 2 && s->gz_st != GZ_DONE) {
+        size_t at = gz_capture(s, strm->next_in, in_used);
+        if (at && s->inf_wrap == 2) {
+            /* inflate.c:597-602: gzip only, and the first two bytes are not its magic.  The reference refuses the stream
+             * right there; the device parser would wait for the whole fixed header.  What followed goes back to the caller. */
+            if (zb200i_inflate_resync(s->inf) != 0) return Z_STREAM_ERROR;       /* drops the bytes the device holds */
+            in_used = at; out_len = 0;
+            status = Z_DATA_ERROR; msg = 1;                                         /* "incorrect header check" */
+        }
+    }
+    if (in_used || out_len) s->sync_on = 0;                     /* decoding went on: an earlier inflateSync is over */
     strm->next_in += in_used; strm->avail_in -= (uInt)in_used; strm->total_in += in_used;
     strm->next_out += out_len; strm->avail_out -= (uInt)out_len; strm->total_out += out_len;
     if (s->inf_wrap) strm->adler = check;
@@ -688,32 +716,34 @@ static unsigned syncsearch(unsigned *have, const unsigned char *buf, unsigned le
 ZAPI int inflateSync(z_streamp strm)                            /* inflate.c:1262-1303 */
 {
     zs *s;
-    unsigned have = 0, used;
+    unsigned used;
     uLong in, out;
     if (strm == Z_NULL || strm->state == Z_NULL || strm->state->kind != KIND_INFLATE) return Z_STREAM_ERROR;
     s = strm->state;
-    if (strm->avail_in == 0 && zb200i_inflate_pending_input(s->inf) == 0) return Z_BUF_ERROR;
-    /* bytes the stream already holds are searched first, then the caller's */
-    {
+    if (strm->avail_in == 0 && (s->sync_on || zb200i_inflate_pending_input(s->inf) == 0)) return Z_BUF_ERROR;
+    if (!s->sync_on) {
+        /* the first call searches the bytes the stream already holds (the reference: its bit buffer), then the caller's;
+         * later calls go on with the caller's bytes and the part of a marker matched so far */
         size_t pn = zb200i_inflate_pending_input(s->inf);
+        s->sync_on = 1; s->sync_have = 0;
         if (pn) {
-            unsigned at = syncsearch(&have, zb200i_inflate_pending_bytes(s->inf), (unsigned)pn);
-            if (have == 4) {                                    /* the marker lies inside held bytes: decoding resumes right behind it */
+            unsigned at = syncsearch(&s->sync_have, zb200i_inflate_pending_bytes(s->inf), (unsigned)pn);
+            if (s->sync_have == 4) {                            /* the marker lies inside held bytes: decoding resumes right behind it */
                 in = strm->total_in; out = strm->total_out;
                 if (zb200i_inflate_resync_keep(s->inf, at) != 0) return Z_STREAM_ERROR;
                 strm->total_in = in; strm->total_out = out;
-                s->inf_bad = 0; s->inf_done = 0;
+                s->inf_bad = 0; s->inf_done = 0; s->sync_on = 0; s->sync_have = 0;
                 return Z_OK;
             }
         }
     }
-    used = syncsearch(&have, strm->next_in, strm->avail_in);
+    used = syncsearch(&s->sync_have, strm->next_in, strm->avail_in);
     strm->avail_in -= used; strm->next_in += used; strm->total_in += used;
-    if (have != 4) return Z_DATA_ERROR;
+    if (s->sync_have != 4) return Z_DATA_ERROR;
     in = strm->total_in; out = strm->total_out;
     if (zb200i_inflate_resync(s->inf) != 0) return Z_STREAM_ERROR;
     strm->total_in = in; strm->total_out = out;
-    s->inf_bad = 0; s->inf_done = 0;
+    s->inf_bad = 0; s->inf_done = 0; s->sync_on = 0; s->sync_have = 0;
     return Z_OK;
 }
 

@@ -951,10 +951,12 @@ k_huff_build(uint64_t n, BlockMeta* __restrict__ blk, const uint32_t* __restrict
         const uint32_t opt_len = dyn + tree_bits, static_len = fix;
         uint32_t opt_lenb = (opt_len + 3 + 7) >> 3;
         const uint32_t static_lenb = (static_len + 3 + 7) >> 3;
-        if (static_lenb <= opt_lenb) opt_lenb = static_lenb;
+        // trees.c _tr_flush_block: under Z_FIXED the block is fixed or stored, so stored is weighed against fixed alone;
+        // stored wins whenever it is cheapest, under every strategy (the engine's capacity counts on it)
+        if (static_lenb <= opt_lenb || force_fixed) opt_lenb = static_lenb;
         // a stored block holds at most 65535 bytes: a block of 64 KiB or more would go out as two (5 more bytes)
-        if (in_len + 4 + (in_len > 65535u ? 5u : 0u) <= opt_lenb && !force_fixed) { type = 0; body = 0; }
-        else if (static_lenb == opt_lenb || force_fixed) { type = 1; body = static_len; }
+        if (in_len + 4 + (in_len > 65535u ? 5u : 0u) <= opt_lenb) { type = 0; body = 0; }
+        else if (static_lenb == opt_lenb) { type = 1; body = static_len; }
         else {
             type = 2; body = opt_len;
             BitSink sink{blk_hdr + b * kHdrWords, 0, 0, 0, 0};

@@ -2107,11 +2107,20 @@ extern "C" int zb200i_inflate_run(zb200i_inflater* h, const uint8_t* in, size_t 
         if (st == ZB200I_NEED_INPUT || st == ZB_NEED_DICT || st == ZB_STREAM_END || st == ZB_DATA_ERROR) {
             // whatever is left of this call's window of input stays with the stream
             std::vector<uint8_t> rest(h->h_pin + res.in_used, h->h_pin + total_in);
-            if (st == ZB_STREAM_END || st == ZB_DATA_ERROR) {
-                // bytes after the end of the stream belong to the caller again
+            if (st == ZB_STREAM_END || st == ZB_DATA_ERROR || st == ZB_NEED_DICT) {
+                // bytes after the end of the stream, or after the dictionary id (inflate.c:1138 stops there too), belong to
+                // the caller again; bytes taken by an earlier call stay queued for the decode behind the dictionary
+                // The carry holds bytes only after a NEED_INPUT stop, which the decoder makes only when those bytes do not
+                // complete the item it must read next (a code and its extra bits, a header field, a stored length, the
+                // trailer): so a stream cannot end inside them.  They were counted into an earlier call's total_in and could
+                // not be handed back; should that ever happen, say so rather than drop the start of what follows.
+                if (st == ZB_STREAM_END && res.in_used < carry_n) {
+                    set_error("internal error: the stream ended inside %zu bytes held from an earlier call", carry_n - (size_t)res.in_used);
+                    return ZB_STREAM_ERROR;
+                }
                 rest.clear();
                 taken += from_new;
-                if (res.in_used < carry_n) { /* the stream ended inside bytes taken earlier: cannot hand them back */ }
+                if (st == ZB_NEED_DICT && res.in_used < carry_n) rest.assign(h->h_pin + res.in_used, h->h_pin + carry_n);
             } else {
                 taken += feed;
             }
